@@ -2,6 +2,9 @@
 """bench.py -- headline benchmark of the MultiSWAG posterior-predictive hot path.
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun)
+    python bench.py ... --dump-outputs DIR                   (also writes the last timed step's predictions, from
+                                                              inputs that are the same in every run with the same
+                                                              arguments, to compare two builds output for output)
     python bench.py --impl reference ...                     (CPU arm: the unmodified reference from baseline/_ref,
                                                               else the oracle port)
 
@@ -387,6 +390,23 @@ def ncu_traffic_bytes():
         return None
 
 
+def dump_outputs(out, out_dir, budget=32 << 20):
+    """Write the predictions [systems, samples, 2] of the last timed step to out_dir/predictions.npy (float32): all of
+    them when they fit the budget, else the rows of a fixed, seeded sample of systems (in index order), and of weight
+    samples too when one row alone exceeds it."""
+    n_sys, n_samp = out.shape[:2]
+    rng = np.random.default_rng(0)
+    cols = np.arange(n_samp)
+    if n_samp * 8 > budget:
+        cols = np.sort(rng.choice(n_samp, budget // 8, replace=False))
+    rows = np.arange(n_sys)
+    if n_sys * len(cols) * 8 > budget:
+        rows = np.sort(rng.choice(n_sys, budget // (len(cols) * 8), replace=False))
+    sel = out[torch.from_numpy(rows).to(out.device)][:, torch.from_numpy(cols).to(out.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "predictions.npy"), sel.float().cpu().numpy())
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -503,6 +523,8 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms, k_ms = float(t[0]), float(t[1])
     assert bool(torch.isfinite(out).all())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
 
     # ---- end to end through the public API with HOST buffers (pinned): H2D of x, D2H of the result
     out_h = torch.empty((n_sys, n_samp, 2), dtype=torch.float32).pin_memory()
@@ -661,7 +683,11 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the BASELINE configs[2] / configs[4] sections")
     ap.add_argument("--config3-systems", type=int, default=100_000, help="total systems of the configs[2] section")
     ap.add_argument("--config5-systems", type=int, default=125_000, help="5-planet systems per GPU of the configs[4] section")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the predictions of the last timed step to "
+                    "DIR/predictions.npy (float32; a fixed, seeded sample of systems when they exceed 32 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

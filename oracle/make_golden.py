@@ -105,7 +105,10 @@ def gen_predict():
         with RandQueue([z1[0][None].clone(), z2[0][:, None].clone(), eps[0, :, :L].clone(), eps[0, :, L:].clone()]):
             o2 = m.forward_swag(X, scale=0.5).detach()
         assert torch.equal(o2, outs[0])
+    # the noise draws go to a file of their own so that each file stays under 1 MB
+    eps = {k: out.pop(k) for k in [k for k in out if k.startswith("eps_s")]}
     np.savez_compressed(os.path.join(GOLD, "predict_v50.npz"), **out)
+    np.savez_compressed(os.path.join(GOLD, "predict_v50_eps.npz"), **eps)
 
 
 def gen_loss():
@@ -195,6 +198,9 @@ def gen_train():
         opt.step()
         rec[f"theta_ref_{s}"] = m.flatten().detach().numpy().copy()
     rec = {k: v for k, v in rec.items() if v is not None}
+    # the input noise, one step per file, keeps each file under 1 MB (tests/conftest.py::load_train_golden joins them)
+    for s, e in enumerate(rec.pop("eps_in")):
+        np.savez_compressed(os.path.join(GOLD, f"train_v50_eps_in{s}.npz"), eps_in=e)
     np.savez_compressed(os.path.join(GOLD, "train_v50.npz"), **rec)
 
 

@@ -32,12 +32,19 @@ def load_golden(name):
 
 @pytest.fixture(scope="session")
 def gold_predict():
-    return load_golden("predict_v50.npz")
+    return {**load_golden("predict_v50.npz"), **load_golden("predict_v50_eps.npz")}
+
+
+def load_train_golden():
+    """train_v50.npz with its input-noise draws, which are stored one step per file to keep each file under 1 MB."""
+    g = dict(load_golden("train_v50.npz"))
+    g["eps_in"] = np.stack([load_golden(f"train_v50_eps_in{s}.npz")["eps_in"] for s in range(3)])
+    return g
 
 
 @pytest.fixture(scope="session")
 def gold_train():
-    return load_golden("train_v50.npz")
+    return load_train_golden()
 
 
 @pytest.fixture(scope="session")

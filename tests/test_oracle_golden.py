@@ -1,6 +1,12 @@
 """CPU: the oracle restatement (oracle/restatement.py) against golden vectors that were
-produced by the unmodified reference (oracle/make_golden.py).  Bit-exact where the
-restatement uses the same torch operators in the same order."""
+produced by the unmodified reference (oracle/make_golden.py).
+
+The restatement uses the same torch operators in the same order as the reference, so on
+the torch CPU build that wrote the goldens it reproduced them bit for bit.  Other builds
+and CPUs round torch's vectorised erf / log / exp / tanh and MKL's reductions differently
+in the last bits, so the results that pass through them are held to the goldens within a
+few fp32 roundings (EPS32), a bound stated per test; inputs, draws and exact identities
+are still compared bit for bit."""
 import json
 import zlib
 
@@ -14,10 +20,19 @@ from oracle import restatement as R
 
 torch.set_num_threads(1)
 SEEDS = (0, 3, 17)
+EPS32 = float(np.finfo(np.float32).eps)
 
 
 def spec_for(seed):
     return R.ModelSpec.from_hparams(swag_stats(seed)["hparams"])
+
+
+def assert_within_eps(got, ref, n_eps, scale=None):
+    """|got - ref| <= n_eps * EPS32 * scale element-wise, in float64; scale defaults to |ref|."""
+    got, ref = np.asarray(got, np.float64), np.asarray(ref, np.float64)
+    scale = np.abs(ref) if scale is None else np.asarray(scale, np.float64)
+    err = np.abs(got - ref) / (EPS32 * scale)
+    assert err.max() <= n_eps, f"{err.max():.2f} x EPS32 (bound {n_eps})"
 
 
 def test_layout_matches_survey_offsets():
@@ -44,12 +59,17 @@ def test_sample_weights_bit_exact(gold_predict, seed):
     z1 = torch.from_numpy(gold_predict[f"z1_s{seed}"])
     z2 = torch.from_numpy(gold_predict[f"z2_s{seed}"])
     ref = torch.from_numpy(gold_predict[f"theta_ref_s{seed}"])
+    # theta = w_avg + c1 z1 sqrt(sigma) + c2 (D @ z2): the K-term sum can cancel to far below its terms, so the bound is
+    # in roundings of the terms' magnitudes (an AVX-512 x86 build: 2.9)
+    D = (pre_D - w_avg[:, None]).double()
     for i in range(z1.shape[0]):
         th = R.sample_weights(w_avg, w2_avg, pre_D, 30, 0.5, z1[i], z2[i])
-        assert torch.equal(th, ref[i])
-    # the dense d x d form of the reference (230 MB) once: identical bits
+        terms = (w_avg.double().abs() + 0.5 / np.sqrt(2.0) * z1[i].double().abs() * (w2_avg - w_avg**2).double().abs().sqrt()
+                 + 0.5 / np.sqrt(2.0 * 29) * (D.abs() @ z2[i].double().abs()))
+        assert_within_eps(th, ref[i], 8, scale=terms)
+    # the dense d x d form of the reference (230 MB) once: identical bits to the element-wise form
     th = R.sample_weights(w_avg, w2_avg, pre_D, 30, 0.5, z1[0], z2[0], dense_diag=True)
-    assert torch.equal(th, ref[0])
+    assert torch.equal(th, R.sample_weights(w_avg, w2_avg, pre_D, 30, 0.5, z1[0], z2[0]))
 
 
 @pytest.mark.parametrize("seed", SEEDS)
@@ -61,7 +81,7 @@ def test_forward_swag_fast_bit_exact(gold_predict, seed):
     ref = torch.from_numpy(gold_predict[f"out_ref_s{seed}"])
     for i in range(theta.shape[0]):
         out = R.forward_swag_fast(spec, theta[i], X, eps[i, :, :20], eps[i, :, 20:])
-        assert torch.equal(out, ref[i])
+        assert_within_eps(out, ref[i], 16)  # an AVX-512 x86 build: 3.7
     # the goldens are in-distribution (not pinned at the soft clamps)
     mu = ref[..., 0]
     assert 5.0 < float(mu.median()) < 6.5 and float((mu < 4.001).float().mean()) < 0.05
@@ -71,11 +91,14 @@ def test_loss_and_grad(gold_loss):
     testy = torch.from_numpy(gold_loss["testy"]).requires_grad_(True)
     y = torch.from_numpy(gold_loss["y"])
     per = R.lossfnc_per_system(testy, y)
-    assert torch.equal(per.detach(), torch.from_numpy(gold_loss["loss_ref"]))
+    assert_within_eps(per.detach(), gold_loss["loss_ref"], 4)  # an AVX-512 x86 build: 1.0
     (g,) = torch.autograd.grad(per.sum(), testy)
-    assert torch.equal(g, torch.from_numpy(gold_loss["grad_ref"]))
+    # relative per element, floored at 1/128 of the column's largest gradient where the terms cancel (an AVX-512 x86
+    # build: 31 x EPS32 of a cancelled element, 0.006 x EPS32 of its column's largest)
+    gref = gold_loss["grad_ref"]
+    assert_within_eps(g, gref, 4, scale=np.abs(gref) + np.abs(gref).max(0) / 128)
     sle = R.safe_log_erf(torch.from_numpy(gold_loss["sle_x"]))
-    assert torch.equal(sle, torch.from_numpy(gold_loss["sle_ref"]))
+    assert_within_eps(sle, gold_loss["sle_ref"], 4)  # an AVX-512 x86 build: 0.7
     # SURVEY fact 8: the x >= -1 branch carries f_under(0) (2.7512632e-5 in exact arithmetic,
     # 2.7477741e-5 once the two 0.6432... constants are rounded to fp32)
     assert float(R.safe_log_erf(torch.tensor([0.0]))) == 2.7477741241455078e-05
@@ -102,7 +125,7 @@ def test_training_steps(gold_train):
     theta = torch.from_numpy(g["theta0"]).clone()
     eps12 = torch.from_numpy(g["eps12"])
     out, _ = R.forward(spec, theta, X, False, None, eps12[0, :, :20], eps12[0, :, 20:], None)
-    assert float(R.lossfnc_per_system(out, y).sum()) == float(g["val_loss_ref"])
+    assert_within_eps(float(R.lossfnc_per_system(out, y).sum()), float(g["val_loss_ref"]), 4)  # an AVX-512 x86 build: 0.8
     buf = torch.zeros_like(theta)
     for s in range(3):
         th = theta.clone().requires_grad_(True)
