@@ -50,8 +50,20 @@ class TrainHParams(C.Structure):
     ]
 
 
+class AdamHParams(C.Structure):
+    """bnn_adam_hparams (include/bnnchaos.h)."""
+
+    _fields_ = [
+        ("beta1", C.c_double),
+        ("beta2", C.c_double),
+        ("eps", C.c_double),
+        ("step", C.c_int64),
+    ]
+
+
 _CFG = C.POINTER(ModelConfig)
 _HP = C.POINTER(TrainHParams)
+_ADAM = C.POINTER(AdamHParams)
 
 # name -> (restype, argtypes); must list every symbol of include/bnnchaos.h
 SIGNATURES = {
@@ -91,6 +103,11 @@ SIGNATURES = {
         C.c_int,
         [_CFG, _HP, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, C.c_int64, c_f32p, c_f32p, c_f32p, C.c_uint64,
          C.c_uint64, c_f32p, c_f32p, C.c_void_p, C.c_void_p],
+    ),
+    "bnn_train_step_adam": (
+        C.c_int,
+        [_CFG, _HP, _ADAM, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, C.c_int64, c_f32p, c_f32p, c_f32p,
+         C.c_uint64, C.c_uint64, c_f32p, c_f32p, C.c_void_p, C.c_void_p],
     ),
     "bnn_train_noise": (
         C.c_int,

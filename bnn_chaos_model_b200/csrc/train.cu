@@ -1,4 +1,4 @@
-// K4: fused SWAG training step -- noisy forward + analytic backward + clip + SGD-momentum for n_seeds
+// K4: fused SWAG training step -- noisy forward + analytic backward + clip + SGD-momentum or Adam for n_seeds
 // independent models in one call, and the validation loss (bnn_eval_loss).
 //
 // Reference: SWAGModel.training_step (/root/reference/spock_reg_model.py:722-732) -> lossfnc (:579-583) ->
@@ -22,7 +22,8 @@
 // input, both hidden activations and the latent rows stay in shared memory (feature-major [feature][row]) for the
 // whole forward + backward; every thread accumulates its own block of every weight gradient in registers over all
 // systems of the CTA, writes one partial gradient vector per CTA, and a second kernel adds the partials in a fixed
-// order (bit-reproducible SWAG moments), a third computes the global norm, clips and applies SGD.
+// order (bit-reproducible SWAG moments), a third computes the global norm, clips and applies SGD (bnn_train_step) or
+// Adam (bnn_train_step_adam).
 #include <stdlib.h>
 #include <string.h>
 
@@ -97,41 +98,86 @@ __global__ void __launch_bounds__(256) train_reduce_kernel(const float* __restri
     if (threadIdx.x == 0) sq[s * gridDim.x + blockIdx.x] = sh[0];
 }
 
-// clip_grad_norm_ (coef = clip / (norm + 1e-6), applied when < 1) + torch.optim.SGD with momentum / weight decay.
-__global__ void __launch_bounds__(256) train_update_kernel(const float* __restrict__ grad, const float* __restrict__ sq,
-                                                           int n_blocks, int d, int F, int B, bnn_train_hparams hp,
-                                                           float* __restrict__ theta, float* __restrict__ mom,
-                                                           float* __restrict__ grad_out, float* __restrict__ metrics) {
+// Prologue of both update kernels: clip_grad_norm_ over seed s's whole gradient (coef = clip / (norm + 1e-6), applied
+// when < 1), grad_out and the metric slots known from the gradient.  Returns the factor the gradient is scaled by
+// (min(1, coef)) and this thread's gradient element in gi (0 past d).
+__device__ __forceinline__ float clip_prologue(const float* __restrict__ grad, const float* __restrict__ sq, int n_blocks,
+                                               int d, int B, const bnn_train_hparams& hp, float* __restrict__ grad_out,
+                                               float* __restrict__ metrics, float& gi) {
     const int s = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
-    const int DP = d + DPAD;
     float ss = 0.f;
     for (int b = 0; b < n_blocks; ++b) ss += sq[s * n_blocks + b];
     const float norm = sqrtf(ss);
     const float coef = hp.clip_norm / (norm + 1e-6f);
-    const float* g = grad + (int64_t)s * DP;
-    if (i < d) {
-        const float gi = g[i];
-        if (grad_out) grad_out[(int64_t)s * d + i] = gi;
-        if (hp.apply_update) {
-            const int64_t o = (int64_t)s * d + i;
-            const float th = theta[o];
-            float dp = coef < 1.0f ? gi * coef : gi;
-            if (hp.weight_decay != 0.f) dp = fmaf(hp.weight_decay, th, dp);
-            const float buf = hp.first_step ? dp : fmaf(hp.momentum, mom[o], dp);
-            mom[o] = buf;
-            theta[o] = th - hp.lr * buf;
-        }
-    }
+    const float clip = coef < 1.0f ? coef : 1.0f;
+    const float* g = grad + (int64_t)s * (d + DPAD);
+    gi = i < d ? g[i] : 0.f;
+    if (grad_out && i < d) grad_out[(int64_t)s * d + i] = gi;
     if (metrics && blockIdx.x == gridDim.x - 1 && threadIdx.x == 255) {
         float* m = metrics + s * 8;
         const float nll = g[d + SLOT_NLL], skl = g[d + SLOT_SKL] * hp.beta_out;
         m[0] = nll / (float)B;
         m[3] = skl / (float)B;
         m[4] = norm;
-        m[5] = coef < 1.0f ? coef : 1.0f;
+        m[5] = clip;
         m[6] = isfinite(nll + skl + norm) ? 0.f : 1.f;
         m[7] = 0.f;
         // m[1] (loss with reg) and m[2] (input_kl) are completed by train_metrics_kernel, which reads lv_in before the update
+    }
+    return clip;
+}
+
+// clip_grad_norm_ + torch.optim.SGD with momentum / weight decay.
+__global__ void __launch_bounds__(256) train_update_kernel(const float* __restrict__ grad, const float* __restrict__ sq,
+                                                           int n_blocks, int d, int B, bnn_train_hparams hp,
+                                                           float* __restrict__ theta, float* __restrict__ mom,
+                                                           float* __restrict__ grad_out, float* __restrict__ metrics) {
+    const int s = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+    float gi;
+    const float clip = clip_prologue(grad, sq, n_blocks, d, B, hp, grad_out, metrics, gi);
+    if (i < d && hp.apply_update) {
+        const int64_t o = (int64_t)s * d + i;
+        const float th = theta[o];
+        float dp = gi * clip;   // clip == 1 when not clipping: exact
+        if (hp.weight_decay != 0.f) dp = fmaf(hp.weight_decay, th, dp);
+        const float buf = hp.first_step ? dp : fmaf(hp.momentum, mom[o], dp);
+        mom[o] = buf;
+        theta[o] = th - hp.lr * buf;
+    }
+}
+
+// The per-step scalars of torch.optim.Adam, computed on the host in double (torch's Python floats) and cast once.
+struct AdamStep {
+    float step_size;   // lr / (1 - beta1^t), beta1 of THIS step (the one-cycle schedule cycles it)
+    float bc2_sqrt;    // sqrt(1 - beta2^t)
+    float w1;          // 1 - beta1: exp_avg.lerp_(g, 1 - beta1)
+    float beta2, w2;   // beta2, 1 - beta2: exp_avg_sq.mul_(beta2).addcmul_(g, g, value=1 - beta2)
+    float eps;
+    int first;         // t == 1: both buffers are zero and are not read (a fresh optimizer; no memset needed)
+};
+
+// clip_grad_norm_ + torch.optim.Adam (amsgrad=False, maximize=False; weight decay is L2 added to the gradient, not AdamW):
+//   g += wd theta;  m = lerp(m, g, 1 - beta1);  v = beta2 v + (1 - beta2) g^2;  theta -= step_size m / (sqrt(v) / bc2_sqrt + eps)
+__global__ void __launch_bounds__(256) train_adam_update_kernel(const float* __restrict__ grad, const float* __restrict__ sq,
+                                                                int n_blocks, int d, int B, bnn_train_hparams hp, AdamStep a,
+                                                                float* __restrict__ theta, float* __restrict__ exp_avg,
+                                                                float* __restrict__ exp_avg_sq, float* __restrict__ grad_out,
+                                                                float* __restrict__ metrics) {
+    const int s = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+    float gi;
+    const float clip = clip_prologue(grad, sq, n_blocks, d, B, hp, grad_out, metrics, gi);
+    if (i < d && hp.apply_update) {
+        const int64_t o = (int64_t)s * d + i;
+        const float th = theta[o];
+        float g = gi * clip;
+        if (hp.weight_decay != 0.f) g = fmaf(hp.weight_decay, th, g);
+        const float m0 = a.first ? 0.f : exp_avg[o], v0 = a.first ? 0.f : exp_avg_sq[o];
+        const float diff = g - m0;   // torch's lerp: from the nearer end of the weight
+        const float m = a.w1 < 0.5f ? fmaf(a.w1, diff, m0) : fmaf(-diff, 1.0f - a.w1, g);
+        const float v = fmaf(a.w2 * g, g, v0 * a.beta2);
+        exp_avg[o] = m;
+        exp_avg_sq[o] = v;
+        theta[o] = th - a.step_size * (m / (sqrtf(v) / a.bc2_sqrt + a.eps));
     }
 }
 
@@ -289,6 +335,85 @@ static SeedPlan pick_plan(const bnn_model_config* cfg, int64_t B, int n_seeds) {
 }
 static int pick_n_cta(const bnn_model_config* cfg, int64_t B, int n_seeds) { return pick_plan(cfg, B, n_seeds).n_cta; }
 
+// Everything of a training step before the optimizer's update, shared by bnn_train_step (SGD) and bnn_train_step_adam:
+// the argument checks (`who` names the entry in messages; `state_ok`: the optimizer's state buffers are given, required
+// when hp->apply_update), the seed-group launches of the training kernel, the fixed-order reduce and the logged metrics.
+// On BNN_OK the reduced gradient and its per-block sums of squares are enqueued on st for the update kernel.
+struct Gradient { const float* grad; const float* sq; int nb, d; };
+static int train_gradient(const char* who, bool state_ok, const char* state_name, const bnn_model_config* cfg,
+                          const bnn_train_hparams* hp, int32_t n_seeds, const float* d_theta, const float* d_x,
+                          const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
+                          const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_metrics,
+                          void* d_workspace, cudaStream_t st, Gradient* out) {
+    int rc = validate_config(cfg);
+    if (rc != BNN_OK) return rc;
+    if ((rc = check_device()) != BNN_OK) return rc;
+    BNN_REQUIRE(hp && d_theta && d_x && d_y && d_workspace, BNN_E_ARG, "%s: null pointer", who);
+    BNN_REQUIRE(n_seeds >= 1 && n_seeds <= 65535 && B >= 1 && B < (1ll << 30), BNN_E_ARG,
+                "%s: n_seeds=%d B=%lld out of range", who, n_seeds, (long long)B);
+    BNN_REQUIRE(!hp->apply_update || state_ok, BNN_E_ARG, "%s: %s required to update", who, state_name);
+    const bool any = d_eps_in || d_eps12 || d_eps_sum, all = d_eps_in && d_eps12 && d_eps_sum;
+    BNN_REQUIRE(!any || all, BNN_E_ARG, "%s: give all of eps_in, eps12, eps_sum or none", who);
+    BNN_REQUIRE(aligned16(d_workspace) && (!d_eps12 || (aligned16(d_eps12) && aligned16(d_eps_sum))), BNN_E_ALIGN,
+                "%s: workspace / eps12 / eps_sum must be 16-byte aligned", who);
+    const int F = cfg->n_features, T = cfg->n_times, FP = (F + 3) & ~3;
+    BNN_REQUIRE(shape_ok(cfg), BNN_E_CONFIG, "%s: compiled for the reference's shape T=100, F=41 (got T=%d, F=%d)", who, T, F);
+    const FlatLayout fl(F);
+    const SeedPlan plan = pick_plan(cfg, B, n_seeds);
+    const int n_cta = plan.n_cta;
+    const int DP = fl.d + DPAD, nb = (DP + 255) / 256;
+    float* partial = (float*)d_workspace;
+    float* grad = partial + (size_t)n_seeds * n_cta * DP;
+    float* sq = grad + (size_t)n_seeds * DP;
+    float* head_rec = sq + (size_t)n_seeds * nb;
+    head_rec += (4 - ((uintptr_t)head_rec / sizeof(float)) % 4) % 4;  // 16-byte aligned records
+
+    Params prm;
+    prm.theta = d_theta; prm.X = d_x; prm.Y = d_y; prm.batch_index = d_batch_index;
+    prm.eps_in = d_eps_in; prm.eps12 = d_eps12; prm.eps_sum = d_eps_sum;
+    prm.partial = partial;
+    prm.head_rec = head_rec;
+    prm.xprod = head_rec + (size_t)n_seeds * B * REC;   // REC is a multiple of 4: stays 16-byte aligned
+    prm.B = (int)B; prm.T = T; prm.F = F; prm.FP = FP; prm.n_cta = n_cta; prm.seed0 = 0;
+    prm.seed = seed; prm.step = step; prm.zero_mask = cfg->zero_mask;
+    prm.hc = HeadConsts{cfg->lo_mu, cfg->hi_mu, cfg->lo_sd, cfg->hi_sd};
+    prm.beta_out = hp->beta_out;
+    prm.saliency = 0; prm.gx_out = nullptr; prm.mu_out = nullptr;
+    if (use_tc(cfg, B)) {
+        const size_t smem_tc = (size_t)tcx::SmemTC(cfg->zero_mask).total * sizeof(float);
+        static PerDeviceOnce attr_tc_done;
+        if (attr_tc_done.need()) {
+            BNN_CUDA(cudaFuncSetAttribute(train_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        }
+        for (int s0 = 0; s0 < n_seeds; s0 += plan.per) {   // seed groups (pick_plan); every buffer is indexed by the global seed
+            prm.seed0 = s0;
+            train_tc_kernel<<<dim3(n_cta, n_seeds - s0 < plan.per ? n_seeds - s0 : plan.per), tcx::NTHR_TC, smem_tc, st>>>(prm);
+        }
+    } else {
+        const size_t smem3 = (size_t)Smem3(T, F).total * sizeof(float);
+        static PerDeviceOnce attr3_done;
+        if (attr3_done.need()) {
+            BNN_CUDA(cudaFuncSetAttribute(train_fwd_bwd3_kernel<100, 41>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          227 * 1024));
+        }
+        for (int s0 = 0; s0 < n_seeds; s0 += plan.per) {
+            prm.seed0 = s0;
+            train_fwd_bwd3_kernel<100, 41><<<dim3(n_cta, n_seeds - s0 < plan.per ? n_seeds - s0 : plan.per), NTHR3, smem3, st>>>(
+                prm);
+        }
+    }
+    BNN_CUDA(cudaGetLastError());
+    train_reduce_kernel<<<dim3(nb, n_seeds), 256, 0, st>>>(partial, d_theta, n_cta, fl.d, F, hp->beta_in * (float)B,
+                                                          hp->beta_out * (float)B, grad, sq);
+    BNN_CUDA(cudaGetLastError());
+    if (d_metrics) {
+        train_metrics_kernel<<<n_seeds, 32, 0, st>>>(d_theta, grad, fl.d, F, (int)B, *hp, d_metrics);
+        BNN_CUDA(cudaGetLastError());
+    }
+    *out = Gradient{grad, sq, nb, fl.d};
+    return BNN_OK;
+}
+
 }  // namespace train
 }  // namespace bnn
 
@@ -312,76 +437,53 @@ int bnn_train_step(const bnn_model_config* cfg, const bnn_train_hparams* hp, int
                    const float* d_eps_in, const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
                    float* d_grad_out, float* d_metrics, void* d_workspace, void* stream) {
     using namespace bnn;
-    int rc = validate_config(cfg);
-    if (rc != BNN_OK) return rc;
-    if ((rc = check_device()) != BNN_OK) return rc;
-    BNN_REQUIRE(hp && d_theta && d_x && d_y && d_workspace, BNN_E_ARG, "bnn_train_step: null pointer");
-    BNN_REQUIRE(n_seeds >= 1 && n_seeds <= 65535 && B >= 1 && B < (1ll << 30), BNN_E_ARG,
-                "bnn_train_step: n_seeds=%d B=%lld out of range", n_seeds, (long long)B);
-    BNN_REQUIRE(!hp->apply_update || d_momentum, BNN_E_ARG, "bnn_train_step: momentum buffer required to update");
-    const bool any = d_eps_in || d_eps12 || d_eps_sum, all = d_eps_in && d_eps12 && d_eps_sum;
-    BNN_REQUIRE(!any || all, BNN_E_ARG, "bnn_train_step: give all of eps_in, eps12, eps_sum or none");
-    BNN_REQUIRE(aligned16(d_workspace) && (!d_eps12 || (aligned16(d_eps12) && aligned16(d_eps_sum))), BNN_E_ALIGN,
-                "bnn_train_step: workspace / eps12 / eps_sum must be 16-byte aligned");
-    const int F = cfg->n_features, T = cfg->n_times, FP = (F + 3) & ~3;
-    BNN_REQUIRE(train::shape_ok(cfg), BNN_E_CONFIG,
-                "bnn_train_step: compiled for the reference's shape T=100, F=41 (got T=%d, F=%d)", T, F);
-    const FlatLayout fl(F);
     cudaStream_t st = (cudaStream_t)stream;
-    const train::SeedPlan plan = train::pick_plan(cfg, B, n_seeds);
-    const int n_cta = plan.n_cta;
-    const int DP = fl.d + train::DPAD, nb = (DP + 255) / 256;
-    float* partial = (float*)d_workspace;
-    float* grad = partial + (size_t)n_seeds * n_cta * DP;
-    float* sq = grad + (size_t)n_seeds * DP;
-    float* head_rec = sq + (size_t)n_seeds * nb;
-    head_rec += (4 - ((uintptr_t)head_rec / sizeof(float)) % 4) % 4;  // 16-byte aligned records
+    train::Gradient gr;
+    const int rc = train::train_gradient("bnn_train_step", d_momentum, "momentum buffer", cfg, hp, n_seeds, d_theta, d_x, d_y,
+                                        d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step, d_metrics, d_workspace,
+                                        st, &gr);
+    if (rc != BNN_OK) return rc;
+    train::train_update_kernel<<<dim3(gr.nb, n_seeds), 256, 0, st>>>(gr.grad, gr.sq, gr.nb, gr.d, (int)B, *hp, d_theta,
+                                                                    d_momentum, d_grad_out, d_metrics);
+    BNN_CUDA(cudaGetLastError());
+    return BNN_OK;
+}
 
-    train::Params prm;
-    prm.theta = d_theta; prm.X = d_x; prm.Y = d_y; prm.batch_index = d_batch_index;
-    prm.eps_in = d_eps_in; prm.eps12 = d_eps12; prm.eps_sum = d_eps_sum;
-    prm.partial = partial;
-    prm.head_rec = head_rec;
-    prm.xprod = head_rec + (size_t)n_seeds * B * train::REC;   // REC is a multiple of 4: stays 16-byte aligned
-    prm.B = (int)B; prm.T = T; prm.F = F; prm.FP = FP; prm.n_cta = n_cta; prm.seed0 = 0;
-    prm.seed = seed; prm.step = step; prm.zero_mask = cfg->zero_mask;
-    prm.hc = HeadConsts{cfg->lo_mu, cfg->hi_mu, cfg->lo_sd, cfg->hi_sd};
-    prm.beta_out = hp->beta_out;
-    prm.saliency = 0; prm.gx_out = nullptr; prm.mu_out = nullptr;
-    if (train::use_tc(cfg, B)) {
-        const size_t smem_tc = (size_t)train::tcx::SmemTC(cfg->zero_mask).total * sizeof(float);
-        static PerDeviceOnce attr_tc_done;
-        if (attr_tc_done.need()) {
-            BNN_CUDA(cudaFuncSetAttribute(train::train_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        }
-        for (int s0 = 0; s0 < n_seeds; s0 += plan.per) {   // seed groups (pick_plan); every buffer is indexed by the global seed
-            prm.seed0 = s0;
-            train::train_tc_kernel<<<dim3(n_cta, n_seeds - s0 < plan.per ? n_seeds - s0 : plan.per), train::tcx::NTHR_TC, smem_tc,
-                                     st>>>(prm);
-        }
-    } else {
-        const size_t smem3 = (size_t)train::Smem3(T, F).total * sizeof(float);
-        static PerDeviceOnce attr3_done;
-        if (attr3_done.need()) {
-            BNN_CUDA(cudaFuncSetAttribute(train::train_fwd_bwd3_kernel<100, 41>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          227 * 1024));
-        }
-        for (int s0 = 0; s0 < n_seeds; s0 += plan.per) {
-            prm.seed0 = s0;
-            train::train_fwd_bwd3_kernel<100, 41><<<dim3(n_cta, n_seeds - s0 < plan.per ? n_seeds - s0 : plan.per), train::NTHR3,
-                                                   smem3, st>>>(prm);
-        }
-    }
-    BNN_CUDA(cudaGetLastError());
-    train::train_reduce_kernel<<<dim3(nb, n_seeds), 256, 0, st>>>(partial, d_theta, n_cta, fl.d, F,
-                                                                 hp->beta_in * (float)B, hp->beta_out * (float)B, grad, sq);
-    BNN_CUDA(cudaGetLastError());
-    if (d_metrics) {
-        train::train_metrics_kernel<<<n_seeds, 32, 0, st>>>(d_theta, grad, fl.d, F, (int)B, *hp, d_metrics);
-        BNN_CUDA(cudaGetLastError());
-    }
-    train::train_update_kernel<<<dim3(nb, n_seeds), 256, 0, st>>>(grad, sq, nb, fl.d, F, (int)B, *hp, d_theta, d_momentum,
-                                                                 d_grad_out, d_metrics);
+int bnn_train_step_adam(const bnn_model_config* cfg, const bnn_train_hparams* hp, const bnn_adam_hparams* adam,
+                        int32_t n_seeds, float* d_theta, float* d_exp_avg, float* d_exp_avg_sq, const float* d_x,
+                        const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
+                        const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_grad_out,
+                        float* d_metrics, void* d_workspace, void* stream) {
+    using namespace bnn;
+    // torch.optim.Adam's constructor checks, written so that NaN fails them too
+    BNN_REQUIRE(hp && adam, BNN_E_ARG, "bnn_train_step_adam: null pointer");
+    BNN_REQUIRE(hp->lr >= 0.f, BNN_E_ARG, "bnn_train_step_adam: invalid learning rate %g", (double)hp->lr);
+    BNN_REQUIRE(hp->weight_decay >= 0.f, BNN_E_ARG, "bnn_train_step_adam: invalid weight_decay %g", (double)hp->weight_decay);
+    BNN_REQUIRE(adam->beta1 >= 0.0 && adam->beta1 < 1.0, BNN_E_ARG, "bnn_train_step_adam: invalid beta1 %g (need [0, 1))",
+                adam->beta1);
+    BNN_REQUIRE(adam->beta2 >= 0.0 && adam->beta2 < 1.0, BNN_E_ARG, "bnn_train_step_adam: invalid beta2 %g (need [0, 1))",
+                adam->beta2);
+    BNN_REQUIRE(adam->eps >= 0.0, BNN_E_ARG, "bnn_train_step_adam: invalid eps %g", adam->eps);
+    BNN_REQUIRE(adam->step >= 1, BNN_E_ARG, "bnn_train_step_adam: step %lld (t is 1-based)", (long long)adam->step);
+    cudaStream_t st = (cudaStream_t)stream;
+    train::Gradient gr;
+    const int rc = train::train_gradient("bnn_train_step_adam", d_exp_avg && d_exp_avg_sq, "exp_avg and exp_avg_sq", cfg, hp,
+                                        n_seeds, d_theta, d_x, d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step,
+                                        d_metrics, d_workspace, st, &gr);
+    if (rc != BNN_OK) return rc;
+    // bias corrections as torch computes them from Python floats, with this step's beta1
+    const double t = (double)adam->step;
+    train::AdamStep a;
+    a.step_size = (float)((double)hp->lr / (1.0 - pow(adam->beta1, t)));
+    a.bc2_sqrt = (float)sqrt(1.0 - pow(adam->beta2, t));
+    a.w1 = (float)(1.0 - adam->beta1);
+    a.beta2 = (float)adam->beta2;
+    a.w2 = (float)(1.0 - adam->beta2);
+    a.eps = (float)adam->eps;
+    a.first = adam->step == 1;
+    train::train_adam_update_kernel<<<dim3(gr.nb, n_seeds), 256, 0, st>>>(gr.grad, gr.sq, gr.nb, gr.d, (int)B, *hp, a,
+                                                                         d_theta, d_exp_avg, d_exp_avg_sq, d_grad_out,
+                                                                         d_metrics);
     BNN_CUDA(cudaGetLastError());
     return BNN_OK;
 }

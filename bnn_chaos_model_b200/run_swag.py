@@ -132,7 +132,7 @@ def run(args, X_train, y_train, X_val, y_val, out_dir: Optional[str] = None, gro
             m.load(torch.load(os.path.join(args.init, checkpoint_filename(args, s) + ".pt"), map_location=dev, weights_only=True))
         models.append(m)
     trainer = MultiSeedSWAGTrainer(models, X_train, y_train, X_val, y_val, batch_size=args.batch_size, device=dev,
-                                   seed=args.noise_seed + 1000003 * rank, swa_start=swa["swa_start"])
+                                   seed=args.noise_seed + 1000003 * rank, swa_start=swa["swa_start"], optimizer=args.optimizer)
     logs = trainer.fit(epochs, validate=X_val is not None)
     stats = gather_seed_statistics(trainer, args.n_seeds, group)
     paths = None
@@ -153,6 +153,8 @@ def build_parser():
     ap.add_argument("--batch_size", type=int, default=2000)
     ap.add_argument("--epochs", type=int, default=0, help="override 1 + swa_steps / steps_per_epoch")
     ap.add_argument("--noise_seed", type=int, default=0)
+    ap.add_argument("--optimizer", choices=("sgd", "adam"), default="sgd",
+                    help="sgd: the reference's SGD with momentum; adam: torch.optim.Adam (betas 0.9, 0.999, eps 1e-8)")
     ap.add_argument("--data", default=None, help="npz with X_train, y_train, X_val, y_val (normalised)")
     ap.add_argument("--synthetic", type=int, nargs=2, default=(8000, 1000), metavar=("N_TRAIN", "N_VAL"))
     ap.add_argument("--init", default=None, help="directory of <checkpoint_filename>.pt flat weight vectors")

@@ -3,13 +3,14 @@
 Replaces, for a group of seeds, the reference's sequential per-seed runs (train.sh:3-6) of
 ``run_swag.py``: Lightning ``Trainer.fit`` (run_swag.py:74-82) looping over
 ``SWAGModel.training_step`` (spock_reg_model.py:722-732) + backward + ``gradient_clip_val`` +
-``SGD(momentum)`` (:709-711), per-epoch ``validation_step`` at w and w_avg (:787-799) and
-``aggregate_model`` once ``global_step > swa_start`` (:801-813, :763-785).
+``SGD(momentum)`` (:709-711) -- or ``torch.optim.Adam`` (``optimizer="adam"``) -- per-epoch
+``validation_step`` at w and w_avg (:787-799) and ``aggregate_model`` once ``global_step > swa_start`` (:801-813,
+:763-785).
 
-Everything stays on the device: the data set, one flat weight / momentum vector per seed, the SWAG
-statistics.  A step is ONE ``bnn_train_step`` call for all seeds of this rank (per-seed shuffles are
-an index tensor, the four noise tensors are counter-based Philox draws); an epoch ends with one
-``bnn_eval_loss`` over both weight sets and one ``bnn_swag_collect``.  Seeds are independent: ranks
+Everything stays on the device: the data set, one flat weight vector and the optimizer state (momentum, or Adam's two
+moment vectors) per seed, the SWAG statistics.  A step is ONE ``bnn_train_step`` (``bnn_train_step_adam``) call for all
+seeds of this rank (per-seed shuffles are an index tensor, the four noise tensors are counter-based Philox draws); an
+epoch ends with one ``bnn_eval_loss`` over both weight sets and one ``bnn_swag_collect``.  Seeds are independent: ranks
 own disjoint seed groups and exchange nothing (SURVEY.md section 8e).
 """
 from __future__ import annotations
@@ -19,7 +20,7 @@ from typing import List, Optional, Sequence
 import torch
 
 from . import _lib
-from ._lib import BnnChaosError, TrainHParams
+from ._lib import AdamHParams, BnnChaosError, TrainHParams
 from .multiswag import shard_range
 from .spock_reg_model import ScheduleFinished, SWAGModel, VarModel, one_cycle_lr_momentum
 
@@ -30,6 +31,20 @@ def seeds_of_rank(n_seeds: int, rank: int, world: int):
     return list(range(lo, hi))
 
 
+def check_optimizer(optimizer: str, betas, eps):
+    """The optimizer name and torch.optim.Adam's checks of betas / eps, as ValueError.  Returns (beta1, beta2, eps)."""
+    if optimizer not in ("sgd", "adam"):
+        raise ValueError(f"optimizer must be 'sgd' or 'adam', got {optimizer!r}")
+    beta1, beta2 = (float(b) for b in betas)
+    if not 0.0 <= beta1 < 1.0:
+        raise ValueError(f"Invalid beta parameter at index 0: {beta1}")
+    if not 0.0 <= beta2 < 1.0:
+        raise ValueError(f"Invalid beta parameter at index 1: {beta2}")
+    if not 0.0 <= float(eps):
+        raise ValueError(f"Invalid epsilon value: {eps}")
+    return beta1, beta2, float(eps)
+
+
 class MultiSeedSWAGTrainer:
     """Arguments beyond the data: ``swa_start`` -- the moment-collection gate (default hparams['swa_start'], the value
     :808 reads; SURVEY section 0 fact 13); ``noisy_val`` -- validate with the input / summary noise on, the reference's
@@ -37,11 +52,18 @@ class MultiSeedSWAGTrainer:
     reference's ``MultiStepLR([swa_params['swa_start']], swa_recording_lr_factor)`` (:709-720) per optimizer step.  The
     reference registers both of its schedulers with 'interval': 'steps'; its pre-training run ENDS through the one-cycle
     scheduler's ValueError (find_minima.py:79-82), so in the reference's Lightning version such schedulers do step every
-    optimizer step -- both trainers here follow that reading (pass ``lr_milestone=False`` for a constant swa_lr)."""
+    optimizer step -- both trainers here follow that reading (pass ``lr_milestone=False`` for a constant swa_lr).
+
+    ``optimizer`` -- "sgd" (the reference's SGD with hparams['momentum']) or "adam": torch.optim.Adam with ``betas`` and
+    ``eps`` (amsgrad off, L2 weight decay hparams['weight_decay']) on the same clipped gradient; per seed it keeps
+    ``exp_avg`` / ``exp_avg_sq`` and counts its steps in ``adam_step``.  Validation, ``collect`` and ``export`` do not
+    depend on the choice."""
 
     def __init__(self, models: Sequence[SWAGModel], X_train, y_train, X_val=None, y_val=None, batch_size=2000,
                  device=None, seed=0, swa_start: Optional[int] = None, noisy_val: Optional[bool] = None,
-                 lr_milestone: bool = True):
+                 lr_milestone: bool = True, optimizer: str = "sgd", betas=(0.9, 0.999), eps: float = 1e-8):
+        beta1, beta2, eps = check_optimizer(optimizer, betas, eps)   # before anything touches a device
+        self.optimizer, self.betas, self.eps = optimizer, (beta1, beta2), eps
         if len(models) == 0:
             raise ValueError("no seed models")
         self.models: List[SWAGModel] = list(models)
@@ -68,7 +90,11 @@ class MultiSeedSWAGTrainer:
         self.lr_factor = float(sp.get("swa_recording_lr_factor", 0.5))
         self.swa_start = int(m0.hparams["swa_start"] if swa_start is None else swa_start)  # :808 reads hparams
         self.theta = torch.stack([m._flat().detach().float() for m in self.models]).to(dev).contiguous()  # [S,d]
-        self.momentum = torch.zeros_like(self.theta)
+        sgd = optimizer == "sgd"
+        self.momentum = torch.zeros_like(self.theta) if sgd else None
+        self.exp_avg = None if sgd else torch.empty_like(self.theta)       # not read at Adam's first step
+        self.exp_avg_sq = None if sgd else torch.empty_like(self.theta)
+        self.adam_step = 0
         d = self.theta.shape[1]
         self.w_avg = torch.zeros((self.S, d), device=dev)
         self.w2_avg = torch.zeros((self.S, d), device=dev)
@@ -97,13 +123,16 @@ class MultiSeedSWAGTrainer:
             nbytes = lib.bnn_train_workspace_bytes(cfg, B, self.S)
             if self._ws is None or self._ws.numel() * 4 < nbytes:
                 self._ws = torch.empty((nbytes + 3) // 4, device=self.device, dtype=torch.float32)
-            _lib.check(
-                lib.bnn_train_step(cfg, hp, self.S, _lib.ptr(self.theta), _lib.ptr(self.momentum), _lib.ptr(self.X),
-                                   _lib.ptr(self.y), _lib.ptr(batch_index), B, None, None, None, self.seed,
-                                   self.global_step, None, _lib.ptr(self.metrics), _lib.ptr(self._ws),
-                                   _lib.current_stream_ptr()),
-                "bnn_train_step",
-            )
+            rest = (_lib.ptr(self.X), _lib.ptr(self.y), _lib.ptr(batch_index), B, None, None, None, self.seed, self.global_step,
+                    None, _lib.ptr(self.metrics), _lib.ptr(self._ws), _lib.current_stream_ptr())
+            if self.optimizer == "adam":
+                adam = AdamHParams(beta1=self.step_beta1(), beta2=self.betas[1], eps=self.eps, step=self.adam_step + 1)
+                _lib.check(lib.bnn_train_step_adam(cfg, hp, adam, self.S, _lib.ptr(self.theta), _lib.ptr(self.exp_avg),
+                                                   _lib.ptr(self.exp_avg_sq), *rest), "bnn_train_step_adam")
+                self.adam_step += 1
+            else:
+                _lib.check(lib.bnn_train_step(cfg, hp, self.S, _lib.ptr(self.theta), _lib.ptr(self.momentum), *rest),
+                           "bnn_train_step")
         self.first_step = False
         self.global_step += 1
 
@@ -118,6 +147,10 @@ class MultiSeedSWAGTrainer:
     def step_hparams(self):
         """momentum, weight decay, clip and KL weights of the coming step (constant in the SWAG phase, :722-732)."""
         return self.hp
+
+    def step_beta1(self) -> float:
+        """Adam's beta1 for the coming step (constant in the SWAG phase)."""
+        return self.betas[0]
 
     def epoch_batches(self):
         """Per-seed shuffles of the training set (DataLoader(shuffle=True), :276): [n_batches] of ([S,B] int32, B)."""
@@ -229,7 +262,8 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
 
     * KL annealing of ``VarModel.training_step`` (:595-598): both KL weights ramp over the first 30 % of ``steps``;
     * the custom one-cycle schedule (:27-159, :634) over ``int(0.9 * steps)`` optimizer steps: lr AND momentum
-      (0.95 -> 0.85 -> 0.95) change every step;
+      (0.95 -> 0.85 -> 0.95) change every step -- with ``optimizer="adam"`` the cycled momentum is Adam's beta1 of the
+      step (``betas[0]`` is not used), as CustomOneCycleLR sets ``betas[0]`` of an optimizer that has betas;
     * no moment collection; validation once per epoch, the weights of the best epoch are kept
       (ModelCheckpoint, find_minima.py:67,82);
     * the run ends when the scheduler is stepped past its total -- the reference's ValueError
@@ -237,13 +271,15 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
     """
 
     def __init__(self, models: Sequence[VarModel], X_train, y_train, X_val=None, y_val=None, batch_size=None,
-                 device=None, seed=0, noisy_val: Optional[bool] = None):
+                 device=None, seed=0, noisy_val: Optional[bool] = None, optimizer: str = "sgd", betas=(0.9, 0.999),
+                 eps: float = 1e-8):
         m0 = models[0]
         for m in models:  # the SWAG bookkeeping of the base class reads these; unused here
             if not hasattr(m, "K"):
                 m.K, m.c, m.swa_params = 1, 1, {"swa_lr": m.lr}
         super().__init__(models, X_train, y_train, X_val, y_val, batch_size=batch_size or m0.batch_size, device=device,
-                         seed=seed, swa_start=1 << 62, noisy_val=noisy_val, lr_milestone=False)
+                         seed=seed, swa_start=1 << 62, noisy_val=noisy_val, lr_milestone=False, optimizer=optimizer,
+                         betas=betas, eps=eps)
         self.steps = int(m0.steps)
         self.max_lr = float(m0.lr)
         self.total_sched = int(0.9 * self.steps)
@@ -269,6 +305,10 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
     def step_hparams(self):
         _, mom, b_in, b_out = self.schedule()
         return dict(self.hp, momentum=mom, beta_in=b_in, beta_out=b_out)
+
+    def step_beta1(self) -> float:
+        """The one-cycle momentum of the coming step, Adam's beta1 (CustomOneCycleLR with use_beta1)."""
+        return self.schedule()[1]
 
     def train_step(self, batch_index, B, lr=None):
         if lr is None:

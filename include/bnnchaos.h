@@ -183,6 +183,31 @@ int bnn_train_step(const bnn_model_config* cfg, const bnn_train_hparams* hp, int
                    const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
                    const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
                    float* d_grad_out, float* d_metrics, void* d_workspace, void* stream);
+
+/* The same step with torch.optim.Adam (amsgrad=False, maximize=False) in place of SGD -- what a caller of
+ * clip_grad_norm_ + Adam.step() after the training step's backward gets.  Weight decay is L2 added to the gradient
+ * (not AdamW):
+ *   g *= min(1, clip/(|g|_2 + 1e-6));  g += wd*theta;  m = m + (1-beta1)(g - m);  v = beta2 v + (1-beta2) g^2;
+ *   theta -= lr/(1 - beta1^t) * m / (sqrt(v)/sqrt(1 - beta2^t) + eps).
+ * The bias corrections are computed in double from this call's beta1 / beta2 / t, as torch does; beta1 may change from
+ * call to call (the one-cycle schedule sets betas[0] every step).  At t == 1 d_exp_avg / d_exp_avg_sq are not read (a
+ * fresh optimizer's zero state): they need no initialisation.
+ * From hp: lr, weight_decay, clip_norm, beta_in, beta_out, apply_update; momentum and first_step are not read.
+ * State per seed (device, caller-owned): d_exp_avg, d_exp_avg_sq [n_seeds,d] (required when apply_update = 1;
+ * apply_update = 0 leaves theta and both buffers untouched).  BNN_E_ARG for what torch.optim.Adam rejects: lr < 0,
+ * weight_decay < 0, beta outside [0, 1), eps < 0, and t < 1.  Every other argument, the metrics and the workspace
+ * (bnn_train_workspace_bytes) as bnn_train_step.
+ */
+typedef struct bnn_adam_hparams {
+    double beta1, beta2, eps;  /* torch.optim.Adam betas / eps; beta1 may change per call (one-cycle schedule) */
+    int64_t step;              /* t of this update, 1-based; t == 1: both moment buffers are treated as zero */
+} bnn_adam_hparams;
+
+int bnn_train_step_adam(const bnn_model_config* cfg, const bnn_train_hparams* hp, const bnn_adam_hparams* adam,
+                        int32_t n_seeds, float* d_theta, float* d_exp_avg, float* d_exp_avg_sq, const float* d_x,
+                        const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
+                        const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
+                        float* d_grad_out, float* d_metrics, void* d_workspace, void* stream);
 /* Saliency (figures/feature_importance.py:93-131, gradforward): for each of n_models weight vectors d_theta[m]
  * (flatten() order; the script uses w_avg) and each system b: mu_b = predict_instability(compute_summary_stats(
  * mask(x_b)))[0] and g = d mu_b / d x (all F columns of the masked input; no input noise, no summary noise).
