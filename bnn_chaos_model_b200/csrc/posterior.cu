@@ -11,11 +11,16 @@
 //   "median of dists": median of mu and of std over the weight samples              main_figures.py:276-277
 //
 // Keeping this on the device turns the [N, U, 2] prediction block (48 GB at BASELINE config 3) into [N, 8].
+//
+// Held-out score of the same block against labels [N, 2]: per system, the log of the ensemble's mean likelihood of the
+// label pair and the mean of the per-unit losses, with the model's own loss (VarModel._lossfnc, loss_device.cuh) as the
+// per-unit term.  [N, U, 2] -> [N, 2].
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
+#include "loss_device.cuh"
 
 namespace bnn {
 
@@ -326,6 +331,56 @@ __global__ void __launch_bounds__(512) summarize_select_kernel(const float* __re
     }
 }
 
+// ---- held-out score: one CTA per system.  loss[u] = -(l(y0) + l(y1)) of nll_terms, bit for bit bnn_nll_fwd_bwd's
+// per-system loss.  Each thread walks the units tid, tid + 256, ... keeping, in double, m = max of -loss, s = sum of
+// exp(-loss - m) (rescaled when m grows) and t = sum of loss; the 256 partials are merged by a fixed tree.  No atomics:
+// a row's result is a function of that row's inputs alone, and repeated calls are bit-identical.
+constexpr int SCORE_THREADS = 256;
+
+// (m, s) <- (m, s) merged with (m2, s2); s == 0 marks a partial that has seen no finite term
+__device__ __forceinline__ void lse_merge(double& m, double& s, double m2, double s2) {
+    if (s2 == 0.0) return;
+    if (s == 0.0) { m = m2; s = s2; return; }
+    if (m2 > m) { s = s * exp(m - m2) + s2; m = m2; }
+    else s += s2 * exp(m2 - m);
+}
+
+__global__ void __launch_bounds__(SCORE_THREADS) score_labels_kernel(const float2* __restrict__ pred, int64_t U,
+                                                                     const float2* __restrict__ y, float2* __restrict__ score) {
+    __shared__ double sh_m[SCORE_THREADS], sh_s[SCORE_THREADS], sh_t[SCORE_THREADS];
+    const int64_t n = blockIdx.x;
+    const int tid = threadIdx.x;
+    const float2 yy = y[n];
+    const float2* __restrict__ p = pred + n * U;
+    const double NEG_INF = -__longlong_as_double(0x7ff0000000000000ll);
+    double m = NEG_INF, s = 0.0, t = 0.0;
+    for (int64_t u = tid; u < U; u += SCORE_THREADS) {
+        const float2 ms = p[u];
+        float l0, l1, d0, d1;
+        nll_terms(ms.x, ms.y, yy.x, l0, d0, d1);
+        nll_terms(ms.x, ms.y, yy.y, l1, d0, d1);
+        const float loss = -(l0 + l1);
+        const double v = -(double)loss;
+        t += (double)loss;
+        if (v > m) { s = s * exp(m - v) + 1.0; m = v; }
+        else if (v > NEG_INF) s += exp(v - m);   // -inf only when l0 + l1 overflows fp32: it adds nothing
+    }
+    sh_m[tid] = m; sh_s[tid] = s; sh_t[tid] = t;
+    __syncthreads();
+    for (int w = SCORE_THREADS / 2; w > 0; w >>= 1) {
+        if (tid < w) {
+            lse_merge(m, s, sh_m[tid + w], sh_s[tid + w]);
+            t += sh_t[tid + w];
+            sh_m[tid] = m; sh_s[tid] = s; sh_t[tid] = t;
+        }
+        __syncthreads();
+    }
+    if (tid == 0) {
+        const double lpd = m + (log(s) - log((double)U));   // log((1/U) sum_u exp(-loss[u]))
+        score[n] = make_float2((float)lpd, (float)(t / (double)U));
+    }
+}
+
 }  // namespace bnn
 
 extern "C" {
@@ -396,6 +451,25 @@ int bnn_summarize_instability(const float* d_t, const float* d_pred, int64_t n_s
     }
     summarize_instability_kernel<<<(unsigned)n_systems, threads, smem, (cudaStream_t)stream>>>(
         d_t, (const float2*)d_pred, n_trios, n_units, n_pow2, d_stats);
+    BNN_CUDA(cudaGetLastError());
+    return BNN_OK;
+}
+
+int bnn_score_labels(const float* d_pred, int64_t n_systems, int64_t n_units, const float* d_y, float* d_score,
+                     void* stream) {
+    using namespace bnn;
+    // argument checks first: they need no device
+    BNN_REQUIRE(d_pred && d_y && d_score && n_systems > 0 && n_units > 0, BNN_E_ARG,
+                "bnn_score_labels: null pointer or empty problem");
+    BNN_REQUIRE(n_systems < (1ll << 31) && n_units < (1ll << 32), BNN_E_ARG,
+                "bnn_score_labels: n_systems must be < 2^31 and n_units < 2^32");
+    const auto aligned8 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 7u) == 0; };
+    BNN_REQUIRE(aligned8(d_pred) && aligned8(d_y) && aligned8(d_score), BNN_E_ALIGN,
+                "bnn_score_labels: pointers must be 8-byte aligned");
+    int rc = check_device();
+    if (rc != BNN_OK) return rc;
+    score_labels_kernel<<<(unsigned)n_systems, SCORE_THREADS, 0, (cudaStream_t)stream>>>(
+        (const float2*)d_pred, n_units, (const float2*)d_y, (float2*)d_score);
     BNN_CUDA(cudaGetLastError());
     return BNN_OK;
 }

@@ -427,14 +427,28 @@ class MultiSWAG:
         B200).  Philox draws are keyed on global (unit, row) indices, so the result does not depend on
         either chunking (BASELINE configs[2]: 12,500 systems x 60,000 units per GPU would be 9 GB of predictions and
         4.6 GB of packed weights in one piece; peak here < 1 GB)."""
-        import math
-
         from . import posterior
 
         rows = x.shape[0]
         if rows % n_trios:
             raise ValueError(f"{rows} rows are not a multiple of {n_trios} trios")
-        N = rows // n_trios
+        out = torch.empty((rows // n_trios, 8), device=self.device)
+
+        def consume(lo, hi, row0, pred):
+            out[lo:hi] = posterior.posterior_summary(pred, n_trios, seed, row_offset=row0)
+
+        self._walk_prediction_chunks(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
+                                     consume)
+        return out
+
+    def _walk_prediction_chunks(self, x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes,
+                                unit_chunk, consume):
+        """The chunk walk of ``posterior_summary`` (see there): for each system chunk [lo, hi) of x, the prediction block
+        [(hi - lo) * n_trios, U, 2] of all U units is built and ``consume(lo, hi, row0, pred)`` is called on it (row0: the
+        global index of its first row).  One block exists at a time."""
+        import math
+
+        N = x.shape[0] // n_trios
         U = self.n_models * samples_per_model
         if unit_chunk is None:
             unit_chunk = 16 * torch.cuda.get_device_properties(self.device).multi_processor_count
@@ -447,7 +461,6 @@ class MultiSWAG:
             gs = g // math.gcd(g, n_trios)                      # systems per chunk boundary such that rows stay aligned
             per = max(1, int(max_block_bytes // (12 * U * n_trios)))
             per = max(gs, per // gs * gs)
-            out = torch.empty((N, 8), device=self.device)
             for lo in range(0, N, per):
                 hi = min(lo + per, N)
                 row0 = (system_offset + lo) * n_trios
@@ -462,9 +475,65 @@ class MultiSWAG:
                                                     want_flat=False)
                         self.predict_into(xs, thp, pred, u0, seed, system_offset=row0)
                         del thp
-                out[lo:hi] = posterior.posterior_summary(pred, n_trios, seed, row_offset=row0)
+                consume(lo, hi, row0, pred)
                 del pred
-        return out
+
+    @staticmethod
+    def _check_labelled(x: torch.Tensor, y: torch.Tensor, samples_per_model: int):
+        """Argument checks of ``evaluate``, before any device work."""
+        if x.dim() != 3:
+            raise ValueError(f"x must be [N, T, F], got {tuple(x.shape)}")
+        if y.dim() != 2 or y.shape[1] != 2:
+            raise ValueError(f"y must be [N, 2] (two labels per system), got {tuple(y.shape)}")
+        if y.shape[0] != x.shape[0]:
+            raise ValueError(f"y has {y.shape[0]} rows but x has {x.shape[0]} systems")
+        if int(samples_per_model) < 1:
+            raise ValueError(f"samples_per_model must be >= 1, got {samples_per_model}")
+        _lib.require_cuda(x, "x")
+        _lib.require_cuda(y, "y")
+
+    def evaluate(self, x: torch.Tensor, y: torch.Tensor, samples_per_model: int, seed: int = 0, scale: float = 0.5,
+                 system_offset: int = 0, max_block_bytes: int = 640 << 20, unit_chunk: Optional[int] = None):
+        """Score the ensemble against held-out labels: x [N, T, F] (one trio per system), y [N, 2] -> (summary [N, 8],
+        score [N, 2]).  ``summary`` is exactly ``posterior_summary`` with the same arguments; ``score`` holds per system
+        (``posterior.SCORE_NAMES``) the log predictive density of the label pair under the ensemble, log((1/U) sum_u
+        exp(-loss_u)), and the mean per-unit loss, over the U = n_models * samples_per_model units (``score_labels``;
+        loss_u is the model's own loss, VarModel._lossfnc).  Both come from the same prediction block, one system chunk at
+        a time, so [N, U, 2] never exists beyond one chunk; neither depends on the chunking or on a split into shards
+        with ``system_offset``."""
+        from . import posterior
+
+        self._check_labelled(x, y, samples_per_model)
+        N = x.shape[0]
+        summary = torch.empty((N, 8), device=self.device)
+        score = torch.empty((N, 2), device=self.device)
+
+        def consume(lo, hi, row0, pred):
+            summary[lo:hi] = posterior.posterior_summary(pred, 1, seed, row_offset=row0)
+            score[lo:hi] = posterior.score_labels(pred, y[lo:hi])
+
+        self._walk_prediction_chunks(x, samples_per_model, 1, seed, scale, system_offset, max_block_bytes, unit_chunk,
+                                     consume)
+        return summary, score
+
+    def evaluate_sharded(self, x_local: torch.Tensor, y_local: torch.Tensor, n_total: int, samples_per_model: int,
+                         seed: int = 0, scale: float = 0.5, group=None):
+        """``evaluate`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE all_gather
+        moves [N, 10] (summary | score).  Returns (summary [n_total, 8], score [n_total, 2]) on every rank."""
+        import torch.distributed as dist
+
+        self._check_labelled(x_local, y_local, samples_per_model)
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+        rank = dist.get_rank(group) if dist.is_initialized() else 0
+        granule = self.system_granule(x_local.shape[1])
+        lo, hi = shard_range(n_total, rank, world, granule)
+        if x_local.shape[0] != hi - lo:
+            raise ValueError(f"rank {rank} owns systems [{lo}, {hi}) of {n_total} but was given {x_local.shape[0]}")
+        summary, score = self.evaluate(x_local, y_local, samples_per_model, seed, scale, system_offset=lo)
+        if world == 1:
+            return summary, score
+        full = gather_system_shards(torch.cat([summary, score], 1), n_total, group, granule)
+        return full[:, :8].contiguous(), full[:, 8:].contiguous()
 
     def posterior_summary_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int, n_trios: int = 1,
                                   seed: int = 0, scale: float = 0.5, group=None):

@@ -50,3 +50,29 @@ def summarize_instability(t: torch.Tensor, pred: torch.Tensor, n_trios: int = 1)
 def posterior_summary(pred: torch.Tensor, n_trios: int = 1, seed: int = 0, row_offset: int = 0):
     """[N*n_trios, U, 2] predictions -> [N, 8] summary (sampling + min over trios + order statistics)."""
     return summarize_instability(sample_instability(pred, seed, row_offset), pred, n_trios)
+
+
+SCORE_NAMES = ("lpd", "mean_nll")
+
+
+def score_labels(pred: torch.Tensor, y: torch.Tensor):
+    """pred [N, U, 2] (system-major (mu, std)), y [N, 2] labels -> [N, 2] (SCORE_NAMES): per system, the log of the
+    ensemble's mean likelihood of the label pair, log((1/U) sum_u exp(-loss_u)), and the mean loss, with loss_u the
+    model's own truncated-normal loss (VarModel._lossfnc, ``bnn_nll_fwd_bwd``) of unit u.  Both in nats."""
+    if pred.dim() != 3 or pred.shape[2] != 2:
+        raise ValueError(f"pred must be [N, U, 2], got {tuple(pred.shape)}")
+    N, U = pred.shape[0], pred.shape[1]
+    if tuple(y.shape) != (N, 2):
+        raise ValueError(f"y must be [{N}, 2] (two labels per system), got {tuple(y.shape)}")
+    if U == 0:
+        raise ValueError("pred has no units to score")
+    lib = _lib.load()
+    _lib.require_cuda(pred, "pred")
+    pred, y = pred.contiguous().float(), y.contiguous().float()
+    score = torch.empty((N, 2), device=pred.device, dtype=torch.float32)
+    if N == 0:
+        return score
+    with torch.cuda.device(pred.device), _lib.nvtx("bnn:K7 score_labels"):
+        _lib.check(lib.bnn_score_labels(_lib.ptr(pred), N, U, _lib.dev_ptr(y, pred.device, "y"), _lib.ptr(score),
+                                        _lib.current_stream_ptr()), "bnn_score_labels")
+    return score

@@ -272,6 +272,19 @@ int bnn_sample_instability(const float* d_pred, int64_t n_rows, int64_t n_units,
 int bnn_summarize_instability(const float* d_t, const float* d_pred, int64_t n_systems, int32_t n_trios,
                               int32_t n_units, float* d_stats, void* stream);
 
+/* Held-out score of the ensemble on the same system-major block d_pred [n_systems, U, 2] (one trio per system) against
+ * the labels d_y [n_systems, 2] (the two labels of a system, as bnn_nll_fwd_bwd takes them).  loss[n,u] is
+ * bnn_nll_fwd_bwd's per-system loss of (mu, sd) = d_pred[n,u] and d_y[n] (VarModel._lossfnc, non-finite terms -> 100).
+ * d_score [n_systems, 2]:
+ *   [0] lpd      = log((1/U) sum_u exp(-loss[n,u])), the log predictive density of the label pair in nats;
+ *   [1] mean_nll = (1/U) sum_u loss[n,u].
+ * Both are evaluated in double (lpd as m + log sum_u exp(-loss - m) - log U, m = max_u -loss) and rounded to fp32 once.
+ * A row's result depends on that row's inputs only, through a fixed reduction order: any row slice of a block scores
+ * bit-identically, and repeated calls are bit-identical.  Pointers need only 8-byte alignment, so a slice at any row is
+ * accepted.  BNN_E_ARG: null pointer, n_systems <= 0 or >= 2^31, n_units <= 0 or >= 2^32; checked before the device. */
+int bnn_score_labels(const float* d_pred, int64_t n_systems, int64_t n_units, const float* d_y, float* d_score,
+                     void* stream);
+
 #ifdef __cplusplus
 }
 #endif
