@@ -15,9 +15,14 @@
 // Held-out score of the same block against labels [N, 2]: per system, the log of the ensemble's mean likelihood of the
 // label pair and the mean of the per-unit losses, with the model's own loss (VarModel._lossfnc, loss_device.cuh) as the
 // per-unit term.  [N, U, 2] -> [N, 2].
+//
+// Survival probability per system from the same sampled times: the fraction of the U weight samples whose min over trios
+// exceeds each of J thresholds, P(T_inst > thr_j), counted exactly.  [N*R, U] -> [N, J].
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
+
+#include <algorithm>
 
 #include "common.cuh"
 #include "loss_device.cuh"
@@ -381,6 +386,68 @@ __global__ void __launch_bounds__(SCORE_THREADS) score_labels_kernel(const float
     }
 }
 
+// ---- survival: one CTA per system.  tmin[u] = min over trios of t, fminf from +inf exactly as the summary computes it
+// (a unit whose trio draws are all NaN counts as +inf); bin(u) = number of thresholds strictly below tmin[u], found by a
+// binary search over the ascending thresholds and counted in per-warp shared-memory histograms; then
+// count_j = #{u : bin(u) > j}, a suffix sum.  Integer counts: a row's result depends on that row alone and repeated
+// calls are bit-identical.
+constexpr int SURV_THREADS = 256, SURV_MAXJ = 64, SURV_UNROLL = 4;
+
+struct SurvivalThresholds {   // passed by value in the kernel's parameters
+    float thr[SURV_MAXJ];      // ascending
+    int32_t col[SURV_MAXJ];    // output column of thr[j]
+    int32_t J;
+};
+
+__global__ void __launch_bounds__(SURV_THREADS) survival_kernel(const float* __restrict__ t, int R, int64_t U,
+                                                                const __grid_constant__ SurvivalThresholds th,
+                                                                float* __restrict__ surv) {
+    constexpr int WARPS = SURV_THREADS / 32;
+    __shared__ float s_thr[SURV_MAXJ];
+    __shared__ uint32_t hist[WARPS][SURV_MAXJ + 1], s_tot[SURV_MAXJ + 1];
+    const int tid = threadIdx.x, J = th.J;
+    const float INF = __int_as_float(0x7f800000);
+    if (tid < J) s_thr[tid] = th.thr[tid];
+    for (int i = tid; i < WARPS * (SURV_MAXJ + 1); i += SURV_THREADS) (&hist[0][0])[i] = 0;
+    __syncthreads();
+    const int64_t n = blockIdx.x;
+    const float* __restrict__ rows = t + n * (int64_t)R * U;
+    uint32_t* __restrict__ h = hist[tid >> 5];
+    // whole warps stay in the loop: hist_add_warp is warp-collective
+    for (int64_t u0 = 0; u0 < U; u0 += SURV_THREADS * SURV_UNROLL) {
+        float v[SURV_UNROLL];
+#pragma unroll
+        for (int k = 0; k < SURV_UNROLL; ++k) v[k] = INF;
+        for (int r = 0; r < R; ++r) {   // SURV_UNROLL independent coalesced loads in flight per trio row
+#pragma unroll
+            for (int k = 0; k < SURV_UNROLL; ++k) {
+                const int64_t u = u0 + k * SURV_THREADS + tid;
+                if (u < U) v[k] = fminf(v[k], rows[r * U + u]);
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < SURV_UNROLL; ++k) {
+            int b = 0;   // #{j : thr[j] < v}: the predicate is monotone in j, so the greedy power-of-two steps find it
+#pragma unroll
+            for (int step = SURV_MAXJ; step > 0; step >>= 1)
+                if (b + step <= J && s_thr[b + step - 1] < v[k]) b += step;
+            hist_add_warp(h, (uint32_t)b, u0 + k * SURV_THREADS + tid < U);
+        }
+    }
+    __syncthreads();
+    if (tid <= J) {
+        uint32_t c = 0;
+        for (int w = 0; w < WARPS; ++w) c += hist[w][tid];
+        s_tot[tid] = c;
+    }
+    __syncthreads();
+    if (tid < J) {
+        uint32_t c = 0;   // tmin > thr[tid]  <=>  bin > tid
+        for (int b = tid + 1; b <= J; ++b) c += s_tot[b];
+        surv[n * J + th.col[tid]] = (float)((double)c / (double)U);
+    }
+}
+
 }  // namespace bnn
 
 extern "C" {
@@ -470,6 +537,33 @@ int bnn_score_labels(const float* d_pred, int64_t n_systems, int64_t n_units, co
     if (rc != BNN_OK) return rc;
     score_labels_kernel<<<(unsigned)n_systems, SCORE_THREADS, 0, (cudaStream_t)stream>>>(
         (const float2*)d_pred, n_units, (const float2*)d_y, (float2*)d_score);
+    BNN_CUDA(cudaGetLastError());
+    return BNN_OK;
+}
+
+int bnn_survival_instability(const float* d_t, int64_t n_systems, int32_t n_trios, int64_t n_units,
+                             const float* h_thresholds, int32_t n_thresholds, float* d_surv, void* stream) {
+    using namespace bnn;
+    // argument checks first: they need no device
+    BNN_REQUIRE(d_t && h_thresholds && d_surv && n_systems > 0 && n_units > 0 && n_trios >= 1, BNN_E_ARG,
+                "bnn_survival_instability: null pointer or empty problem");
+    BNN_REQUIRE(n_thresholds >= 1 && n_thresholds <= SURV_MAXJ, BNN_E_ARG,
+                "bnn_survival_instability: n_thresholds must be in [1, %d], got %d", SURV_MAXJ, (int)n_thresholds);
+    BNN_REQUIRE(n_systems < (1ll << 31) && n_units < (1ll << 32), BNN_E_ARG,
+                "bnn_survival_instability: n_systems must be < 2^31 and n_units < 2^32");
+    for (int j = 0; j < n_thresholds; ++j)
+        BNN_REQUIRE(!isnan(h_thresholds[j]), BNN_E_ARG, "bnn_survival_instability: threshold %d is NaN", j);
+    const auto aligned4 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 3u) == 0; };
+    BNN_REQUIRE(aligned4(d_t) && aligned4(d_surv), BNN_E_ALIGN, "bnn_survival_instability: pointers must be 4-byte aligned");
+    SurvivalThresholds th;
+    th.J = n_thresholds;
+    for (int j = 0; j < n_thresholds; ++j) th.col[j] = j;
+    std::stable_sort(th.col, th.col + n_thresholds, [&](int a, int b) { return h_thresholds[a] < h_thresholds[b]; });
+    for (int j = 0; j < n_thresholds; ++j) th.thr[j] = h_thresholds[th.col[j]];
+    for (int j = n_thresholds; j < SURV_MAXJ; ++j) { th.thr[j] = 0.f; th.col[j] = 0; }
+    int rc = check_device();
+    if (rc != BNN_OK) return rc;
+    survival_kernel<<<(unsigned)n_systems, SURV_THREADS, 0, (cudaStream_t)stream>>>(d_t, n_trios, n_units, th, d_surv);
     BNN_CUDA(cudaGetLastError());
     return BNN_OK;
 }

@@ -6,7 +6,14 @@ for every labelled system and reduces on the device (``MultiSWAG.evaluate``): pe
 under the ensemble and mean per-unit loss, in nats).  Writes ``metrics.json`` (means over systems) and
 ``per_system.npz`` (summary, score) to ``--out``.
 
+``--survival T [T ...]`` (log10 orbits) adds, from the same walk over the predictions, the survival probability
+P(T_inst > T) per system (``MultiSWAG.posterior_survival``): ``survival`` [N, J] and ``thresholds`` in the npz,
+``survival_mean`` in the metrics, and when 9 is among the thresholds the Brier score of the stable-past-1e9-orbits
+prediction against the labels, ``brier_stable`` = mean over every finite label y of (S(9) - [y >= 9])^2, with
+``n_stable_labels`` the number of those labels that are >= 9 (the loss's censored branch).
+
     python -m bnn_chaos_model_b200.evaluate --models DIR/*_output.pkl --samples 100 --out EVAL_DIR
+    python -m bnn_chaos_model_b200.evaluate --models DIR/*_output.pkl --survival 6 9 --out EVAL_DIR
     python -m torch.distributed.run --nproc-per-node 8 -m bnn_chaos_model_b200.evaluate --models ... --out EVAL_DIR
 
 Labelled data: ``--data file.npz`` with X_val, y_val in run_swag's format (already normalised), or by default the
@@ -35,7 +42,20 @@ def build_parser():
     ap.add_argument("--seed", type=int, default=0, help="Philox seed of the weight and summary-statistic draws")
     ap.add_argument("--scale", type=float, default=0.5, help="SWAG sampling scale")
     ap.add_argument("--out", required=True, help="directory for metrics.json and per_system.npz")
+    ap.add_argument("--survival", type=float, nargs="+", default=None, metavar="T",
+                    help="also estimate P(T_inst > T) per system for these log10 instability times (1 to 64 values)")
     return ap
+
+
+def brier_stable(s9, y):
+    """(mean over every finite label of (s9 - [label >= 9])^2, number of those labels that are >= 9); s9 [N], y [N, 2].
+    The mean is None when no label is finite."""
+    y = np.asarray(y, np.float64)
+    finite = np.isfinite(y)
+    stable = (y >= 9.0).astype(np.float64)
+    sq = (np.asarray(s9, np.float64)[:, None] - stable) ** 2
+    n = int(finite.sum())
+    return (float(sq[finite].mean()) if n else None), int((finite & (y >= 9.0)).sum())
 
 
 def load_labelled(args):
@@ -54,9 +74,11 @@ def main(argv=None):
     import torch.distributed as dist
 
     from .multiswag import load_ensemble, shard_range
-    from .posterior import SCORE_NAMES, STAT_NAMES
+    from .posterior import SCORE_NAMES, STAT_NAMES, survival_thresholds
 
     args = build_parser().parse_args(argv)
+    if args.survival is not None:
+        survival_thresholds(args.survival)   # bad thresholds fail before any device work
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local_rank)
@@ -66,14 +88,16 @@ def main(argv=None):
     X, y = load_labelled(args)
     ens = load_ensemble(args.models, device=dev)
     N = X.shape[0]
+    # summary, score and (with --survival) survival come from one walk over the prediction block
     if world > 1:
         lo, hi = shard_range(N, dist.get_rank(), world, ens.system_granule(X.shape[1]))
-        summary, score = ens.evaluate_sharded(X[lo:hi].to(dev), y[lo:hi].to(dev), N, args.samples, args.seed, args.scale)
+        outs = ens._reduce_sharded(X[lo:hi].to(dev), N, args.samples, 1, args.seed, args.scale,
+                                   y=y[lo:hi].to(dev), thresholds=args.survival)
     else:
-        summary, score = ens.evaluate(X.to(dev), y.to(dev), args.samples, args.seed, args.scale)
+        outs = ens._reduce(X.to(dev), args.samples, 1, args.seed, args.scale, y=y.to(dev), thresholds=args.survival)
     metrics = None
     if world == 1 or dist.get_rank() == 0:
-        summary, score = summary.cpu().numpy(), score.cpu().numpy()
+        summary, score = outs[0].cpu().numpy(), outs[1].cpu().numpy()
         lpd_mean = float(score[:, 0].astype(np.float64).mean())
         metrics = {"n_systems": int(N), "n_units": ens.n_models * args.samples, "n_models": ens.n_models,
                    "samples_per_model": args.samples, "seed": args.seed, "scale": args.scale,
@@ -81,13 +105,21 @@ def main(argv=None):
                    "mean_nll": float(score[:, 1].astype(np.float64).mean()),
                    "data": args.data or f"synthetic({args.synthetic}, seed={VAL_SEED})",
                    "device": torch.cuda.get_device_name(dev)}
+        arrays = dict(summary=summary, score=score, stat_names=np.array(STAT_NAMES), score_names=np.array(SCORE_NAMES))
+        if args.survival is not None:
+            surv = outs[2].cpu().numpy()
+            arrays.update(survival=surv, thresholds=survival_thresholds(args.survival))
+            metrics["survival_mean"] = [float(v) for v in surv.astype(np.float64).mean(0)]
+            if 9.0 in args.survival:
+                metrics["brier_stable"], metrics["n_stable_labels"] = brier_stable(surv[:, args.survival.index(9.0)],
+                                                                                   y.numpy())
         os.makedirs(args.out, exist_ok=True)
         with open(os.path.join(args.out, "metrics.json"), "w") as f:
             json.dump(metrics, f, indent=1)
-        np.savez(os.path.join(args.out, "per_system.npz"), summary=summary, score=score,
-                 stat_names=np.array(STAT_NAMES), score_names=np.array(SCORE_NAMES))
-        print(f"{N} systems x {metrics['n_units']} units: lpd_mean {lpd_mean:.6f}, mean_nll {metrics['mean_nll']:.6f}; "
-              f"wrote {args.out}/metrics.json and per_system.npz")
+        np.savez(os.path.join(args.out, "per_system.npz"), **arrays)
+        print(f"{N} systems x {metrics['n_units']} units: lpd_mean {lpd_mean:.6f}, mean_nll {metrics['mean_nll']:.6f}"
+              + (f", brier_stable {metrics['brier_stable']}" if "brier_stable" in metrics else "")
+              + f"; wrote {args.out}/metrics.json and per_system.npz")
     if world > 1:
         dist.destroy_process_group()
     return metrics

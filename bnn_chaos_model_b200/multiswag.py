@@ -492,6 +492,76 @@ class MultiSWAG:
         _lib.require_cuda(x, "x")
         _lib.require_cuda(y, "y")
 
+    @staticmethod
+    def _check_reduce(x: torch.Tensor, samples_per_model: int, n_trios: int, y=None, thresholds=None):
+        """Argument checks of ``_reduce`` / ``_reduce_sharded``, before any device work.  Returns the thresholds as
+        ``posterior.survival_thresholds`` (or None)."""
+        from . import posterior
+
+        if y is not None:
+            MultiSWAG._check_labelled(x, y, samples_per_model)
+        if thresholds is None:
+            return None
+        if x.dim() != 3:
+            raise ValueError(f"x must be [N*n_trios, T, F], got {tuple(x.shape)}")
+        if int(n_trios) < 1 or x.shape[0] % n_trios:
+            raise ValueError(f"{x.shape[0]} rows are not a multiple of {n_trios} trios")
+        if int(samples_per_model) < 1:
+            raise ValueError(f"samples_per_model must be >= 1, got {samples_per_model}")
+        thr = posterior.survival_thresholds(thresholds)
+        _lib.require_cuda(x, "x")
+        return thr
+
+    def _reduce(self, x, samples_per_model, n_trios=1, seed=0, scale=0.5, system_offset=0, max_block_bytes=640 << 20,
+                unit_chunk=None, y=None, thresholds=None):
+        """One walk over the prediction block (``_walk_prediction_chunks``) that reduces every system chunk on the device
+        and returns [summary [N, 8]] + [score [N, 2]] if labels y are given + [survival [N, J]] if thresholds are given.
+        Each chunk's instability times are sampled once and feed both the summary and the survival counts."""
+        from . import posterior
+
+        thr = self._check_reduce(x, samples_per_model, n_trios, y, thresholds)
+        N = x.shape[0] // n_trios
+        outs = [torch.empty((N, 8), device=self.device)]
+        if y is not None:
+            outs.append(torch.empty((N, 2), device=self.device))
+        if thr is not None:
+            outs.append(torch.empty((N, thr.size), device=self.device))
+
+        def consume(lo, hi, row0, pred):
+            t = posterior.sample_instability(pred, seed, row_offset=row0)
+            outs[0][lo:hi] = posterior.summarize_instability(t, pred, n_trios)
+            if y is not None:
+                outs[1][lo:hi] = posterior.score_labels(pred, y[lo:hi])
+            if thr is not None:
+                outs[-1][lo:hi] = posterior.survival(t, thr, n_trios)
+
+        self._walk_prediction_chunks(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
+                                     consume)
+        return outs
+
+    def _reduce_sharded(self, x_local, n_total, samples_per_model, n_trios=1, seed=0, scale=0.5, group=None, y=None,
+                        thresholds=None):
+        """``_reduce`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE all_gather
+        moves the concatenated columns [N, 8 (+ 2) (+ J)].  Returns the same list, [n_total, ...] each, on every rank."""
+        import math
+
+        import torch.distributed as dist
+
+        self._check_reduce(x_local, samples_per_model, n_trios, y, thresholds)
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+        rank = dist.get_rank(group) if dist.is_initialized() else 0
+        g = self.system_granule(x_local.shape[1])
+        granule = g // math.gcd(g, n_trios)  # shard boundaries in SYSTEMS such that rows stay granule-aligned
+        lo, hi = shard_range(n_total, rank, world, granule)
+        if x_local.shape[0] != (hi - lo) * n_trios:
+            raise ValueError(f"rank {rank} owns systems [{lo}, {hi}) of {n_total} but was given "
+                             f"{x_local.shape[0]} rows of {n_trios} trios")
+        outs = self._reduce(x_local, samples_per_model, n_trios, seed, scale, system_offset=lo, y=y, thresholds=thresholds)
+        if world == 1:
+            return outs
+        full = gather_system_shards(torch.cat(outs, 1), n_total, group, granule)
+        return [c.contiguous() for c in torch.split(full, [o.shape[1] for o in outs], 1)]
+
     def evaluate(self, x: torch.Tensor, y: torch.Tensor, samples_per_model: int, seed: int = 0, scale: float = 0.5,
                  system_offset: int = 0, max_block_bytes: int = 640 << 20, unit_chunk: Optional[int] = None):
         """Score the ensemble against held-out labels: x [N, T, F] (one trio per system), y [N, 2] -> (summary [N, 8],
@@ -501,39 +571,39 @@ class MultiSWAG:
         loss_u is the model's own loss, VarModel._lossfnc).  Both come from the same prediction block, one system chunk at
         a time, so [N, U, 2] never exists beyond one chunk; neither depends on the chunking or on a split into shards
         with ``system_offset``."""
-        from . import posterior
-
-        self._check_labelled(x, y, samples_per_model)
-        N = x.shape[0]
-        summary = torch.empty((N, 8), device=self.device)
-        score = torch.empty((N, 2), device=self.device)
-
-        def consume(lo, hi, row0, pred):
-            summary[lo:hi] = posterior.posterior_summary(pred, 1, seed, row_offset=row0)
-            score[lo:hi] = posterior.score_labels(pred, y[lo:hi])
-
-        self._walk_prediction_chunks(x, samples_per_model, 1, seed, scale, system_offset, max_block_bytes, unit_chunk,
-                                     consume)
+        summary, score = self._reduce(x, samples_per_model, 1, seed, scale, system_offset, max_block_bytes, unit_chunk, y=y)
         return summary, score
 
     def evaluate_sharded(self, x_local: torch.Tensor, y_local: torch.Tensor, n_total: int, samples_per_model: int,
                          seed: int = 0, scale: float = 0.5, group=None):
         """``evaluate`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE all_gather
         moves [N, 10] (summary | score).  Returns (summary [n_total, 8], score [n_total, 2]) on every rank."""
-        import torch.distributed as dist
+        summary, score = self._reduce_sharded(x_local, n_total, samples_per_model, 1, seed, scale, group, y=y_local)
+        return summary, score
 
-        self._check_labelled(x_local, y_local, samples_per_model)
-        world = dist.get_world_size(group) if dist.is_initialized() else 1
-        rank = dist.get_rank(group) if dist.is_initialized() else 0
-        granule = self.system_granule(x_local.shape[1])
-        lo, hi = shard_range(n_total, rank, world, granule)
-        if x_local.shape[0] != hi - lo:
-            raise ValueError(f"rank {rank} owns systems [{lo}, {hi}) of {n_total} but was given {x_local.shape[0]}")
-        summary, score = self.evaluate(x_local, y_local, samples_per_model, seed, scale, system_offset=lo)
-        if world == 1:
-            return summary, score
-        full = gather_system_shards(torch.cat([summary, score], 1), n_total, group, granule)
-        return full[:, :8].contiguous(), full[:, 8:].contiguous()
+    def posterior_survival(self, x: torch.Tensor, thresholds, samples_per_model: int, n_trios: int = 1, seed: int = 0,
+                           scale: float = 0.5, system_offset: int = 0, max_block_bytes: int = 640 << 20,
+                           unit_chunk: Optional[int] = None):
+        """Survival probability per system: x [N*n_trios, T, F] (as ``posterior_summary``), thresholds [J] (1 to 64 log10
+        instability times, e.g. 9 = stable past 1e9 orbits) -> (summary [N, 8], survival [N, J]).  ``summary`` is exactly
+        ``posterior_summary`` with the same arguments; survival[n, j] = S_j is the fraction of the U = n_models *
+        samples_per_model sampled instability times of system n (min over trios) that exceed thresholds[j] strictly
+        (``posterior.survival``).  S_j is a Monte Carlo estimate of P(T_inst > thresholds[j]) with standard error
+        sqrt(S_j (1 - S_j) / U), and it counts the very draws the summary's percentiles come from: each system chunk's
+        times are sampled once and feed both, so the predictive kernel runs once.  Neither output depends on the
+        chunking or on a split into shards with ``system_offset``."""
+        summary, surv = self._reduce(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
+                                     thresholds=thresholds)
+        return summary, surv
+
+    def posterior_survival_sharded(self, x_local: torch.Tensor, thresholds, n_total: int, samples_per_model: int,
+                                   n_trios: int = 1, seed: int = 0, scale: float = 0.5, group=None):
+        """``posterior_survival`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE
+        all_gather moves [N, 8 + J] (summary | survival).  Returns (summary [n_total, 8], survival [n_total, J]) on every
+        rank."""
+        summary, surv = self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale, group,
+                                             thresholds=thresholds)
+        return summary, surv
 
     def posterior_summary_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int, n_trios: int = 1,
                                   seed: int = 0, scale: float = 0.5, group=None):

@@ -3,10 +3,14 @@
 Replaces the host-side numpy tail of the reference's evaluation scripts -- ``fast_truncnorm`` (left = 4),
 resampling of draws >= 9 from the analytic prior, min over trios, per-system median / percentiles
 (figures/main_figures.py:167-277, figures/multiswag_5_planet.py:306-481) -- so that only ``[N, 8]`` leaves the
-device instead of the ``[N, U, 2]`` prediction block.
+device instead of the ``[N, U, 2]`` prediction block.  ``survival`` counts the same sampled times against thresholds:
+P(T_inst > t) per system.
 """
 from __future__ import annotations
 
+import ctypes
+
+import numpy as np
 import torch
 
 from . import _lib
@@ -76,3 +80,46 @@ def score_labels(pred: torch.Tensor, y: torch.Tensor):
         _lib.check(lib.bnn_score_labels(_lib.ptr(pred), N, U, _lib.dev_ptr(y, pred.device, "y"), _lib.ptr(score),
                                         _lib.current_stream_ptr()), "bnn_score_labels")
     return score
+
+
+MAX_THRESHOLDS = 64
+
+
+def survival_thresholds(thresholds) -> np.ndarray:
+    """The thresholds of ``survival`` as the kernel compares them: a float32 array of 1 to 64 values, none NaN (+-inf
+    allowed).  Raises ValueError otherwise."""
+    thr = np.array([float(v) for v in thresholds], np.float32)
+    if not 1 <= thr.size <= MAX_THRESHOLDS:
+        raise ValueError(f"between 1 and {MAX_THRESHOLDS} thresholds are needed, got {thr.size}")
+    if np.isnan(thr).any():
+        raise ValueError(f"thresholds must not be NaN, got {thr.tolist()}")
+    return thr
+
+
+def survival(t: torch.Tensor, thresholds, n_trios: int = 1):
+    """t [N*n_trios, U] sampled log10 instability times (``sample_instability``), thresholds [J] (log10 orbits, host
+    values, rounded to fp32) -> [N, J]: the fraction of the U weight samples whose min over trios exceeds each
+    threshold, S_j = #{u : min_r t > thr_j} / U.  S_j is a Monte Carlo estimate of P(T_inst > thr_j) with standard error
+    sqrt(S_j (1 - S_j) / U); it counts the same draws as ``summarize_instability``'s percentiles."""
+    if t.dim() != 2:
+        raise ValueError(f"t must be [N*n_trios, U], got {tuple(t.shape)}")
+    if int(n_trios) < 1:
+        raise ValueError(f"n_trios must be >= 1, got {n_trios}")
+    rows, U = t.shape
+    if rows % n_trios:
+        raise ValueError(f"{rows} rows are not a multiple of {n_trios} trios")
+    if U == 0:
+        raise ValueError("t has no units to count")
+    thr = survival_thresholds(thresholds)
+    lib = _lib.load()
+    _lib.require_cuda(t, "t")
+    t = t.contiguous().float()
+    N = rows // n_trios
+    surv = torch.empty((N, thr.size), device=t.device, dtype=torch.float32)
+    if N == 0:
+        return surv
+    h_thr = (ctypes.c_float * thr.size)(*thr.tolist())
+    with torch.cuda.device(t.device), _lib.nvtx("bnn:K7 survival_instability"):
+        _lib.check(lib.bnn_survival_instability(_lib.ptr(t), N, int(n_trios), U, h_thr, thr.size, _lib.ptr(surv),
+                                                _lib.current_stream_ptr()), "bnn_survival_instability")
+    return surv

@@ -285,6 +285,20 @@ int bnn_summarize_instability(const float* d_t, const float* d_pred, int64_t n_s
 int bnn_score_labels(const float* d_pred, int64_t n_systems, int64_t n_units, const float* d_y, float* d_score,
                      void* stream);
 
+/* Survival probability per system from the sampled times d_t [n_systems * n_trios, U] that bnn_sample_instability
+ * writes (row = system * n_trios + trio).  tmin[n,u] is the min over trios exactly as bnn_summarize_instability takes
+ * it: fminf from +inf, so a unit whose trio draws are all NaN counts as +inf.  For the J = n_thresholds host values
+ * h_thresholds (log10 orbits, any order, duplicates and +-inf allowed):
+ *   d_surv [n_systems, J]:  surv[n,j] = #{u : tmin[n,u] > h_thresholds[j]} / U   (strict comparison),
+ * the count exact, converted once as (float)((double)count / U).  It is a Monte Carlo estimate of P(T_inst > thr) with
+ * standard error sqrt(S (1 - S) / U), from the same draws as the summary's percentiles.  The thresholds travel in the
+ * kernel's parameters (no device copy).  A row's result depends on that row only, and repeated calls are bit-identical.
+ * d_t and d_surv need only 4-byte alignment, so a row slice at any offset is accepted.  BNN_E_ARG: null pointer,
+ * n_systems <= 0 or >= 2^31, n_units <= 0 or >= 2^32, n_trios < 1, n_thresholds outside [1, 64], a NaN threshold;
+ * checked before the device. */
+int bnn_survival_instability(const float* d_t, int64_t n_systems, int32_t n_trios, int64_t n_units,
+                             const float* h_thresholds, int32_t n_thresholds, float* d_surv, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
