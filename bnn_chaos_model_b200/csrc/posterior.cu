@@ -18,6 +18,10 @@
 //
 // Survival probability per system from the same sampled times: the fraction of the U weight samples whose min over trios
 // exceeds each of J thresholds, P(T_inst > thr_j), counted exactly.  [N*R, U] -> [N, J].
+//
+// Variance decomposition of each prediction row of the block: the ensemble's mean mu, the aleatoric part (mean sigma^2),
+// and the epistemic part (variance of mu over the units) split into between-model and within-model parts.
+// [rows, U, 2] -> [rows, 5].
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -448,6 +452,115 @@ __global__ void __launch_bounds__(SURV_THREADS) survival_kernel(const float* __r
     }
 }
 
+// ---- variance decomposition: one CTA per prediction row, unit u = k*S + s of model k.  Pass 1: the units of a warp's
+// 32 lanes are consecutive, so their model indices are sorted and form a few contiguous segments; a segmented shuffle
+// scan sums each segment and its last lane adds the sum to the warp's own accumulator acc[warp][k] in shared memory.
+// The model sums are then the sums over warps in warp order.  Pass 2 re-reads the row for (mu - m_k)^2 against the model
+// means.  Everything accumulates in double in a fixed order with no atomics: a row's result depends on that row alone.
+constexpr int UNC_THREADS = 256, UNC_WARPS = UNC_THREADS / 32, UNC_UNROLL = 4, UNC_MAXM = 1024;
+
+// sum over the CTA, the same bits in every thread: xor butterfly (commutative pairs, so every lane agrees) + warp order
+__device__ __forceinline__ double block_sum_d(double v, double* red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    __syncthreads();   // red may still be read by the previous call
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    double s = 0.0;
+#pragma unroll
+    for (int w = 0; w < UNC_WARPS; ++w) s += red[w];
+    return s;
+}
+
+__global__ void __launch_bounds__(UNC_THREADS) uncertainty_kernel(const float2* __restrict__ pred, int64_t U, uint32_t S,
+                                                                  int M, float* __restrict__ out) {
+    extern __shared__ double acc[];   // [UNC_WARPS][M] per-warp model sums of mu; then acc[k] = m_k
+    __shared__ double red[UNC_WARPS];
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int64_t row = blockIdx.x;
+    const float2* __restrict__ p = pred + row * U;
+    for (int i = tid; i < UNC_WARPS * M; i += UNC_THREADS) acc[i] = 0.0;
+    __syncthreads();
+    double* __restrict__ mine = acc + (tid >> 5) * M;
+    double sd2 = 0.0;
+    bool bad_mu = false, bad_sd = false;
+    // pass 1: model sums of mu, sum of sigma^2.  Whole warps stay in the loop: the scan is warp-collective.
+    for (int64_t u0 = 0; u0 < U; u0 += UNC_THREADS * UNC_UNROLL) {
+        float2 v[UNC_UNROLL];
+#pragma unroll
+        for (int k = 0; k < UNC_UNROLL; ++k) {   // UNC_UNROLL independent coalesced loads in flight
+            const int64_t u = u0 + k * UNC_THREADS + tid;
+            v[k] = u < U ? p[u] : make_float2(0.f, 0.f);
+        }
+#pragma unroll
+        for (int k = 0; k < UNC_UNROLL; ++k) {
+            const int64_t u = u0 + k * UNC_THREADS + tid;
+            const bool valid = u < U;
+            bad_mu |= !isfinite(v[k].x);
+            bad_sd |= !isfinite(v[k].y);
+            sd2 += (double)v[k].y * (double)v[k].y;
+            const uint32_t model = valid ? (uint32_t)u / S : (uint32_t)M;
+            const uint32_t peers = __match_any_sync(0xffffffffu, model);
+            const int first = __ffs(peers) - 1;
+            double s = (double)v[k].x;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const double up = __shfl_up_sync(0xffffffffu, s, d);
+                if (lane - d >= first) s += up;
+            }
+            if (valid && lane == 31 - __clz(peers)) mine[model] += s;
+            __syncwarp();   // the next segment's lane may update the same entry
+        }
+    }
+    __syncthreads();
+    // model means m_k, their mean, and the between-model moment
+    double part = 0.0;
+    for (int k = tid; k < M; k += UNC_THREADS) {
+        double s = 0.0;
+        for (int w = 0; w < UNC_WARPS; ++w) s += acc[w * M + k];
+        const double m = s / (double)S;
+        acc[k] = m;   // column k is read by this thread only
+        part += m;
+    }
+    const double mean = block_sum_d(part, red) / (double)M;   // its barriers publish acc[k]
+    part = 0.0;
+    for (int k = tid; k < M; k += UNC_THREADS) {
+        const double d = acc[k] - mean;
+        part += d * d;
+    }
+    const double between = block_sum_d(part, red) / (double)M;
+    // pass 2: within-model moment (1/M) sum_k (1/S) sum_s (mu - m_k)^2 = (1/U) sum_u (mu_u - m_k(u))^2
+    part = 0.0;
+    for (int64_t u0 = 0; u0 < U; u0 += UNC_THREADS * UNC_UNROLL) {
+        float mu[UNC_UNROLL];
+#pragma unroll
+        for (int k = 0; k < UNC_UNROLL; ++k) {
+            const int64_t u = u0 + k * UNC_THREADS + tid;
+            mu[k] = u < U ? p[u].x : 0.f;
+        }
+#pragma unroll
+        for (int k = 0; k < UNC_UNROLL; ++k) {
+            const int64_t u = u0 + k * UNC_THREADS + tid;
+            if (u < U) {
+                const double d = (double)mu[k] - acc[(uint32_t)u / S];
+                part += d * d;
+            }
+        }
+    }
+    const double within = block_sum_d(part, red) / (double)U;
+    const double aleatoric = block_sum_d(sd2, red) / (double)U;
+    const int nonfinite_mu = __syncthreads_or(bad_mu), nonfinite_sd = __syncthreads_or(bad_sd);
+    if (tid == 0) {
+        const float NaN = __int_as_float(0x7fffffff);
+        float* o = out + row * 5;
+        o[0] = nonfinite_mu ? NaN : (float)mean;
+        o[1] = nonfinite_sd ? NaN : (float)aleatoric;
+        o[2] = nonfinite_mu ? NaN : (float)(between + within);
+        o[3] = nonfinite_mu ? NaN : (float)between;
+        o[4] = nonfinite_mu ? NaN : (float)within;
+    }
+}
+
 }  // namespace bnn
 
 extern "C" {
@@ -564,6 +677,36 @@ int bnn_survival_instability(const float* d_t, int64_t n_systems, int32_t n_trio
     int rc = check_device();
     if (rc != BNN_OK) return rc;
     survival_kernel<<<(unsigned)n_systems, SURV_THREADS, 0, (cudaStream_t)stream>>>(d_t, n_trios, n_units, th, d_surv);
+    BNN_CUDA(cudaGetLastError());
+    return BNN_OK;
+}
+
+int bnn_decompose_uncertainty(const float* d_pred, int64_t n_rows, int64_t n_units, int64_t units_per_model,
+                              float* d_out, void* stream) {
+    using namespace bnn;
+    // argument checks first: they need no device
+    BNN_REQUIRE(d_pred && d_out && n_rows > 0 && n_units > 0, BNN_E_ARG,
+                "bnn_decompose_uncertainty: null pointer or empty problem");
+    BNN_REQUIRE(n_rows < (1ll << 31) && n_units < (1ll << 32), BNN_E_ARG,
+                "bnn_decompose_uncertainty: n_rows must be < 2^31 and n_units < 2^32");
+    BNN_REQUIRE(units_per_model >= 1 && n_units % units_per_model == 0, BNN_E_ARG,
+                "bnn_decompose_uncertainty: n_units (%lld) must be a positive multiple of units_per_model (%lld)",
+                (long long)n_units, (long long)units_per_model);
+    const int64_t n_models = n_units / units_per_model;
+    BNN_REQUIRE(n_models <= UNC_MAXM, BNN_E_ARG, "bnn_decompose_uncertainty: %lld models, at most %d supported",
+                (long long)n_models, UNC_MAXM);
+    BNN_REQUIRE((reinterpret_cast<uintptr_t>(d_pred) & 7u) == 0 && (reinterpret_cast<uintptr_t>(d_out) & 3u) == 0,
+                BNN_E_ALIGN, "bnn_decompose_uncertainty: d_pred must be 8-byte and d_out 4-byte aligned");
+    int rc = check_device();
+    if (rc != BNN_OK) return rc;
+    static PerDeviceOnce attr_done;
+    if (attr_done.need()) {
+        BNN_CUDA(cudaFuncSetAttribute(uncertainty_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)(UNC_WARPS * UNC_MAXM * sizeof(double))));
+    }
+    const size_t smem = (size_t)UNC_WARPS * n_models * sizeof(double);
+    uncertainty_kernel<<<(unsigned)n_rows, UNC_THREADS, smem, (cudaStream_t)stream>>>(
+        (const float2*)d_pred, n_units, (uint32_t)units_per_model, (int)n_models, d_out);
     BNN_CUDA(cudaGetLastError());
     return BNN_OK;
 }

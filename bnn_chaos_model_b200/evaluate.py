@@ -12,8 +12,13 @@ P(T_inst > T) per system (``MultiSWAG.posterior_survival``): ``survival`` [N, J]
 prediction against the labels, ``brier_stable`` = mean over every finite label y of (S(9) - [y >= 9])^2, with
 ``n_stable_labels`` the number of those labels that are >= 9 (the loss's censored branch).
 
+``--uncertainty`` adds, from the same walk, each system's predictive variance split into its aleatoric, between-model
+and within-model parts (``MultiSWAG.posterior_uncertainty``): ``uncertainty`` [N, 5] and ``uncertainty_names`` in the
+npz, ``uncertainty_mean`` (the mean over systems of each column) in the metrics.
+
     python -m bnn_chaos_model_b200.evaluate --models DIR/*_output.pkl --samples 100 --out EVAL_DIR
     python -m bnn_chaos_model_b200.evaluate --models DIR/*_output.pkl --survival 6 9 --out EVAL_DIR
+    python -m bnn_chaos_model_b200.evaluate --models DIR/*_output.pkl --uncertainty --out EVAL_DIR
     python -m torch.distributed.run --nproc-per-node 8 -m bnn_chaos_model_b200.evaluate --models ... --out EVAL_DIR
 
 Labelled data: ``--data file.npz`` with X_val, y_val in run_swag's format (already normalised), or by default the
@@ -44,6 +49,9 @@ def build_parser():
     ap.add_argument("--out", required=True, help="directory for metrics.json and per_system.npz")
     ap.add_argument("--survival", type=float, nargs="+", default=None, metavar="T",
                     help="also estimate P(T_inst > T) per system for these log10 instability times (1 to 64 values)")
+    ap.add_argument("--uncertainty", action="store_true",
+                    help="also split each system's predictive variance into aleatoric, between-model and within-model "
+                         "parts")
     return ap
 
 
@@ -74,7 +82,7 @@ def main(argv=None):
     import torch.distributed as dist
 
     from .multiswag import load_ensemble, shard_range
-    from .posterior import SCORE_NAMES, STAT_NAMES, survival_thresholds
+    from .posterior import SCORE_NAMES, STAT_NAMES, UNCERTAINTY_NAMES, survival_thresholds
 
     args = build_parser().parse_args(argv)
     if args.survival is not None:
@@ -88,13 +96,15 @@ def main(argv=None):
     X, y = load_labelled(args)
     ens = load_ensemble(args.models, device=dev)
     N = X.shape[0]
-    # summary, score and (with --survival) survival come from one walk over the prediction block
+    # summary, score, (with --survival) survival and (with --uncertainty) uncertainty come from one walk over the
+    # prediction block, in that order
     if world > 1:
         lo, hi = shard_range(N, dist.get_rank(), world, ens.system_granule(X.shape[1]))
         outs = ens._reduce_sharded(X[lo:hi].to(dev), N, args.samples, 1, args.seed, args.scale,
-                                   y=y[lo:hi].to(dev), thresholds=args.survival)
+                                   y=y[lo:hi].to(dev), thresholds=args.survival, uncertainty=args.uncertainty)
     else:
-        outs = ens._reduce(X.to(dev), args.samples, 1, args.seed, args.scale, y=y.to(dev), thresholds=args.survival)
+        outs = ens._reduce(X.to(dev), args.samples, 1, args.seed, args.scale, y=y.to(dev), thresholds=args.survival,
+                           uncertainty=args.uncertainty)
     metrics = None
     if world == 1 or dist.get_rank() == 0:
         summary, score = outs[0].cpu().numpy(), outs[1].cpu().numpy()
@@ -113,6 +123,10 @@ def main(argv=None):
             if 9.0 in args.survival:
                 metrics["brier_stable"], metrics["n_stable_labels"] = brier_stable(surv[:, args.survival.index(9.0)],
                                                                                    y.numpy())
+        if args.uncertainty:
+            unc = outs[3 if args.survival is not None else 2].cpu().numpy()[:, 0]   # one trio per system
+            arrays.update(uncertainty=unc, uncertainty_names=np.array(UNCERTAINTY_NAMES))
+            metrics["uncertainty_mean"] = [float(v) for v in unc.astype(np.float64).mean(0)]
         os.makedirs(args.out, exist_ok=True)
         with open(os.path.join(args.out, "metrics.json"), "w") as f:
             json.dump(metrics, f, indent=1)

@@ -493,14 +493,15 @@ class MultiSWAG:
         _lib.require_cuda(y, "y")
 
     @staticmethod
-    def _check_reduce(x: torch.Tensor, samples_per_model: int, n_trios: int, y=None, thresholds=None):
+    def _check_reduce(x: torch.Tensor, samples_per_model: int, n_trios: int, y=None, thresholds=None,
+                      uncertainty=False):
         """Argument checks of ``_reduce`` / ``_reduce_sharded``, before any device work.  Returns the thresholds as
         ``posterior.survival_thresholds`` (or None)."""
         from . import posterior
 
         if y is not None:
             MultiSWAG._check_labelled(x, y, samples_per_model)
-        if thresholds is None:
+        if thresholds is None and not uncertainty:
             return None
         if x.dim() != 3:
             raise ValueError(f"x must be [N*n_trios, T, F], got {tuple(x.shape)}")
@@ -508,46 +509,56 @@ class MultiSWAG:
             raise ValueError(f"{x.shape[0]} rows are not a multiple of {n_trios} trios")
         if int(samples_per_model) < 1:
             raise ValueError(f"samples_per_model must be >= 1, got {samples_per_model}")
-        thr = posterior.survival_thresholds(thresholds)
+        thr = posterior.survival_thresholds(thresholds) if thresholds is not None else None
         _lib.require_cuda(x, "x")
         return thr
 
     def _reduce(self, x, samples_per_model, n_trios=1, seed=0, scale=0.5, system_offset=0, max_block_bytes=640 << 20,
-                unit_chunk=None, y=None, thresholds=None):
+                unit_chunk=None, y=None, thresholds=None, uncertainty=False):
         """One walk over the prediction block (``_walk_prediction_chunks``) that reduces every system chunk on the device
-        and returns [summary [N, 8]] + [score [N, 2]] if labels y are given + [survival [N, J]] if thresholds are given.
-        Each chunk's instability times are sampled once and feed both the summary and the survival counts."""
+        and returns [summary [N, 8]] + [score [N, 2]] if labels y are given + [survival [N, J]] if thresholds are given
+        + [uncertainty [N, n_trios, 5]] if ``uncertainty`` is set.  Each chunk's instability times are sampled once and
+        feed both the summary and the survival counts; the uncertainty decomposes the same prediction block."""
         from . import posterior
 
-        thr = self._check_reduce(x, samples_per_model, n_trios, y, thresholds)
+        thr = self._check_reduce(x, samples_per_model, n_trios, y, thresholds, uncertainty)
         N = x.shape[0] // n_trios
         outs = [torch.empty((N, 8), device=self.device)]
+        i_score = i_surv = i_unc = None
         if y is not None:
+            i_score = len(outs)
             outs.append(torch.empty((N, 2), device=self.device))
         if thr is not None:
+            i_surv = len(outs)
             outs.append(torch.empty((N, thr.size), device=self.device))
+        if uncertainty:
+            i_unc = len(outs)
+            outs.append(torch.empty((N, n_trios, 5), device=self.device))
 
         def consume(lo, hi, row0, pred):
             t = posterior.sample_instability(pred, seed, row_offset=row0)
             outs[0][lo:hi] = posterior.summarize_instability(t, pred, n_trios)
-            if y is not None:
-                outs[1][lo:hi] = posterior.score_labels(pred, y[lo:hi])
-            if thr is not None:
-                outs[-1][lo:hi] = posterior.survival(t, thr, n_trios)
+            if i_score is not None:
+                outs[i_score][lo:hi] = posterior.score_labels(pred, y[lo:hi])
+            if i_surv is not None:
+                outs[i_surv][lo:hi] = posterior.survival(t, thr, n_trios)
+            if i_unc is not None:
+                outs[i_unc][lo:hi] = posterior.uncertainty(pred, samples_per_model).view(hi - lo, n_trios, 5)
 
         self._walk_prediction_chunks(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
                                      consume)
         return outs
 
     def _reduce_sharded(self, x_local, n_total, samples_per_model, n_trios=1, seed=0, scale=0.5, group=None, y=None,
-                        thresholds=None):
+                        thresholds=None, uncertainty=False):
         """``_reduce`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE all_gather
-        moves the concatenated columns [N, 8 (+ 2) (+ J)].  Returns the same list, [n_total, ...] each, on every rank."""
+        moves the concatenated columns [N, 8 (+ 2) (+ J) (+ 5 n_trios)].  Returns the same list, [n_total, ...] each, on
+        every rank."""
         import math
 
         import torch.distributed as dist
 
-        self._check_reduce(x_local, samples_per_model, n_trios, y, thresholds)
+        self._check_reduce(x_local, samples_per_model, n_trios, y, thresholds, uncertainty)
         world = dist.get_world_size(group) if dist.is_initialized() else 1
         rank = dist.get_rank(group) if dist.is_initialized() else 0
         g = self.system_granule(x_local.shape[1])
@@ -556,11 +567,15 @@ class MultiSWAG:
         if x_local.shape[0] != (hi - lo) * n_trios:
             raise ValueError(f"rank {rank} owns systems [{lo}, {hi}) of {n_total} but was given "
                              f"{x_local.shape[0]} rows of {n_trios} trios")
-        outs = self._reduce(x_local, samples_per_model, n_trios, seed, scale, system_offset=lo, y=y, thresholds=thresholds)
+        outs = self._reduce(x_local, samples_per_model, n_trios, seed, scale, system_offset=lo, y=y, thresholds=thresholds,
+                            uncertainty=uncertainty)
         if world == 1:
             return outs
-        full = gather_system_shards(torch.cat(outs, 1), n_total, group, granule)
-        return [c.contiguous() for c in torch.split(full, [o.shape[1] for o in outs], 1)]
+        tails = [tuple(o.shape[1:]) for o in outs]
+        widths = [math.prod(t) for t in tails]
+        full = gather_system_shards(torch.cat([o.reshape(o.shape[0], w) for o, w in zip(outs, widths)], 1), n_total, group,
+                                    granule)
+        return [c.contiguous().view((n_total,) + t) for c, t in zip(torch.split(full, widths, 1), tails)]
 
     def evaluate(self, x: torch.Tensor, y: torch.Tensor, samples_per_model: int, seed: int = 0, scale: float = 0.5,
                  system_offset: int = 0, max_block_bytes: int = 640 << 20, unit_chunk: Optional[int] = None):
@@ -604,6 +619,32 @@ class MultiSWAG:
         summary, surv = self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale, group,
                                              thresholds=thresholds)
         return summary, surv
+
+    def posterior_uncertainty(self, x: torch.Tensor, samples_per_model: int, n_trios: int = 1, seed: int = 0,
+                              scale: float = 0.5, system_offset: int = 0, max_block_bytes: int = 640 << 20,
+                              unit_chunk: Optional[int] = None):
+        """Why a system's posterior is wide: x [N*n_trios, T, F] (as ``posterior_summary``) -> (summary [N, 8],
+        uncertainty [N, n_trios, 5]).  ``summary`` is exactly ``posterior_summary`` with the same arguments;
+        uncertainty[n, r] is ``posterior.uncertainty`` of the U = n_models * samples_per_model predicted normals of trio r
+        of system n (``posterior.UNCERTAINTY_NAMES``: mean_mu, aleatoric = mean sigma^2, epistemic = between_models +
+        within_models, the spread of mu between the models' means and among each model's SWAG samples).  These are
+        population (ddof = 0) moments of the untruncated normals, so aleatoric + epistemic is the variance of their
+        equal-weight mixture; they are per trio because the min over trios has no closed form, and they are not the
+        variance of the summary's truncated, prior-resampled sampled times.  Both outputs come from the same prediction
+        block, one system chunk at a time, so the predictive kernel runs once; neither depends on the chunking or on a
+        split into shards with ``system_offset``."""
+        summary, unc = self._reduce(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
+                                    uncertainty=True)
+        return summary, unc
+
+    def posterior_uncertainty_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int,
+                                      n_trios: int = 1, seed: int = 0, scale: float = 0.5, group=None):
+        """``posterior_uncertainty`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE
+        all_gather moves [N, 8 + 5 n_trios] (summary | uncertainty).  Returns (summary [n_total, 8], uncertainty
+        [n_total, n_trios, 5]) on every rank."""
+        summary, unc = self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale, group,
+                                            uncertainty=True)
+        return summary, unc
 
     def posterior_summary_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int, n_trios: int = 1,
                                   seed: int = 0, scale: float = 0.5, group=None):

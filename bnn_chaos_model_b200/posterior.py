@@ -4,7 +4,8 @@ Replaces the host-side numpy tail of the reference's evaluation scripts -- ``fas
 resampling of draws >= 9 from the analytic prior, min over trios, per-system median / percentiles
 (figures/main_figures.py:167-277, figures/multiswag_5_planet.py:306-481) -- so that only ``[N, 8]`` leaves the
 device instead of the ``[N, U, 2]`` prediction block.  ``survival`` counts the same sampled times against thresholds:
-P(T_inst > t) per system.
+P(T_inst > t) per system.  ``uncertainty`` splits each row's predictive variance into aleatoric, between-model and
+within-model parts.
 """
 from __future__ import annotations
 
@@ -123,3 +124,40 @@ def survival(t: torch.Tensor, thresholds, n_trios: int = 1):
         _lib.check(lib.bnn_survival_instability(_lib.ptr(t), N, int(n_trios), U, h_thr, thr.size, _lib.ptr(surv),
                                                 _lib.current_stream_ptr()), "bnn_survival_instability")
     return surv
+
+
+UNCERTAINTY_NAMES = ("mean_mu", "aleatoric", "epistemic", "between_models", "within_models")
+MAX_UNCERTAINTY_MODELS = 1024
+
+
+def uncertainty(pred: torch.Tensor, units_per_model: int):
+    """pred [rows, U, 2] (system-major (mu, sigma), unit u = model * units_per_model + sample as
+    ``MultiSWAG.sample_thetas`` numbers them) -> [rows, 5] (UNCERTAINTY_NAMES), per row in log10 orbits squared:
+    with m_k the mean mu of model k's S = units_per_model samples and mean the mean of the M = U / S model means,
+    ``mean_mu`` = mean, ``aleatoric`` = mean sigma^2, ``between_models`` = (1/M) sum_k (m_k - mean)^2,
+    ``within_models`` = (1/M) sum_k (1/S) sum_s (mu_{k,s} - m_k)^2 and ``epistemic`` = between + within
+    = (1/U) sum_u (mu_u - mean)^2.  Population (ddof = 0) moments, so by the law of total variance the equal-weight
+    mixture of the U predicted normals has variance aleatoric + epistemic.  They describe those untruncated normals, not
+    the sampled times of ``sample_instability`` (truncated at 4, resampled from the prior above 9, min over trios).
+    Accumulated in double, two-pass, rounded once.  A non-finite mu makes every column but ``aleatoric`` NaN; a
+    non-finite sigma makes ``aleatoric`` NaN."""
+    if pred.dim() != 3 or pred.shape[2] != 2:
+        raise ValueError(f"pred must be [rows, U, 2], got {tuple(pred.shape)}")
+    rows, U = pred.shape[0], pred.shape[1]
+    S = int(units_per_model)
+    if U == 0:
+        raise ValueError("pred has no units")
+    if S < 1 or U % S:
+        raise ValueError(f"{U} units are not a positive multiple of units_per_model = {units_per_model}")
+    if U // S > MAX_UNCERTAINTY_MODELS:
+        raise ValueError(f"{U // S} models: at most {MAX_UNCERTAINTY_MODELS} are supported")
+    lib = _lib.load()
+    _lib.require_cuda(pred, "pred")
+    pred = pred.contiguous().float()
+    out = torch.empty((rows, 5), device=pred.device, dtype=torch.float32)
+    if rows == 0:
+        return out
+    with torch.cuda.device(pred.device), _lib.nvtx("bnn:K7 decompose_uncertainty"):
+        _lib.check(lib.bnn_decompose_uncertainty(_lib.ptr(pred), rows, U, S, _lib.ptr(out), _lib.current_stream_ptr()),
+                   "bnn_decompose_uncertainty")
+    return out

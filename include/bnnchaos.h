@@ -299,6 +299,26 @@ int bnn_score_labels(const float* d_pred, int64_t n_systems, int64_t n_units, co
 int bnn_survival_instability(const float* d_t, int64_t n_systems, int32_t n_trios, int64_t n_units,
                              const float* h_thresholds, int32_t n_thresholds, float* d_surv, void* stream);
 
+/* Variance decomposition of every row of the system-major block d_pred [n_rows, U, 2] (row = system * n_trios + trio).
+ * Unit u = k * S + s is weight sample s of model k, S = units_per_model, M = U / S models; mu_{k,s} and sigma_{k,s} are
+ * its predicted normal in log10 orbits.  With m_k = (1/S) sum_s mu_{k,s} and mean = (1/M) sum_k m_k, d_out [n_rows, 5]:
+ *   [0] mean_mu        = mean
+ *   [1] aleatoric      = (1/U) sum_u sigma_u^2
+ *   [2] epistemic      = between_models + within_models (added in double) = (1/U) sum_u (mu_u - mean)^2
+ *   [3] between_models = (1/M) sum_k (m_k - mean)^2
+ *   [4] within_models  = (1/M) sum_k (1/S) sum_s (mu_{k,s} - m_k)^2
+ * Population (ddof = 0) moments: by the law of total variance the equal-weight mixture of the U normals has variance
+ * aleatoric + epistemic.  They describe the untruncated per-unit normals, not the sampled times of
+ * bnn_sample_instability (truncated at 4, resampled above 9, min over trios).  Two-pass in double (model means first,
+ * then deviations), rounded to fp32 once: between_models is exactly 0 when M = 1, within_models when S = 1, and both
+ * and epistemic when all mu of a row are equal.  A non-finite mu in a row makes columns 0, 2, 3, 4 NaN; a non-finite
+ * sigma makes column 1 NaN.  A row's result depends on that row only (fixed reduction order, no atomics): any row slice
+ * reproduces its rows bit for bit, and repeated calls are bit-identical.  BNN_E_ARG: null pointer, n_rows <= 0 or
+ * >= 2^31, n_units <= 0 or >= 2^32, units_per_model < 1, n_units not a multiple of units_per_model, more than 1024
+ * models; BNN_E_ALIGN: d_pred not 8-byte or d_out not 4-byte aligned; checked before the device. */
+int bnn_decompose_uncertainty(const float* d_pred, int64_t n_rows, int64_t n_units, int64_t units_per_model,
+                              float* d_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
