@@ -130,6 +130,10 @@ SIGNATURES = {
     "bnn_score_labels": (C.c_int, [c_f32p, C.c_int64, C.c_int64, c_f32p, c_f32p, C.c_void_p]),
     "bnn_survival_instability": (
         C.c_int, [c_f32p, C.c_int64, C.c_int32, C.c_int64, C.POINTER(C.c_float), C.c_int32, c_f32p, C.c_void_p]),
+    "bnn_summarize_instability_ragged": (
+        C.c_int, [c_f32p, c_f32p, C.c_int64, C.c_void_p, C.c_int32, c_f32p, C.c_void_p]),
+    "bnn_survival_instability_ragged": (
+        C.c_int, [c_f32p, C.c_int64, C.c_void_p, C.c_int64, C.POINTER(C.c_float), C.c_int32, c_f32p, C.c_void_p]),
     "bnn_decompose_uncertainty": (C.c_int, [c_f32p, C.c_int64, C.c_int64, C.c_int64, c_f32p, C.c_void_p]),
     "bnn_saliency": (C.c_int, [_CFG, C.c_int32, c_f32p, c_f32p, C.c_int64, c_f32p, C.c_uint64, c_f32p, c_f32p, c_f32p,
                                C.c_void_p, C.c_void_p]),

@@ -22,6 +22,11 @@
 // Variance decomposition of each prediction row of the block: the ensemble's mean mu, the aleatoric part (mean sigma^2),
 // and the epistemic part (variance of mu over the units) split into between-model and within-model parts.
 // [rows, U, 2] -> [rows, 5].
+//
+// The summary and survival kernels find a system's trio rows through a row map: UniformRows (every system has R rows,
+// system n starts at row n*R) or RaggedRows (a catalogue of mixed planet counts: per-system row offsets in device
+// memory, system n owns rows off[n] - off[0] .. off[n+1] - off[0] - 1).  One template per kernel; the uniform entries
+// instantiate UniformRows.
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -103,6 +108,33 @@ __global__ void __launch_bounds__(256) sample_instability_kernel(const float2* _
     t[idx] = val;
 }
 
+// ---- which rows belong to system n (rows are system-major: a system's trio rows are contiguous) ----
+struct UniformRows {   // every system has R trio rows; the first one, n*R, is formed where it is used
+    int R;
+    struct Span {
+        int64_t n;
+        int R;
+        __device__ __forceinline__ int64_t first() const { return n * R; }
+        __device__ __forceinline__ int count() const { return R; }
+    };
+    __device__ __forceinline__ Span operator()(int64_t n) const { return {n, R}; }
+    static __device__ __forceinline__ bool empty(const Span&) { return false; }
+};
+struct RaggedRows {    // per-system counts as offsets [n_systems + 1]; rows are counted from off[0]
+    const int64_t* __restrict__ off;
+    struct Span {
+        int64_t first_, count_;
+        __device__ __forceinline__ int64_t first() const { return first_; }
+        __device__ __forceinline__ int64_t count() const { return count_; }
+    };
+    __device__ __forceinline__ Span operator()(int64_t n) const {   // read once per CTA
+        const int64_t o0 = off[0], a = off[n], b = off[n + 1];
+        return {a - o0, b - a};
+    }
+    // a count <= 0 (malformed offsets) gives a NaN row instead of a read outside the block
+    static __device__ __forceinline__ bool empty(const Span& s) { return s.count_ <= 0; }
+};
+
 // ---- per-system order statistics over the weight samples: bitonic sort in shared memory ----
 __device__ __forceinline__ void bitonic_sort(float* s, int n) {
     for (int k = 2; k <= n; k <<= 1) {
@@ -143,22 +175,28 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
     return red[0];
 }
 
-// one CTA per system.  t[(n*R + r)*U + u]; pred[(n*R + r)*U + u] = (mu, std).  stats[n][8]:
+// one CTA per system.  t[(first + r)*U + u]; pred[(first + r)*U + u] = (mu, std), r < count (the system's Rows span).  stats[n][8]:
 // average, median, p84, p16, p97.5, p2.5 of min_r t; median over units of mu* = min_r mu and of its std.
+template <class Rows>
 __global__ void __launch_bounds__(512) summarize_instability_kernel(const float* __restrict__ t, const float2* __restrict__ pred,
-                                                                    int R, int U, int n_pow2, float* __restrict__ stats) {
+                                                                    Rows rows, int U, int n_pow2, float* __restrict__ stats) {
     extern __shared__ float sh[];
     float* s = sh;               // n_pow2 sort buffer
     float* red = sh + n_pow2;    // blockDim.x
     const int64_t n = blockIdx.x;
     const float INF = __int_as_float(0x7f800000);
     float* out = stats + n * 8;
+    const auto sp = rows(n);
+    if (Rows::empty(sp)) {   // uniform in the CTA: nobody reaches a barrier
+        if (threadIdx.x < 8) out[threadIdx.x] = __int_as_float(0x7fffffff);
+        return;
+    }
     // ---- min over trios of the sampled time ----
     float part = 0.f;
     for (int u = threadIdx.x; u < n_pow2; u += blockDim.x) {
         float v = INF;
         if (u < U) {
-            for (int r = 0; r < R; ++r) v = fminf(v, t[(n * R + r) * (int64_t)U + u]);
+            for (decltype(sp.count()) r = 0; r < sp.count(); ++r) v = fminf(v, t[(sp.first() + r) * (int64_t)U + u]);
             part += v;
         }
         s[u] = v;
@@ -180,8 +218,8 @@ __global__ void __launch_bounds__(512) summarize_instability_kernel(const float*
             float v = INF;
             if (u < U) {
                 float best = INF, bsd = 0.f;
-                for (int r = 0; r < R; ++r) {
-                    const float2 p = pred[(n * R + r) * (int64_t)U + u];
+                for (decltype(sp.count()) r = 0; r < sp.count(); ++r) {
+                    const float2 p = pred[(sp.first() + r) * (int64_t)U + u];
                     if (p.x < best || r == 0) { best = p.x; bsd = p.y; }
                 }
                 v = pass == 0 ? best : bsd;
@@ -209,17 +247,18 @@ __device__ __forceinline__ float key_value(uint32_t k) {
     return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
 }
 
-// which: 0 = min over trios of t, 1 = mu* (min over trios of mu), 2 = std of the arg-min trio
-__device__ __forceinline__ float summary_value(const float* __restrict__ t, const float2* __restrict__ pred, int64_t n, int R,
+// which: 0 = min over trios of t, 1 = mu* (min over trios of mu), 2 = std of the arg-min trio, over the rows of sp
+template <class Span>
+__device__ __forceinline__ float summary_value(const float* __restrict__ t, const float2* __restrict__ pred, const Span& sp,
                                                int U, int u, int which) {
     if (which == 0) {
         float v = __int_as_float(0x7f800000);
-        for (int r = 0; r < R; ++r) v = fminf(v, t[(n * R + r) * (int64_t)U + u]);
+        for (decltype(sp.count()) r = 0; r < sp.count(); ++r) v = fminf(v, t[(sp.first() + r) * (int64_t)U + u]);
         return v;
     }
     float best = 0.f, bsd = 0.f;
-    for (int r = 0; r < R; ++r) {
-        const float2 p = pred[(n * R + r) * (int64_t)U + u];
+    for (decltype(sp.count()) r = 0; r < sp.count(); ++r) {
+        const float2 p = pred[(sp.first() + r) * (int64_t)U + u];
         if (r == 0 || p.x < best) { best = p.x; bsd = p.y; }
     }
     return which == 1 ? best : bsd;
@@ -266,14 +305,20 @@ __device__ __forceinline__ int select_bin(const uint32_t* __restrict__ hist, int
     return bin;
 }
 
+template <class Rows>
 __global__ void __launch_bounds__(512) summarize_select_kernel(const float* __restrict__ t, const float2* __restrict__ pred,
-                                                               int R, int U, float* __restrict__ stats) {
+                                                               Rows rows, int U, float* __restrict__ stats) {
     extern __shared__ uint32_t hist[];            // [SEL_MAXT][2048]
     __shared__ uint32_t s_rank[SEL_MAXT], s_prefix[SEL_MAXT];
     __shared__ float s_val[SEL_MAXT], red[512];
     const int64_t n = blockIdx.x;
     const int warp = threadIdx.x >> 5;
     float* out = stats + n * 8;
+    const auto sp = rows(n);
+    if (Rows::empty(sp)) {   // uniform in the CTA: nobody reaches a barrier
+        if (threadIdx.x < 8) out[threadIdx.x] = __int_as_float(0x7fffffff);
+        return;
+    }
     const double qs[5] = {50.0, 50.0 + 68.0 / 2, 50.0 - 68.0 / 2, 50.0 + 95.0 / 2, 50.0 - 95.0 / 2};
     for (int which = 0; which < 3; ++which) {
         const int nq = which == 0 ? 5 : 1, nt = 2 * nq;
@@ -291,7 +336,7 @@ __global__ void __launch_bounds__(512) summarize_select_kernel(const float* __re
         for (int u0 = 0; u0 < U; u0 += blockDim.x) {   // whole warps stay in the loop: the merge below is warp-collective
             const int u = u0 + threadIdx.x;
             const bool valid = u < U;
-            const float v = valid ? summary_value(t, pred, n, R, U, u, which) : 0.f;
+            const float v = valid ? summary_value(t, pred, sp, U, u, which) : 0.f;
             if (valid) part += v;
             hist_add_warp(hist, order_key(v) >> 21, valid);
         }
@@ -312,7 +357,7 @@ __global__ void __launch_bounds__(512) summarize_select_kernel(const float* __re
             for (int i = threadIdx.x; i < nt * 2048; i += blockDim.x) hist[i] = 0;
             __syncthreads();
             for (int u = threadIdx.x; u < U; u += blockDim.x) {
-                const uint32_t k = order_key(summary_value(t, pred, n, R, U, u, which));
+                const uint32_t k = order_key(summary_value(t, pred, sp, U, u, which));
                 const uint32_t pre = k >> (shift + bits);
                 for (int tt = 0; tt < nt; ++tt)
                     if (pre == s_prefix[tt]) atomicAdd(&hist[tt * 2048 + ((k >> shift) & (nb - 1))], 1u);
@@ -403,7 +448,8 @@ struct SurvivalThresholds {   // passed by value in the kernel's parameters
     int32_t J;
 };
 
-__global__ void __launch_bounds__(SURV_THREADS) survival_kernel(const float* __restrict__ t, int R, int64_t U,
+template <class Rows>
+__global__ void __launch_bounds__(SURV_THREADS) survival_kernel(const float* __restrict__ t, Rows sys_rows, int64_t U,
                                                                 const __grid_constant__ SurvivalThresholds th,
                                                                 float* __restrict__ surv) {
     constexpr int WARPS = SURV_THREADS / 32;
@@ -411,18 +457,23 @@ __global__ void __launch_bounds__(SURV_THREADS) survival_kernel(const float* __r
     __shared__ uint32_t hist[WARPS][SURV_MAXJ + 1], s_tot[SURV_MAXJ + 1];
     const int tid = threadIdx.x, J = th.J;
     const float INF = __int_as_float(0x7f800000);
+    const int64_t n = blockIdx.x;
+    const auto sp = sys_rows(n);
+    if (Rows::empty(sp)) {   // uniform in the CTA: nobody reaches a barrier
+        if (tid < J) surv[n * J + tid] = __int_as_float(0x7fffffff);
+        return;
+    }
     if (tid < J) s_thr[tid] = th.thr[tid];
     for (int i = tid; i < WARPS * (SURV_MAXJ + 1); i += SURV_THREADS) (&hist[0][0])[i] = 0;
     __syncthreads();
-    const int64_t n = blockIdx.x;
-    const float* __restrict__ rows = t + n * (int64_t)R * U;
+    const float* __restrict__ rows = t + sp.first() * U;
     uint32_t* __restrict__ h = hist[tid >> 5];
     // whole warps stay in the loop: hist_add_warp is warp-collective
     for (int64_t u0 = 0; u0 < U; u0 += SURV_THREADS * SURV_UNROLL) {
         float v[SURV_UNROLL];
 #pragma unroll
         for (int k = 0; k < SURV_UNROLL; ++k) v[k] = INF;
-        for (int r = 0; r < R; ++r) {   // SURV_UNROLL independent coalesced loads in flight per trio row
+        for (decltype(sp.count()) r = 0; r < sp.count(); ++r) {   // SURV_UNROLL independent coalesced loads in flight per trio row
 #pragma unroll
             for (int k = 0; k < SURV_UNROLL; ++k) {
                 const int64_t u = u0 + k * SURV_THREADS + tid;
@@ -599,18 +650,19 @@ int bnn_set_summary_variant(int32_t variant) {
     return BNN_OK;
 }
 
-int bnn_summarize_instability(const float* d_t, const float* d_pred, int64_t n_systems, int32_t n_trios, int32_t n_units,
-                              float* d_stats, void* stream) {
+}  // extern "C"
+
+namespace {
+
+// summary launch for either row map: the shared-memory sort while U fits, else (or when forced) the radix select
+template <class Rows>
+int launch_summary(const float* d_t, const float* d_pred, int64_t n_systems, Rows rows, int32_t n_units, float* d_stats,
+                   void* stream) {
     using namespace bnn;
-    int rc = check_device();
-    if (rc != BNN_OK) return rc;
-    BNN_REQUIRE(d_t && d_pred && d_stats && n_systems > 0 && n_trios > 0 && n_units > 0, BNN_E_ARG,
-                "bnn_summarize_instability: null pointer or empty problem");
     int n_pow2 = 1;
     while (n_pow2 < n_units) n_pow2 <<= 1;
     const int threads = 512;
     const size_t smem = (size_t)(n_pow2 + threads) * sizeof(float);
-    BNN_REQUIRE(n_systems < (1ll << 31), BNN_E_ARG, "bnn_summarize_instability: too many systems for one launch");
     const bool use_select = summary_variant() == 1 || smem > 200 * 1024;   // 1: forced (tests cross-check the two)
     if (use_select) {
         // more weight samples than the shared-memory sort holds (30 models x 2000 samples = 60000 at BASELINE config 3):
@@ -618,21 +670,68 @@ int bnn_summarize_instability(const float* d_t, const float* d_pred, int64_t n_s
         const size_t hsm = (size_t)SEL_MAXT * 2048 * sizeof(uint32_t);
         static PerDeviceOnce attr2_done;
         if (attr2_done.need()) {
-            BNN_CUDA(cudaFuncSetAttribute(summarize_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            BNN_CUDA(cudaFuncSetAttribute(summarize_select_kernel<Rows>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          200 * 1024));
         }
-        summarize_select_kernel<<<(unsigned)n_systems, threads, hsm, (cudaStream_t)stream>>>(d_t, (const float2*)d_pred, n_trios,
-                                                                                         n_units, d_stats);
+        summarize_select_kernel<Rows><<<(unsigned)n_systems, threads, hsm, (cudaStream_t)stream>>>(
+            d_t, (const float2*)d_pred, rows, n_units, d_stats);
         BNN_CUDA(cudaGetLastError());
         return BNN_OK;
     }
     static PerDeviceOnce attr_done;
     if (attr_done.need()) {
-        BNN_CUDA(cudaFuncSetAttribute(summarize_instability_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        BNN_CUDA(cudaFuncSetAttribute(summarize_instability_kernel<Rows>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      200 * 1024));
     }
-    summarize_instability_kernel<<<(unsigned)n_systems, threads, smem, (cudaStream_t)stream>>>(
-        d_t, (const float2*)d_pred, n_trios, n_units, n_pow2, d_stats);
+    summarize_instability_kernel<Rows><<<(unsigned)n_systems, threads, smem, (cudaStream_t)stream>>>(
+        d_t, (const float2*)d_pred, rows, n_units, n_pow2, d_stats);
     BNN_CUDA(cudaGetLastError());
     return BNN_OK;
+}
+
+// the thresholds sorted ascending, with their output columns, for the kernel's parameters; BNN_E_ARG on a NaN
+int survival_thresholds(const char* what, const float* h_thresholds, int32_t n_thresholds, bnn::SurvivalThresholds& th) {
+    using namespace bnn;
+    BNN_REQUIRE(n_thresholds >= 1 && n_thresholds <= SURV_MAXJ, BNN_E_ARG,
+                "%s: n_thresholds must be in [1, %d], got %d", what, SURV_MAXJ, (int)n_thresholds);
+    for (int j = 0; j < n_thresholds; ++j)
+        BNN_REQUIRE(!isnan(h_thresholds[j]), BNN_E_ARG, "%s: threshold %d is NaN", what, j);
+    th.J = n_thresholds;
+    for (int j = 0; j < n_thresholds; ++j) th.col[j] = j;
+    std::stable_sort(th.col, th.col + n_thresholds, [&](int a, int b) { return h_thresholds[a] < h_thresholds[b]; });
+    for (int j = 0; j < n_thresholds; ++j) th.thr[j] = h_thresholds[th.col[j]];
+    for (int j = n_thresholds; j < SURV_MAXJ; ++j) { th.thr[j] = 0.f; th.col[j] = 0; }
+    return BNN_OK;
+}
+
+bool aligned(const void* q, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(q) & (bytes - 1)) == 0; }
+
+}  // namespace
+
+extern "C" {
+
+int bnn_summarize_instability(const float* d_t, const float* d_pred, int64_t n_systems, int32_t n_trios, int32_t n_units,
+                              float* d_stats, void* stream) {
+    using namespace bnn;
+    int rc = check_device();
+    if (rc != BNN_OK) return rc;
+    BNN_REQUIRE(d_t && d_pred && d_stats && n_systems > 0 && n_trios > 0 && n_units > 0, BNN_E_ARG,
+                "bnn_summarize_instability: null pointer or empty problem");
+    BNN_REQUIRE(n_systems < (1ll << 31), BNN_E_ARG, "bnn_summarize_instability: too many systems for one launch");
+    return launch_summary(d_t, d_pred, n_systems, UniformRows{n_trios}, n_units, d_stats, stream);
+}
+
+int bnn_summarize_instability_ragged(const float* d_t, const float* d_pred, int64_t n_systems,
+                                     const int64_t* d_row_offsets, int32_t n_units, float* d_stats, void* stream) {
+    using namespace bnn;
+    // argument checks first: they need no device
+    BNN_REQUIRE(d_t && d_pred && d_stats && d_row_offsets && n_systems > 0 && n_units > 0, BNN_E_ARG,
+                "bnn_summarize_instability_ragged: null pointer or empty problem");
+    BNN_REQUIRE(n_systems < (1ll << 31), BNN_E_ARG, "bnn_summarize_instability_ragged: too many systems for one launch");
+    BNN_REQUIRE(aligned(d_row_offsets, 8), BNN_E_ALIGN, "bnn_summarize_instability_ragged: d_row_offsets must be 8-byte aligned");
+    int rc = check_device();
+    if (rc != BNN_OK) return rc;
+    return launch_summary(d_t, d_pred, n_systems, RaggedRows{d_row_offsets}, n_units, d_stats, stream);
 }
 
 int bnn_score_labels(const float* d_pred, int64_t n_systems, int64_t n_units, const float* d_y, float* d_score,
@@ -660,23 +759,38 @@ int bnn_survival_instability(const float* d_t, int64_t n_systems, int32_t n_trio
     // argument checks first: they need no device
     BNN_REQUIRE(d_t && h_thresholds && d_surv && n_systems > 0 && n_units > 0 && n_trios >= 1, BNN_E_ARG,
                 "bnn_survival_instability: null pointer or empty problem");
-    BNN_REQUIRE(n_thresholds >= 1 && n_thresholds <= SURV_MAXJ, BNN_E_ARG,
-                "bnn_survival_instability: n_thresholds must be in [1, %d], got %d", SURV_MAXJ, (int)n_thresholds);
+    SurvivalThresholds th;
+    int rc = survival_thresholds("bnn_survival_instability", h_thresholds, n_thresholds, th);
+    if (rc != BNN_OK) return rc;
     BNN_REQUIRE(n_systems < (1ll << 31) && n_units < (1ll << 32), BNN_E_ARG,
                 "bnn_survival_instability: n_systems must be < 2^31 and n_units < 2^32");
-    for (int j = 0; j < n_thresholds; ++j)
-        BNN_REQUIRE(!isnan(h_thresholds[j]), BNN_E_ARG, "bnn_survival_instability: threshold %d is NaN", j);
-    const auto aligned4 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 3u) == 0; };
-    BNN_REQUIRE(aligned4(d_t) && aligned4(d_surv), BNN_E_ALIGN, "bnn_survival_instability: pointers must be 4-byte aligned");
-    SurvivalThresholds th;
-    th.J = n_thresholds;
-    for (int j = 0; j < n_thresholds; ++j) th.col[j] = j;
-    std::stable_sort(th.col, th.col + n_thresholds, [&](int a, int b) { return h_thresholds[a] < h_thresholds[b]; });
-    for (int j = 0; j < n_thresholds; ++j) th.thr[j] = h_thresholds[th.col[j]];
-    for (int j = n_thresholds; j < SURV_MAXJ; ++j) { th.thr[j] = 0.f; th.col[j] = 0; }
-    int rc = check_device();
+    BNN_REQUIRE(aligned(d_t, 4) && aligned(d_surv, 4), BNN_E_ALIGN, "bnn_survival_instability: pointers must be 4-byte aligned");
+    rc = check_device();
     if (rc != BNN_OK) return rc;
-    survival_kernel<<<(unsigned)n_systems, SURV_THREADS, 0, (cudaStream_t)stream>>>(d_t, n_trios, n_units, th, d_surv);
+    survival_kernel<<<(unsigned)n_systems, SURV_THREADS, 0, (cudaStream_t)stream>>>(d_t, UniformRows{n_trios}, n_units, th,
+                                                                                     d_surv);
+    BNN_CUDA(cudaGetLastError());
+    return BNN_OK;
+}
+
+int bnn_survival_instability_ragged(const float* d_t, int64_t n_systems, const int64_t* d_row_offsets, int64_t n_units,
+                                    const float* h_thresholds, int32_t n_thresholds, float* d_surv, void* stream) {
+    using namespace bnn;
+    // argument checks first: they need no device
+    BNN_REQUIRE(d_t && h_thresholds && d_surv && d_row_offsets && n_systems > 0 && n_units > 0, BNN_E_ARG,
+                "bnn_survival_instability_ragged: null pointer or empty problem");
+    SurvivalThresholds th;
+    int rc = survival_thresholds("bnn_survival_instability_ragged", h_thresholds, n_thresholds, th);
+    if (rc != BNN_OK) return rc;
+    BNN_REQUIRE(n_systems < (1ll << 31) && n_units < (1ll << 32), BNN_E_ARG,
+                "bnn_survival_instability_ragged: n_systems must be < 2^31 and n_units < 2^32");
+    BNN_REQUIRE(aligned(d_t, 4) && aligned(d_surv, 4), BNN_E_ALIGN,
+                "bnn_survival_instability_ragged: pointers must be 4-byte aligned");
+    BNN_REQUIRE(aligned(d_row_offsets, 8), BNN_E_ALIGN, "bnn_survival_instability_ragged: d_row_offsets must be 8-byte aligned");
+    rc = check_device();
+    if (rc != BNN_OK) return rc;
+    survival_kernel<<<(unsigned)n_systems, SURV_THREADS, 0, (cudaStream_t)stream>>>(d_t, RaggedRows{d_row_offsets}, n_units,
+                                                                                     th, d_surv);
     BNN_CUDA(cudaGetLastError());
     return BNN_OK;
 }

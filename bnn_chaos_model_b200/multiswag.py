@@ -37,13 +37,34 @@ def shard_range(n: int, rank: int, world: int, granule: int = 1):
     return min(glo * granule, n), min(ghi * granule, n)
 
 
-def gather_system_shards(local: torch.Tensor, n_total: int, group=None, granule: int = 1) -> torch.Tensor:
+def catalogue_shard_range(n_trios, rank: int, world: int, granule: int = 1):
+    """The shard of a catalogue of mixed planet counts (per-system trio counts ``n_trios`` [N], R rows in all) that rank
+    `rank` of `world` reduces: (sys_lo, sys_hi, row_lo, row_hi).  Systems go to ranks in contiguous blocks balanced by
+    rows: rank r starts at the first system whose first row is >= floor(r R / world), so a shard's rows differ from
+    R / world by less than one system's count; shards may be empty.  [row_lo, row_hi) = [floor_g(off[sys_lo]),
+    min(ceil_g(off[sys_hi]), R)) with g = ``granule`` (``MultiSWAG.system_granule``) is the slice of x the rank passes:
+    its owned rows plus up to g - 1 context rows on each side, which put every owned row at the position in its
+    g-row group that it has in one launch over the whole catalogue (see ``_walk_prediction_chunks``).  An empty shard
+    passes no rows."""
+    from .posterior import row_offsets
+
+    off = row_offsets(n_trios, None)
+    n, R, g = off.size - 1, int(off[-1]), max(1, int(granule))
+    first = lambda r: n if r >= world else int(np.searchsorted(off[:-1], (r * R) // world, side="left"))
+    sys_lo, sys_hi = first(rank), first(rank + 1)
+    row_lo = int(off[sys_lo]) // g * g
+    row_hi = min(-(-int(off[sys_hi]) // g) * g, R) if sys_hi > sys_lo else row_lo
+    return sys_lo, sys_hi, row_lo, row_hi
+
+
+def gather_system_shards(local: torch.Tensor, n_total: int, group=None, granule: int = 1, bounds=None) -> torch.Tensor:
     """The path's only collective: all_gather of the system-major block [N_local, ...] of every
-    rank into [n_total, ...] (ranks own ``shard_range`` blocks, so the result needs no permute)."""
+    rank into [n_total, ...] (ranks own ``shard_range`` blocks, or the explicit per-rank [a, b) ``bounds`` (one pair per
+    rank, contiguous and in rank order), so the result needs no permute)."""
     import torch.distributed as dist
 
     world, rank = dist.get_world_size(group), dist.get_rank(group)
-    sizes = [shard_range(n_total, r, world, granule) for r in range(world)]
+    sizes = bounds if bounds is not None else [shard_range(n_total, r, world, granule) for r in range(world)]
     assert local.shape[0] == sizes[rank][1] - sizes[rank][0]
     tail = tuple(local.shape[1:])
     full = torch.empty((n_total,) + tail, device=local.device, dtype=local.dtype)
@@ -426,9 +447,18 @@ class MultiSWAG:
         systems of prediction; default chunk: 16 units per SM = whole waves of the sampler's 4-unit CTAs, 2368 on a
         B200).  Philox draws are keyed on global (unit, row) indices, so the result does not depend on
         either chunking (BASELINE configs[2]: 12,500 systems x 60,000 units per GPU would be 9 GB of predictions and
-        4.6 GB of packed weights in one piece; peak here < 1 GB)."""
+        4.6 GB of packed weights in one piece; peak here < 1 GB).
+
+        A catalogue of mixed planet counts passes per-system trio counts [N] as ``n_trios`` (1-D integers >= 1 summing to
+        the rows of x, ``posterior.row_offsets``): system n owns the next n_trios[n] rows of x, and the result is [N, 8]
+        with each system's min over its own trios.  ``system_offset`` must then be 0; split a catalogue with the
+        ``_sharded`` methods (``catalogue_shard_range``).  With every count equal to k the result is that of n_trios = k,
+        bit for bit."""
         from . import posterior
 
+        if posterior.is_ragged(n_trios):
+            self._check_catalogue(x, n_trios)
+            return self._reduce(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk)[0]
         rows = x.shape[0]
         if rows % n_trios:
             raise ValueError(f"{rows} rows are not a multiple of {n_trios} trios")
@@ -442,13 +472,25 @@ class MultiSWAG:
         return out
 
     def _walk_prediction_chunks(self, x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes,
-                                unit_chunk, consume):
-        """The chunk walk of ``posterior_summary`` (see there): for each system chunk [lo, hi) of x, the prediction block
-        [(hi - lo) * n_trios, U, 2] of all U units is built and ``consume(lo, hi, row0, pred)`` is called on it (row0: the
-        global index of its first row).  One block exists at a time."""
+                                unit_chunk, consume, off=None, row_offset=0):
+        """The chunk walk of ``posterior_summary`` (see there): x is cut into chunks of whole systems, and for each chunk
+        of systems [lo, hi) that owns the rows [a, b) of x, the prediction block [b - a, U, 2] of all U units is built and
+        ``consume(lo, hi, row0, pred)`` is called on it (row0: the global index of its first row, which keys the Philox
+        draws).  One block exists at a time, of at most ``max_block_bytes`` (12 bytes per (row, unit); one system at
+        least).
+
+        Uniform systems (``off`` None): system n owns rows n*n_trios ..; chunks are cut at multiples of the kernel's
+        system granule g in rows, and row0 = (system_offset + lo) * n_trios.  A catalogue passes its row offsets ``off``
+        [n + 1] relative to x's first row (off[0] > 0 when x starts with context rows) and ``row_offset``, the global
+        row of x's first row.  Its system boundaries need not fall on the granule, so the predictive kernel runs over
+        rows [floor_g(a), min(ceil_g(b), rows of x)) and the up to g - 1 context rows on each side are dropped: a row's
+        bits depend on its position in its g-row group (pooling runs in 32-row blocks) and on the other rows of that
+        group (the layer-1 bias rides in the MMA only for blocks that hold no scaled-down row, DESIGN section 3), and
+        the context rows give both what they are in one launch over all of x.  With the uniform layout every a and b
+        is already aligned, so there are no context rows."""
         import math
 
-        N = x.shape[0] // n_trios
+        rows = x.shape[0]
         U = self.n_models * samples_per_model
         if unit_chunk is None:
             unit_chunk = 16 * torch.cuda.get_device_properties(self.device).multi_processor_count
@@ -458,24 +500,39 @@ class MultiSWAG:
             if U <= unit_chunk + unit_chunk // 2:       # few units: sample once, reuse for every system chunk
                 _, thp_all = self.sample_thetas(samples_per_model, seed, scale, want_flat=False)
             g = self.system_granule(x.shape[1])
-            gs = g // math.gcd(g, n_trios)                      # systems per chunk boundary such that rows stay aligned
-            per = max(1, int(max_block_bytes // (12 * U * n_trios)))
-            per = max(gs, per // gs * gs)
-            for lo in range(0, N, per):
-                hi = min(lo + per, N)
-                row0 = (system_offset + lo) * n_trios
-                xs = x[lo * n_trios:hi * n_trios]
-                pred = torch.empty((xs.shape[0], U, 2), device=self.device)
+            if off is None:
+                N = rows // n_trios
+                off = np.arange(N + 1, dtype=np.int64) * n_trios
+                row_offset = system_offset * n_trios
+                gs = g // math.gcd(g, n_trios)                      # systems per chunk boundary such that rows stay aligned
+                per = max(1, int(max_block_bytes // (12 * U * n_trios)))
+                per = max(gs, per // gs * gs)
+                chunks = [(lo, min(lo + per, N)) for lo in range(0, N, per)]
+            else:
+                N = off.size - 1
+                budget = max(1, int(max_block_bytes // (12 * U)))   # launched rows per chunk, context included
+                end = np.minimum(-(-off // g) * g, rows)            # launch end when a chunk ends before system k
+                chunks, lo = [], 0
+                while lo < N:
+                    la = int(off[lo]) // g * g
+                    hi = min(N, max(lo + 1, int(np.searchsorted(end, la + budget, side="right")) - 1))
+                    chunks.append((lo, hi))
+                    lo = hi
+            for lo, hi in chunks:
+                a, b = int(off[lo]), int(off[hi])
+                la, lb = a // g * g, min(-(-b // g) * g, rows)
+                xs = x[la:lb]
+                pred = torch.empty((lb - la, U, 2), device=self.device)
                 if thp_all is not None:
-                    self.predict_into(xs, thp_all, pred, 0, seed, system_offset=row0)
+                    self.predict_into(xs, thp_all, pred, 0, seed, system_offset=row_offset + la)
                 else:
                     for u0 in range(0, U, unit_chunk):
                         u1 = min(u0 + unit_chunk, U)
                         _, thp = self.sample_thetas(samples_per_model, seed, scale, unit_offset=u0, n_units=u1 - u0,
                                                     want_flat=False)
-                        self.predict_into(xs, thp, pred, u0, seed, system_offset=row0)
+                        self.predict_into(xs, thp, pred, u0, seed, system_offset=row_offset + la)
                         del thp
-                consume(lo, hi, row0, pred)
+                consume(lo, hi, row_offset + a, pred[a - la:b - la])
                 del pred
 
     @staticmethod
@@ -493,19 +550,24 @@ class MultiSWAG:
         _lib.require_cuda(y, "y")
 
     @staticmethod
-    def _check_reduce(x: torch.Tensor, samples_per_model: int, n_trios: int, y=None, thresholds=None,
+    def _check_reduce(x: torch.Tensor, samples_per_model: int, n_trios, y=None, thresholds=None,
                       uncertainty=False):
         """Argument checks of ``_reduce`` / ``_reduce_sharded``, before any device work.  Returns the thresholds as
         ``posterior.survival_thresholds`` (or None)."""
         from . import posterior
 
+        ragged = posterior.is_ragged(n_trios)   # a catalogue: its counts are checked here, its rows by the caller
+        if ragged:
+            if y is not None:
+                raise ValueError("held-out scoring takes one trio per system: pass an int n_trios = 1 with labels")
+            posterior.row_offsets(n_trios, None)
         if y is not None:
             MultiSWAG._check_labelled(x, y, samples_per_model)
-        if thresholds is None and not uncertainty:
+        if thresholds is None and not uncertainty and not ragged:
             return None
         if x.dim() != 3:
             raise ValueError(f"x must be [N*n_trios, T, F], got {tuple(x.shape)}")
-        if int(n_trios) < 1 or x.shape[0] % n_trios:
+        if not ragged and (int(n_trios) < 1 or x.shape[0] % n_trios):
             raise ValueError(f"{x.shape[0]} rows are not a multiple of {n_trios} trios")
         if int(samples_per_model) < 1:
             raise ValueError(f"samples_per_model must be >= 1, got {samples_per_model}")
@@ -513,16 +575,42 @@ class MultiSWAG:
         _lib.require_cuda(x, "x")
         return thr
 
+    @staticmethod
+    def _check_catalogue(x: torch.Tensor, n_trios):
+        """A whole catalogue (the public methods): per-system trio counts must cover the rows of x exactly."""
+        from . import posterior
+
+        if posterior.is_ragged(n_trios):
+            posterior.row_offsets(n_trios, x.shape[0])
+
     def _reduce(self, x, samples_per_model, n_trios=1, seed=0, scale=0.5, system_offset=0, max_block_bytes=640 << 20,
-                unit_chunk=None, y=None, thresholds=None, uncertainty=False):
+                unit_chunk=None, y=None, thresholds=None, uncertainty=False, row_offset=0, first_row=0):
         """One walk over the prediction block (``_walk_prediction_chunks``) that reduces every system chunk on the device
         and returns [summary [N, 8]] + [score [N, 2]] if labels y are given + [survival [N, J]] if thresholds are given
         + [uncertainty [N, n_trios, 5]] if ``uncertainty`` is set.  Each chunk's instability times are sampled once and
-        feed both the summary and the survival counts; the uncertainty decomposes the same prediction block."""
+        feed both the summary and the survival counts; the uncertainty decomposes the same prediction block.
+
+        With per-system trio counts ``n_trios`` [N] (a catalogue, no labels) the systems own the rows first_row ..
+        first_row + sum(n_trios) - 1 of x, any rows around them are context (``catalogue_shard_range``), ``row_offset``
+        is the global row of x's first row (it keys the Philox draws; ``system_offset`` must be 0), and the uncertainty
+        is [sum(n_trios), 5] in row order."""
         from . import posterior
 
+        ragged = posterior.is_ragged(n_trios)
+        if ragged and system_offset:
+            raise ValueError("with per-system trio counts system_offset must be 0: split a catalogue with the _sharded "
+                             "methods")
         thr = self._check_reduce(x, samples_per_model, n_trios, y, thresholds, uncertainty)
-        N = x.shape[0] // n_trios
+        off = None
+        if ragged:
+            off = posterior.row_offsets(n_trios, None) + int(first_row)
+            if first_row < 0 or off[-1] > x.shape[0]:
+                raise ValueError(f"the systems' rows [{int(off[0])}, {int(off[-1])}) do not fit in the {x.shape[0]} rows "
+                                 "of x")
+            N = off.size - 1
+            d_off = posterior.device_offsets(off, self.device)
+        else:
+            N = x.shape[0] // n_trios
         outs = [torch.empty((N, 8), device=self.device)]
         i_score = i_surv = i_unc = None
         if y is not None:
@@ -533,10 +621,19 @@ class MultiSWAG:
             outs.append(torch.empty((N, thr.size), device=self.device))
         if uncertainty:
             i_unc = len(outs)
-            outs.append(torch.empty((N, n_trios, 5), device=self.device))
+            outs.append(torch.empty((int(off[-1] - off[0]), 5) if ragged else (N, n_trios, 5), device=self.device))
 
         def consume(lo, hi, row0, pred):
             t = posterior.sample_instability(pred, seed, row_offset=row0)
+            if ragged:
+                d = d_off[lo:hi + 1]   # rows counted from d[0]: the chunk's first row
+                outs[0][lo:hi] = posterior.summarize_ragged(t, pred, d)
+                if i_surv is not None:
+                    outs[i_surv][lo:hi] = posterior.survival_ragged(t, thr, d)
+                if i_unc is not None:
+                    a = int(off[lo] - off[0])
+                    outs[i_unc][a:a + pred.shape[0]] = posterior.uncertainty(pred, samples_per_model)
+                return
             outs[0][lo:hi] = posterior.summarize_instability(t, pred, n_trios)
             if i_score is not None:
                 outs[i_score][lo:hi] = posterior.score_labels(pred, y[lo:hi])
@@ -546,22 +643,57 @@ class MultiSWAG:
                 outs[i_unc][lo:hi] = posterior.uncertainty(pred, samples_per_model).view(hi - lo, n_trios, 5)
 
         self._walk_prediction_chunks(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
-                                     consume)
+                                     consume, off=off, row_offset=row_offset)
         return outs
 
     def _reduce_sharded(self, x_local, n_total, samples_per_model, n_trios=1, seed=0, scale=0.5, group=None, y=None,
                         thresholds=None, uncertainty=False):
         """``_reduce`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE all_gather
         moves the concatenated columns [N, 8 (+ 2) (+ J) (+ 5 n_trios)].  Returns the same list, [n_total, ...] each, on
-        every rank."""
+        every rank.
+
+        A catalogue passes the trio counts of the WHOLE catalogue [n_total] as ``n_trios`` and, on each rank, the rows
+        [row_lo, row_hi) of ``catalogue_shard_range`` as x_local; one all_gather moves the per-system columns and, with
+        ``uncertainty``, a second one the per-row uncertainty [rows, 5]."""
         import math
 
         import torch.distributed as dist
 
-        self._check_reduce(x_local, samples_per_model, n_trios, y, thresholds, uncertainty)
+        from . import posterior
+
+        thr = self._check_reduce(x_local, samples_per_model, n_trios, y, thresholds, uncertainty)
         world = dist.get_world_size(group) if dist.is_initialized() else 1
         rank = dist.get_rank(group) if dist.is_initialized() else 0
         g = self.system_granule(x_local.shape[1])
+        if posterior.is_ragged(n_trios):
+            counts = np.asarray(n_trios.detach().cpu() if isinstance(n_trios, torch.Tensor) else n_trios)
+            off = posterior.row_offsets(counts, None)
+            if counts.size != n_total:
+                raise ValueError(f"{counts.size} trio counts for a catalogue of n_total = {n_total} systems")
+            shards = [catalogue_shard_range(counts, r, world, g) for r in range(world)]
+            slo, shi, rlo, rhi = shards[rank]
+            if x_local.shape[0] != rhi - rlo:
+                raise ValueError(f"rank {rank} owns systems [{slo}, {shi}) and passes rows [{rlo}, {rhi}) of the catalogue "
+                                 f"but was given {x_local.shape[0]} rows")
+            if shi > slo:
+                outs = self._reduce(x_local, samples_per_model, counts[slo:shi], seed, scale, thresholds=thresholds,
+                                    uncertainty=uncertainty, row_offset=rlo, first_row=int(off[slo]) - rlo)
+            else:   # an empty shard: more ranks than systems
+                outs = [torch.empty((0, 8), device=self.device)]
+                if thr is not None:
+                    outs.append(torch.empty((0, thr.size), device=self.device))
+                if uncertainty:
+                    outs.append(torch.empty((0, 5), device=self.device))
+            if world == 1:
+                return outs
+            cols = outs[:-1] if uncertainty else outs
+            widths = [o.shape[1] for o in cols]
+            full = gather_system_shards(torch.cat(cols, 1), n_total, group, bounds=[(a, b) for a, b, _, _ in shards])
+            res = [c.contiguous() for c in torch.split(full, widths, 1)]
+            if uncertainty:
+                res.append(gather_system_shards(outs[-1], int(off[-1]), group,
+                                                bounds=[(int(off[a]), int(off[b])) for a, b, _, _ in shards]))
+            return res
         granule = g // math.gcd(g, n_trios)  # shard boundaries in SYSTEMS such that rows stay granule-aligned
         lo, hi = shard_range(n_total, rank, world, granule)
         if x_local.shape[0] != (hi - lo) * n_trios:
@@ -606,7 +738,9 @@ class MultiSWAG:
         (``posterior.survival``).  S_j is a Monte Carlo estimate of P(T_inst > thresholds[j]) with standard error
         sqrt(S_j (1 - S_j) / U), and it counts the very draws the summary's percentiles come from: each system chunk's
         times are sampled once and feed both, so the predictive kernel runs once.  Neither output depends on the
-        chunking or on a split into shards with ``system_offset``."""
+        chunking or on a split into shards with ``system_offset``.  ``n_trios`` may be per-system trio counts, as in
+        ``posterior_summary``."""
+        self._check_catalogue(x, n_trios)
         summary, surv = self._reduce(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
                                      thresholds=thresholds)
         return summary, surv
@@ -615,7 +749,7 @@ class MultiSWAG:
                                    n_trios: int = 1, seed: int = 0, scale: float = 0.5, group=None):
         """``posterior_survival`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE
         all_gather moves [N, 8 + J] (summary | survival).  Returns (summary [n_total, 8], survival [n_total, J]) on every
-        rank."""
+        rank.  A catalogue passes the trio counts of the whole catalogue and its ``catalogue_shard_range`` rows."""
         summary, surv = self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale, group,
                                              thresholds=thresholds)
         return summary, surv
@@ -632,7 +766,10 @@ class MultiSWAG:
         equal-weight mixture; they are per trio because the min over trios has no closed form, and they are not the
         variance of the summary's truncated, prior-resampled sampled times.  Both outputs come from the same prediction
         block, one system chunk at a time, so the predictive kernel runs once; neither depends on the chunking or on a
-        split into shards with ``system_offset``."""
+        split into shards with ``system_offset``.  With per-system trio counts ``n_trios`` (as in ``posterior_summary``)
+        the uncertainty is [rows, 5] in x's row order; for an int n_trios that is the same data as a view of
+        [N, n_trios, 5]."""
+        self._check_catalogue(x, n_trios)
         summary, unc = self._reduce(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
                                     uncertainty=True)
         return summary, unc
@@ -641,17 +778,24 @@ class MultiSWAG:
                                       n_trios: int = 1, seed: int = 0, scale: float = 0.5, group=None):
         """``posterior_uncertainty`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE
         all_gather moves [N, 8 + 5 n_trios] (summary | uncertainty).  Returns (summary [n_total, 8], uncertainty
-        [n_total, n_trios, 5]) on every rank."""
+        [n_total, n_trios, 5]) on every rank.  A catalogue passes the trio counts of the whole catalogue and its
+        ``catalogue_shard_range`` rows; a second all_gather then moves the uncertainty [rows, 5]."""
         summary, unc = self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale, group,
                                             uncertainty=True)
         return summary, unc
 
     def posterior_summary_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int, n_trios: int = 1,
                                   seed: int = 0, scale: float = 0.5, group=None):
-        """Systems block-partitioned over ranks; the single all_gather moves [N, 8] instead of [N, U, 2]."""
+        """Systems block-partitioned over ranks; the single all_gather moves [N, 8] instead of [N, U, 2].  A catalogue
+        passes the trio counts of the whole catalogue as ``n_trios`` and its ``catalogue_shard_range`` rows as x_local."""
         import math
 
         import torch.distributed as dist
+
+        from . import posterior
+
+        if posterior.is_ragged(n_trios):
+            return self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale, group)[0]
 
         world = dist.get_world_size(group) if dist.is_initialized() else 1
         rank = dist.get_rank(group) if dist.is_initialized() else 0

@@ -6,10 +6,15 @@ resampling of draws >= 9 from the analytic prior, min over trios, per-system med
 device instead of the ``[N, U, 2]`` prediction block.  ``survival`` counts the same sampled times against thresholds:
 P(T_inst > t) per system.  ``uncertainty`` splits each row's predictive variance into aleatoric, between-model and
 within-model parts.
+
+A catalogue of systems with different numbers of planets (P planets: P - 2 adjacent trios) is passed to ``summarize_instability``
+and ``survival`` as per-system trio counts instead of one ``n_trios``: system n owns the next counts[n] rows, system-major
+as before (``row_offsets``).
 """
 from __future__ import annotations
 
 import ctypes
+from typing import Optional
 
 import numpy as np
 import torch
@@ -34,8 +39,65 @@ def sample_instability(pred: torch.Tensor, seed: int = 0, row_offset: int = 0, l
     return t
 
 
-def summarize_instability(t: torch.Tensor, pred: torch.Tensor, n_trios: int = 1):
-    """t [N*n_trios, U], pred [N*n_trios, U, 2] -> [N, 8] (STAT_NAMES)."""
+def is_ragged(n_trios) -> bool:
+    """True when ``n_trios`` is per-system trio counts (a sequence, array or tensor with a dimension) rather than one
+    count for every system."""
+    if isinstance(n_trios, torch.Tensor):
+        return n_trios.dim() != 0
+    return not isinstance(n_trios, (int, np.integer)) and np.ndim(n_trios) != 0
+
+
+def row_offsets(counts, rows: Optional[int]) -> np.ndarray:
+    """Per-system trio counts c [N] of a catalogue of ``rows`` rows -> row offsets [0, cumsum(c)] (int64 [N + 1]): system
+    n owns rows off[n] .. off[n+1] - 1.  Raises ValueError when the counts are not 1-D, are empty, are not integers,
+    contain a count below 1, or do not sum to ``rows`` (not checked when ``rows`` is None)."""
+    if isinstance(counts, torch.Tensor):
+        counts = counts.detach().cpu().numpy()
+    c = np.asarray(counts)
+    if c.ndim != 1:
+        raise ValueError(f"trio counts must be 1-D, got shape {c.shape}")
+    if c.size == 0:
+        raise ValueError("trio counts are empty: a catalogue needs at least one system")
+    if c.dtype == np.bool_ or not np.issubdtype(c.dtype, np.integer):
+        raise ValueError(f"trio counts must be integers, got dtype {c.dtype}")
+    if (c < 1).any():
+        raise ValueError(f"every system needs at least one trio row, got a count of {int(c.min())}")
+    off = np.zeros(c.size + 1, np.int64)
+    np.cumsum(c, out=off[1:])
+    if rows is not None and off[-1] != rows:
+        raise ValueError(f"trio counts sum to {int(off[-1])} rows but there are {rows}")
+    return off
+
+
+def device_offsets(off: np.ndarray, device) -> torch.Tensor:
+    return torch.from_numpy(np.ascontiguousarray(off, np.int64)).to(device)
+
+
+def summarize_ragged(t: torch.Tensor, pred: torch.Tensor, d_off: torch.Tensor):
+    """``summarize_instability`` of the systems whose row offsets are the device int64 tensor d_off [n + 1], rows
+    counted from d_off[0] (``bnn_summarize_instability_ragged``; the offsets are trusted: validate them with
+    ``row_offsets``) -> [n, 8]."""
+    lib = _lib.load()
+    N, U = d_off.shape[0] - 1, t.shape[1]
+    stats = torch.empty((N, 8), device=t.device, dtype=torch.float32)
+    if N == 0:
+        return stats
+    with torch.cuda.device(t.device), _lib.nvtx("bnn:K7 summarize_instability"):
+        _lib.check(lib.bnn_summarize_instability_ragged(_lib.ptr(t), _lib.ptr(pred), N,
+                                                        _lib.dev_ptr(d_off, t.device, "row offsets", torch.int64), U,
+                                                        _lib.ptr(stats), _lib.current_stream_ptr()),
+                   "bnn_summarize_instability_ragged")
+    return stats
+
+
+def summarize_instability(t: torch.Tensor, pred: torch.Tensor, n_trios=1):
+    """t [N*n_trios, U], pred [N*n_trios, U, 2] -> [N, 8] (STAT_NAMES).  ``n_trios`` may also be per-system trio counts
+    [N] (1-D integers >= 1 summing to the rows of t; ``row_offsets``)."""
+    if is_ragged(n_trios):
+        off = row_offsets(n_trios, t.shape[0])
+        _lib.require_cuda(t, "t")
+        t, pred = t.contiguous().float(), pred.contiguous().float()
+        return summarize_ragged(t, pred, device_offsets(off, t.device))
     lib = _lib.load()
     _lib.require_cuda(t, "t")
     t, pred = t.contiguous().float(), pred.contiguous().float()
@@ -97,13 +159,40 @@ def survival_thresholds(thresholds) -> np.ndarray:
     return thr
 
 
-def survival(t: torch.Tensor, thresholds, n_trios: int = 1):
+def survival_ragged(t: torch.Tensor, thr: np.ndarray, d_off: torch.Tensor):
+    """``survival`` of the systems whose row offsets are the device int64 tensor d_off [n + 1], rows counted from
+    d_off[0] (``bnn_survival_instability_ragged``; thr as ``survival_thresholds`` returns it, the offsets trusted) ->
+    [n, J]."""
+    lib = _lib.load()
+    N, U = d_off.shape[0] - 1, t.shape[1]
+    surv = torch.empty((N, thr.size), device=t.device, dtype=torch.float32)
+    if N == 0:
+        return surv
+    h_thr = (ctypes.c_float * thr.size)(*thr.tolist())
+    with torch.cuda.device(t.device), _lib.nvtx("bnn:K7 survival_instability"):
+        _lib.check(lib.bnn_survival_instability_ragged(_lib.ptr(t), N,
+                                                       _lib.dev_ptr(d_off, t.device, "row offsets", torch.int64), U, h_thr,
+                                                       thr.size, _lib.ptr(surv), _lib.current_stream_ptr()),
+                   "bnn_survival_instability_ragged")
+    return surv
+
+
+def survival(t: torch.Tensor, thresholds, n_trios=1):
     """t [N*n_trios, U] sampled log10 instability times (``sample_instability``), thresholds [J] (log10 orbits, host
     values, rounded to fp32) -> [N, J]: the fraction of the U weight samples whose min over trios exceeds each
     threshold, S_j = #{u : min_r t > thr_j} / U.  S_j is a Monte Carlo estimate of P(T_inst > thr_j) with standard error
-    sqrt(S_j (1 - S_j) / U); it counts the same draws as ``summarize_instability``'s percentiles."""
+    sqrt(S_j (1 - S_j) / U); it counts the same draws as ``summarize_instability``'s percentiles.  ``n_trios`` may also
+    be per-system trio counts [N] (``row_offsets``)."""
     if t.dim() != 2:
         raise ValueError(f"t must be [N*n_trios, U], got {tuple(t.shape)}")
+    if is_ragged(n_trios):
+        off = row_offsets(n_trios, t.shape[0])
+        if t.shape[1] == 0:
+            raise ValueError("t has no units to count")
+        thr = survival_thresholds(thresholds)
+        _lib.require_cuda(t, "t")
+        t = t.contiguous().float()
+        return survival_ragged(t, thr, device_offsets(off, t.device))
     if int(n_trios) < 1:
         raise ValueError(f"n_trios must be >= 1, got {n_trios}")
     rows, U = t.shape

@@ -299,6 +299,25 @@ int bnn_score_labels(const float* d_pred, int64_t n_systems, int64_t n_units, co
 int bnn_survival_instability(const float* d_t, int64_t n_systems, int32_t n_trios, int64_t n_units,
                              const float* h_thresholds, int32_t n_thresholds, float* d_surv, void* stream);
 
+/* Catalogues of mixed planet counts: the same summary and survival for systems with different numbers of trio rows.
+ * d_row_offsets is a DEVICE int64 array [n_systems + 1]; system n owns the rows d_row_offsets[n] - d_row_offsets[0] ..
+ * d_row_offsets[n+1] - d_row_offsets[0] - 1 of d_t (and of d_pred), so its trio count is
+ * c[n] = d_row_offsets[n+1] - d_row_offsets[n], and the min over trios runs over those c[n] rows.  Rows are counted from
+ * d_row_offsets[0]: a slice of systems [a, b) of a catalogue passes a view of the catalogue's offsets (&off[a]) with its
+ * own d_t / d_pred rows, with no rebased copy.  With every c[n] = R the results equal bnn_summarize_instability /
+ * bnn_survival_instability with n_trios = R bit for bit, and a system's result depends on its own rows only.
+ * The offsets are NOT validated on the device (that would need a synchronisation): a system whose count is <= 0 gets a
+ * NaN row (all 8 statistics, all J survival columns), so such an offsets array has a defined result; offsets that are
+ * non-decreasing but run past the rows given read outside the block, and are the caller's to prevent (the Python layer
+ * validates the counts before it uploads them).  Variant choice (sort up to U = 32768, radix select beyond,
+ * bnn_set_summary_variant) is as for bnn_summarize_instability.  BNN_E_ARG as for the uniform entries plus a null
+ * d_row_offsets; BNN_E_ALIGN: d_row_offsets not 8-byte aligned (and, for survival, d_t / d_surv not 4-byte aligned);
+ * every check runs before the device is touched. */
+int bnn_summarize_instability_ragged(const float* d_t, const float* d_pred, int64_t n_systems, const int64_t* d_row_offsets,
+                                     int32_t n_units, float* d_stats, void* stream);
+int bnn_survival_instability_ragged(const float* d_t, int64_t n_systems, const int64_t* d_row_offsets, int64_t n_units,
+                                    const float* h_thresholds, int32_t n_thresholds, float* d_surv, void* stream);
+
 /* Variance decomposition of every row of the system-major block d_pred [n_rows, U, 2] (row = system * n_trios + trio).
  * Unit u = k * S + s is weight sample s of model k, S = units_per_model, M = U / S models; mu_{k,s} and sigma_{k,s} are
  * its predicted normal in log10 orbits.  With m_k = (1/S) sum_s mu_{k,s} and mean = (1/M) sum_k m_k, d_out [n_rows, 5]:
