@@ -23,7 +23,10 @@
 // and the epistemic part (variance of mu over the units) split into between-model and within-model parts.
 // [rows, U, 2] -> [rows, 5].
 //
-// The summary and survival kernels find a system's trio rows through a row map: UniformRows (every system has R rows,
+// Which trio sets each system's instability time: per trio row, the fraction of the U weight samples at which that trio
+// holds the system's min over trios (first such trio on ties), counted exactly.  [N*R, U] -> [N*R].
+//
+// The summary, survival and first-trio kernels find a system's trio rows through a row map: UniformRows (every system has R rows,
 // system n starts at row n*R) or RaggedRows (a catalogue of mixed planet counts: per-system row offsets in device
 // memory, system n owns rows off[n] - off[0] .. off[n+1] - off[0] - 1).  One template per kernel; the uniform entries
 // instantiate UniformRows.
@@ -503,6 +506,54 @@ __global__ void __launch_bounds__(SURV_THREADS) survival_kernel(const float* __r
     }
 }
 
+// ---- which trio sets the system's min: one CTA per system.  tmin[u] = fminf over the system's rows from +inf, as the
+// summary takes it; the winner of unit u is the first row r with t[r][u] == tmin[u], found as a running (best, index)
+// pair that a row takes over when it is strictly smaller, or when it is the first non-NaN row (so a +inf row can win).
+// A unit whose draws are all NaN has no winner.  Per-trio winner counts in one CTA-wide shared-memory histogram; integer
+// counts: a system's result depends on its own rows only and repeated calls are bit-identical.
+constexpr int FIRST_THREADS = 256, FIRST_UNROLL = 4, FIRST_MAXR = 1024;
+
+template <class Rows>
+__global__ void __launch_bounds__(FIRST_THREADS) first_trio_kernel(const float* __restrict__ t, Rows sys_rows, int64_t U,
+                                                                   float* __restrict__ first) {
+    __shared__ uint32_t hist[FIRST_MAXR];
+    const int tid = threadIdx.x;
+    const float INF = __int_as_float(0x7f800000);
+    const auto sp = sys_rows(blockIdx.x);
+    if (sp.count() <= 0) return;   // owns no rows: nothing to write (uniform in the CTA: nobody reaches a barrier)
+    float* __restrict__ out = first + sp.first();
+    if (sp.count() > FIRST_MAXR) {   // more trios than counters (ragged only: the uniform entry refuses it)
+        for (int64_t r = tid; r < sp.count(); r += FIRST_THREADS) out[r] = __int_as_float(0x7fffffff);
+        return;
+    }
+    const int R = (int)sp.count();
+    for (int i = tid; i < R; i += FIRST_THREADS) hist[i] = 0;
+    __syncthreads();
+    const float* __restrict__ rows = t + sp.first() * U;
+    // whole warps stay in the loop: hist_add_warp is warp-collective
+    for (int64_t u0 = 0; u0 < U; u0 += FIRST_THREADS * FIRST_UNROLL) {
+        float best[FIRST_UNROLL];
+        int idx[FIRST_UNROLL];
+#pragma unroll
+        for (int k = 0; k < FIRST_UNROLL; ++k) { best[k] = INF; idx[k] = -1; }
+        for (int r = 0; r < R; ++r) {   // FIRST_UNROLL independent coalesced loads in flight per trio row
+#pragma unroll
+            for (int k = 0; k < FIRST_UNROLL; ++k) {
+                const int64_t u = u0 + k * FIRST_THREADS + tid;
+                if (u < U) {
+                    const float v = rows[r * U + u];
+                    if (v < best[k] || (idx[k] < 0 && v == v)) { best[k] = v; idx[k] = r; }
+                }
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < FIRST_UNROLL; ++k)
+            hist_add_warp(hist, (uint32_t)idx[k], u0 + k * FIRST_THREADS + tid < U && idx[k] >= 0);
+    }
+    __syncthreads();
+    for (int r = tid; r < R; r += FIRST_THREADS) out[r] = (float)((double)hist[r] / (double)U);
+}
+
 // ---- variance decomposition: one CTA per prediction row, unit u = k*S + s of model k.  Pass 1: the units of a warp's
 // 32 lanes are consecutive, so their model indices are sorted and form a few contiguous segments; a segmented shuffle
 // scan sums each segment and its last lane adds the sum to the warp's own accumulator acc[warp][k] in shared memory.
@@ -791,6 +842,46 @@ int bnn_survival_instability_ragged(const float* d_t, int64_t n_systems, const i
     if (rc != BNN_OK) return rc;
     survival_kernel<<<(unsigned)n_systems, SURV_THREADS, 0, (cudaStream_t)stream>>>(d_t, RaggedRows{d_row_offsets}, n_units,
                                                                                      th, d_surv);
+    BNN_CUDA(cudaGetLastError());
+    return BNN_OK;
+}
+
+int bnn_first_trio_instability(const float* d_t, int64_t n_systems, int32_t n_trios, int64_t n_units, float* d_first,
+                               void* stream) {
+    using namespace bnn;
+    // argument checks first: they need no device
+    BNN_REQUIRE(d_t && d_first && n_systems > 0 && n_units > 0 && n_trios >= 1, BNN_E_ARG,
+                "bnn_first_trio_instability: null pointer or empty problem");
+    BNN_REQUIRE(n_trios <= FIRST_MAXR, BNN_E_ARG, "bnn_first_trio_instability: %d trios per system, at most %d supported",
+                (int)n_trios, FIRST_MAXR);
+    BNN_REQUIRE(n_systems < (1ll << 31) && n_units < (1ll << 32), BNN_E_ARG,
+                "bnn_first_trio_instability: n_systems must be < 2^31 and n_units < 2^32");
+    BNN_REQUIRE(aligned(d_t, 4) && aligned(d_first, 4), BNN_E_ALIGN,
+                "bnn_first_trio_instability: pointers must be 4-byte aligned");
+    int rc = check_device();
+    if (rc != BNN_OK) return rc;
+    first_trio_kernel<<<(unsigned)n_systems, FIRST_THREADS, 0, (cudaStream_t)stream>>>(d_t, UniformRows{n_trios}, n_units,
+                                                                                        d_first);
+    BNN_CUDA(cudaGetLastError());
+    return BNN_OK;
+}
+
+int bnn_first_trio_instability_ragged(const float* d_t, int64_t n_systems, const int64_t* d_row_offsets, int64_t n_units,
+                                      float* d_first, void* stream) {
+    using namespace bnn;
+    // argument checks first: they need no device
+    BNN_REQUIRE(d_t && d_first && d_row_offsets && n_systems > 0 && n_units > 0, BNN_E_ARG,
+                "bnn_first_trio_instability_ragged: null pointer or empty problem");
+    BNN_REQUIRE(n_systems < (1ll << 31) && n_units < (1ll << 32), BNN_E_ARG,
+                "bnn_first_trio_instability_ragged: n_systems must be < 2^31 and n_units < 2^32");
+    BNN_REQUIRE(aligned(d_t, 4) && aligned(d_first, 4), BNN_E_ALIGN,
+                "bnn_first_trio_instability_ragged: pointers must be 4-byte aligned");
+    BNN_REQUIRE(aligned(d_row_offsets, 8), BNN_E_ALIGN,
+                "bnn_first_trio_instability_ragged: d_row_offsets must be 8-byte aligned");
+    int rc = check_device();
+    if (rc != BNN_OK) return rc;
+    first_trio_kernel<<<(unsigned)n_systems, FIRST_THREADS, 0, (cudaStream_t)stream>>>(d_t, RaggedRows{d_row_offsets},
+                                                                                        n_units, d_first);
     BNN_CUDA(cudaGetLastError());
     return BNN_OK;
 }

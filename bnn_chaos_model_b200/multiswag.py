@@ -551,7 +551,7 @@ class MultiSWAG:
 
     @staticmethod
     def _check_reduce(x: torch.Tensor, samples_per_model: int, n_trios, y=None, thresholds=None,
-                      uncertainty=False):
+                      uncertainty=False, trios=False):
         """Argument checks of ``_reduce`` / ``_reduce_sharded``, before any device work.  Returns the thresholds as
         ``posterior.survival_thresholds`` (or None)."""
         from . import posterior
@@ -561,9 +561,11 @@ class MultiSWAG:
             if y is not None:
                 raise ValueError("held-out scoring takes one trio per system: pass an int n_trios = 1 with labels")
             posterior.row_offsets(n_trios, None)
+        if trios:
+            posterior.check_trio_counts(n_trios, None)
         if y is not None:
             MultiSWAG._check_labelled(x, y, samples_per_model)
-        if thresholds is None and not uncertainty and not ragged:
+        if thresholds is None and not uncertainty and not trios and not ragged:
             return None
         if x.dim() != 3:
             raise ValueError(f"x must be [N*n_trios, T, F], got {tuple(x.shape)}")
@@ -584,23 +586,25 @@ class MultiSWAG:
             posterior.row_offsets(n_trios, x.shape[0])
 
     def _reduce(self, x, samples_per_model, n_trios=1, seed=0, scale=0.5, system_offset=0, max_block_bytes=640 << 20,
-                unit_chunk=None, y=None, thresholds=None, uncertainty=False, row_offset=0, first_row=0):
+                unit_chunk=None, y=None, thresholds=None, uncertainty=False, row_offset=0, first_row=0, trios=False):
         """One walk over the prediction block (``_walk_prediction_chunks``) that reduces every system chunk on the device
         and returns [summary [N, 8]] + [score [N, 2]] if labels y are given + [survival [N, J]] if thresholds are given
-        + [uncertainty [N, n_trios, 5]] if ``uncertainty`` is set.  Each chunk's instability times are sampled once and
-        feed both the summary and the survival counts; the uncertainty decomposes the same prediction block.
+        + [uncertainty [N, n_trios, 5]] if ``uncertainty`` is set + [first [N, n_trios], trio_summary [N, n_trios, 8]]
+        if ``trios`` is set.  Each chunk's instability times are sampled once and feed the summary, the survival counts,
+        the first-trio counts and the per-trio summary (``summarize_instability`` with one trio per row); the uncertainty
+        decomposes the same prediction block.
 
         With per-system trio counts ``n_trios`` [N] (a catalogue, no labels) the systems own the rows first_row ..
         first_row + sum(n_trios) - 1 of x, any rows around them are context (``catalogue_shard_range``), ``row_offset``
-        is the global row of x's first row (it keys the Philox draws; ``system_offset`` must be 0), and the uncertainty
-        is [sum(n_trios), 5] in row order."""
+        is the global row of x's first row (it keys the Philox draws; ``system_offset`` must be 0), and the per-row
+        outputs are in row order: uncertainty [sum(n_trios), 5], first [sum(n_trios)], trio_summary [sum(n_trios), 8]."""
         from . import posterior
 
         ragged = posterior.is_ragged(n_trios)
         if ragged and system_offset:
             raise ValueError("with per-system trio counts system_offset must be 0: split a catalogue with the _sharded "
                              "methods")
-        thr = self._check_reduce(x, samples_per_model, n_trios, y, thresholds, uncertainty)
+        thr = self._check_reduce(x, samples_per_model, n_trios, y, thresholds, uncertainty, trios)
         off = None
         if ragged:
             off = posterior.row_offsets(n_trios, None) + int(first_row)
@@ -612,7 +616,8 @@ class MultiSWAG:
         else:
             N = x.shape[0] // n_trios
         outs = [torch.empty((N, 8), device=self.device)]
-        i_score = i_surv = i_unc = None
+        i_score = i_surv = i_unc = i_first = None
+        per_row = lambda *tail: (int(off[-1] - off[0]),) + tail if ragged else (N, n_trios) + tail
         if y is not None:
             i_score = len(outs)
             outs.append(torch.empty((N, 2), device=self.device))
@@ -621,18 +626,25 @@ class MultiSWAG:
             outs.append(torch.empty((N, thr.size), device=self.device))
         if uncertainty:
             i_unc = len(outs)
-            outs.append(torch.empty((int(off[-1] - off[0]), 5) if ragged else (N, n_trios, 5), device=self.device))
+            outs.append(torch.empty(per_row(5), device=self.device))
+        if trios:
+            i_first = len(outs)
+            outs.append(torch.empty(per_row(), device=self.device))
+            outs.append(torch.empty(per_row(8), device=self.device))
 
         def consume(lo, hi, row0, pred):
             t = posterior.sample_instability(pred, seed, row_offset=row0)
             if ragged:
                 d = d_off[lo:hi + 1]   # rows counted from d[0]: the chunk's first row
+                a, b = int(off[lo] - off[0]), int(off[hi] - off[0])
                 outs[0][lo:hi] = posterior.summarize_ragged(t, pred, d)
                 if i_surv is not None:
                     outs[i_surv][lo:hi] = posterior.survival_ragged(t, thr, d)
                 if i_unc is not None:
-                    a = int(off[lo] - off[0])
-                    outs[i_unc][a:a + pred.shape[0]] = posterior.uncertainty(pred, samples_per_model)
+                    outs[i_unc][a:b] = posterior.uncertainty(pred, samples_per_model)
+                if i_first is not None:
+                    outs[i_first][a:b] = posterior.first_trio_ragged(t, d)
+                    outs[i_first + 1][a:b] = posterior.summarize_instability(t, pred, 1)
                 return
             outs[0][lo:hi] = posterior.summarize_instability(t, pred, n_trios)
             if i_score is not None:
@@ -641,27 +653,30 @@ class MultiSWAG:
                 outs[i_surv][lo:hi] = posterior.survival(t, thr, n_trios)
             if i_unc is not None:
                 outs[i_unc][lo:hi] = posterior.uncertainty(pred, samples_per_model).view(hi - lo, n_trios, 5)
+            if i_first is not None:
+                outs[i_first][lo:hi] = posterior.first_trio(t, n_trios)
+                outs[i_first + 1][lo:hi] = posterior.summarize_instability(t, pred, 1).view(hi - lo, n_trios, 8)
 
         self._walk_prediction_chunks(x, samples_per_model, n_trios, seed, scale, system_offset, max_block_bytes, unit_chunk,
                                      consume, off=off, row_offset=row_offset)
         return outs
 
     def _reduce_sharded(self, x_local, n_total, samples_per_model, n_trios=1, seed=0, scale=0.5, group=None, y=None,
-                        thresholds=None, uncertainty=False):
+                        thresholds=None, uncertainty=False, trios=False):
         """``_reduce`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE all_gather
-        moves the concatenated columns [N, 8 (+ 2) (+ J) (+ 5 n_trios)].  Returns the same list, [n_total, ...] each, on
-        every rank.
+        moves the concatenated columns [N, 8 (+ 2) (+ J) (+ 5 n_trios) (+ 9 n_trios)].  Returns the same list,
+        [n_total, ...] each, on every rank.
 
         A catalogue passes the trio counts of the WHOLE catalogue [n_total] as ``n_trios`` and, on each rank, the rows
         [row_lo, row_hi) of ``catalogue_shard_range`` as x_local; one all_gather moves the per-system columns and, with
-        ``uncertainty``, a second one the per-row uncertainty [rows, 5]."""
+        ``uncertainty`` or ``trios``, a second one the per-row outputs [rows, (5) (+ 1 + 8)]."""
         import math
 
         import torch.distributed as dist
 
         from . import posterior
 
-        thr = self._check_reduce(x_local, samples_per_model, n_trios, y, thresholds, uncertainty)
+        thr = self._check_reduce(x_local, samples_per_model, n_trios, y, thresholds, uncertainty, trios)
         world = dist.get_world_size(group) if dist.is_initialized() else 1
         rank = dist.get_rank(group) if dist.is_initialized() else 0
         g = self.system_granule(x_local.shape[1])
@@ -677,22 +692,28 @@ class MultiSWAG:
                                  f"but was given {x_local.shape[0]} rows")
             if shi > slo:
                 outs = self._reduce(x_local, samples_per_model, counts[slo:shi], seed, scale, thresholds=thresholds,
-                                    uncertainty=uncertainty, row_offset=rlo, first_row=int(off[slo]) - rlo)
+                                    uncertainty=uncertainty, row_offset=rlo, first_row=int(off[slo]) - rlo, trios=trios)
             else:   # an empty shard: more ranks than systems
                 outs = [torch.empty((0, 8), device=self.device)]
                 if thr is not None:
                     outs.append(torch.empty((0, thr.size), device=self.device))
                 if uncertainty:
                     outs.append(torch.empty((0, 5), device=self.device))
+                if trios:
+                    outs += [torch.empty((0,), device=self.device), torch.empty((0, 8), device=self.device)]
             if world == 1:
                 return outs
-            cols = outs[:-1] if uncertainty else outs
+            n_rows = int(uncertainty) + 2 * int(trios)   # the per-row outputs close the list
+            cols, rows = outs[:len(outs) - n_rows], outs[len(outs) - n_rows:]
             widths = [o.shape[1] for o in cols]
             full = gather_system_shards(torch.cat(cols, 1), n_total, group, bounds=[(a, b) for a, b, _, _ in shards])
             res = [c.contiguous() for c in torch.split(full, widths, 1)]
-            if uncertainty:
-                res.append(gather_system_shards(outs[-1], int(off[-1]), group,
-                                                bounds=[(int(off[a]), int(off[b])) for a, b, _, _ in shards]))
+            if rows:
+                tails = [tuple(o.shape[1:]) for o in rows]
+                widths = [math.prod(t) for t in tails]
+                full = gather_system_shards(torch.cat([o.reshape(o.shape[0], w) for o, w in zip(rows, widths)], 1),
+                                            int(off[-1]), group, bounds=[(int(off[a]), int(off[b])) for a, b, _, _ in shards])
+                res += [c.contiguous().view((int(off[-1]),) + t) for c, t in zip(torch.split(full, widths, 1), tails)]
             return res
         granule = g // math.gcd(g, n_trios)  # shard boundaries in SYSTEMS such that rows stay granule-aligned
         lo, hi = shard_range(n_total, rank, world, granule)
@@ -700,7 +721,7 @@ class MultiSWAG:
             raise ValueError(f"rank {rank} owns systems [{lo}, {hi}) of {n_total} but was given "
                              f"{x_local.shape[0]} rows of {n_trios} trios")
         outs = self._reduce(x_local, samples_per_model, n_trios, seed, scale, system_offset=lo, y=y, thresholds=thresholds,
-                            uncertainty=uncertainty)
+                            uncertainty=uncertainty, trios=trios)
         if world == 1:
             return outs
         tails = [tuple(o.shape[1:]) for o in outs]
@@ -783,6 +804,34 @@ class MultiSWAG:
         summary, unc = self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale, group,
                                             uncertainty=True)
         return summary, unc
+
+    def posterior_trios(self, x: torch.Tensor, samples_per_model: int, n_trios=1, seed: int = 0, scale: float = 0.5,
+                        system_offset: int = 0, max_block_bytes: int = 640 << 20, unit_chunk: Optional[int] = None):
+        """Which trio goes unstable first: x [N*n_trios, T, F] (as ``posterior_summary``) -> (summary [N, 8],
+        first [N, n_trios], trio_summary [N, n_trios, 8]).  ``summary`` is exactly ``posterior_summary`` with the same
+        arguments.  first[n, r] is the fraction of the U = n_models * samples_per_model sampled instability times of
+        system n at which trio r holds the system's min over trios (``posterior.first_trio``: ties go to the earlier
+        trio, a unit whose draws are all NaN has no winner).  trio_summary[n, r] is the posterior summary
+        (``posterior.STAT_NAMES``) of trio r on its own, exactly ``posterior_summary`` with n_trios = 1 on the same rows.
+        All three come from the same sampled times, one system chunk at a time, so the predictive kernel runs once;
+        none depends on the chunking or on a split into shards with ``system_offset``.  With per-system trio counts
+        ``n_trios`` (as in ``posterior_summary``) first is [rows] and trio_summary [rows, 8] in x's row order.  At most
+        ``posterior.MAX_TRIOS_PER_SYSTEM`` trios per system (ValueError before any device work)."""
+        self._check_catalogue(x, n_trios)
+        summary, first, trio_summary = self._reduce(x, samples_per_model, n_trios, seed, scale, system_offset,
+                                                    max_block_bytes, unit_chunk, trios=True)
+        return summary, first, trio_summary
+
+    def posterior_trios_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int, n_trios=1,
+                                seed: int = 0, scale: float = 0.5, group=None):
+        """``posterior_trios`` with the systems block-partitioned over ranks like ``posterior_summary_sharded``; ONE
+        all_gather moves [N, 8 + 9 n_trios] (summary | first | trio_summary).  Returns (summary [n_total, 8], first
+        [n_total, n_trios], trio_summary [n_total, n_trios, 8]) on every rank.  A catalogue passes the trio counts of the
+        whole catalogue and its ``catalogue_shard_range`` rows; a second all_gather then moves first and trio_summary
+        [rows, 1 + 8]."""
+        summary, first, trio_summary = self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale,
+                                                            group, trios=True)
+        return summary, first, trio_summary
 
     def posterior_summary_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int, n_trios: int = 1,
                                   seed: int = 0, scale: float = 0.5, group=None):

@@ -5,10 +5,10 @@ resampling of draws >= 9 from the analytic prior, min over trios, per-system med
 (figures/main_figures.py:167-277, figures/multiswag_5_planet.py:306-481) -- so that only ``[N, 8]`` leaves the
 device instead of the ``[N, U, 2]`` prediction block.  ``survival`` counts the same sampled times against thresholds:
 P(T_inst > t) per system.  ``uncertainty`` splits each row's predictive variance into aleatoric, between-model and
-within-model parts.
+within-model parts.  ``first_trio`` counts, per trio, how often it is the one that sets its system's min.
 
-A catalogue of systems with different numbers of planets (P planets: P - 2 adjacent trios) is passed to ``summarize_instability``
-and ``survival`` as per-system trio counts instead of one ``n_trios``: system n owns the next counts[n] rows, system-major
+A catalogue of systems with different numbers of planets (P planets: P - 2 adjacent trios) is passed to ``summarize_instability``,
+``survival`` and ``first_trio`` as per-system trio counts instead of one ``n_trios``: system n owns the next counts[n] rows, system-major
 as before (``row_offsets``).
 """
 from __future__ import annotations
@@ -213,6 +213,74 @@ def survival(t: torch.Tensor, thresholds, n_trios=1):
         _lib.check(lib.bnn_survival_instability(_lib.ptr(t), N, int(n_trios), U, h_thr, thr.size, _lib.ptr(surv),
                                                 _lib.current_stream_ptr()), "bnn_survival_instability")
     return surv
+
+
+MAX_TRIOS_PER_SYSTEM = 1024
+
+
+def first_trio_ragged(t: torch.Tensor, d_off: torch.Tensor):
+    """``first_trio`` of the systems whose row offsets are the device int64 tensor d_off [n + 1], rows counted from
+    d_off[0] (``bnn_first_trio_instability_ragged``; the offsets are trusted: validate them with ``row_offsets`` and
+    ``MAX_TRIOS_PER_SYSTEM``, and they must cover the rows of t) -> [rows of t] in row order."""
+    lib = _lib.load()
+    N, U = d_off.shape[0] - 1, t.shape[1]
+    first = torch.empty((t.shape[0],), device=t.device, dtype=torch.float32)
+    if N == 0:
+        return first
+    with torch.cuda.device(t.device), _lib.nvtx("bnn:K7 first_trio_instability"):
+        _lib.check(lib.bnn_first_trio_instability_ragged(_lib.ptr(t), N,
+                                                         _lib.dev_ptr(d_off, t.device, "row offsets", torch.int64), U,
+                                                         _lib.ptr(first), _lib.current_stream_ptr()),
+                   "bnn_first_trio_instability_ragged")
+    return first
+
+
+def check_trio_counts(n_trios, rows: Optional[int]) -> Optional[np.ndarray]:
+    """The trio layout of ``first_trio``: the row offsets of per-system counts (``row_offsets``), or None for an int
+    ``n_trios`` (checked to be >= 1 and to divide ``rows`` when given).  Raises ValueError when a system has more than
+    ``MAX_TRIOS_PER_SYSTEM`` trios."""
+    if is_ragged(n_trios):
+        off = row_offsets(n_trios, rows)
+        if int(np.diff(off).max()) > MAX_TRIOS_PER_SYSTEM:
+            raise ValueError(f"a system has {int(np.diff(off).max())} trios: at most {MAX_TRIOS_PER_SYSTEM} are supported")
+        return off
+    if int(n_trios) < 1:
+        raise ValueError(f"n_trios must be >= 1, got {n_trios}")
+    if int(n_trios) > MAX_TRIOS_PER_SYSTEM:
+        raise ValueError(f"n_trios = {n_trios}: at most {MAX_TRIOS_PER_SYSTEM} trios per system are supported")
+    if rows is not None and rows % int(n_trios):
+        raise ValueError(f"{rows} rows are not a multiple of {n_trios} trios")
+    return None
+
+
+def first_trio(t: torch.Tensor, n_trios=1):
+    """t [N*n_trios, U] sampled log10 instability times (``sample_instability``) -> which trio sets each system's
+    instability time: first[r] = the fraction of the U weight samples at which trio row r holds its system's min over
+    trios (fmin from +inf, as ``summarize_instability`` takes it).  Ties go to the earlier trio, +inf is an ordinary value
+    and a unit whose draws are all NaN has no winner, so a system's fractions sum to 1 minus its share of all-NaN units.
+    Counted exactly, each count divided by U in double and rounded once.  [N, n_trios] for an int ``n_trios``; with
+    per-system trio counts [N] (``row_offsets``) [rows] in row order.  At most ``MAX_TRIOS_PER_SYSTEM`` trios per
+    system."""
+    if t.dim() != 2:
+        raise ValueError(f"t must be [N*n_trios, U], got {tuple(t.shape)}")
+    rows, U = t.shape
+    off = check_trio_counts(n_trios, rows)
+    if U == 0:
+        raise ValueError("t has no units to count")
+    _lib.require_cuda(t, "t")
+    t = t.contiguous().float()
+    if off is not None:
+        return first_trio_ragged(t, device_offsets(off, t.device))
+    lib = _lib.load()
+    R = int(n_trios)
+    N = rows // R
+    first = torch.empty((N, R), device=t.device, dtype=torch.float32)
+    if N == 0:
+        return first
+    with torch.cuda.device(t.device), _lib.nvtx("bnn:K7 first_trio_instability"):
+        _lib.check(lib.bnn_first_trio_instability(_lib.ptr(t), N, R, U, _lib.ptr(first), _lib.current_stream_ptr()),
+                   "bnn_first_trio_instability")
+    return first
 
 
 UNCERTAINTY_NAMES = ("mean_mu", "aleatoric", "epistemic", "between_models", "within_models")

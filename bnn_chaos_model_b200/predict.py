@@ -8,6 +8,7 @@ counts): per system the posterior summary [N, 8] (``posterior.STAT_NAMES``) of t
 
     python -m bnn_chaos_model_b200.predict --models DIR/*_output.pkl --data catalogue.npz --samples 100 --out OUT
     python -m bnn_chaos_model_b200.predict --models DIR/*_output.pkl --synthetic 2000 --survival 6 9 --uncertainty --out OUT
+    python -m bnn_chaos_model_b200.predict --models DIR/*_output.pkl --data catalogue.npz --trios --out OUT
     python -m torch.distributed.run --nproc-per-node 8 -m bnn_chaos_model_b200.predict --models ... --out OUT
 
 ``catalogue.npz`` holds ``n_trios`` [N] (trio rows per system, >= 1; system n owns the next n_trios[n] rows) and exactly
@@ -21,7 +22,12 @@ Writes to ``--out``:
   * ``per_system.npz``: ``summary`` [N, 8], ``stat_names``, ``n_trios``; with ``--survival T [T ...]`` (log10 orbits)
     ``survival`` [N, J] = P(T_inst > T) per system and ``thresholds``; with ``--uncertainty`` ``uncertainty`` [R, 5] per
     trio row (aleatoric, between-model and within-model parts of the predictive variance) and ``uncertainty_names``;
-  * ``summary.json``: the settings, the number of systems per trio count and, with ``--survival``, ``survival_mean``.
+    with ``--trios`` ``trio_first`` [R], per trio row the fraction of the weight samples at which that trio sets its
+    system's minimum (which trio goes unstable first), ``trio_summary`` [R, 8], the posterior summary of each trio on
+    its own, and ``trio_stat_names``;
+  * ``summary.json``: the settings, the number of systems per trio count, with ``--survival`` ``survival_mean`` and,
+    with ``--trios``, ``weakest_trio_position``: for each trio count k >= 2, how many of the systems of k trios have
+    their largest ``trio_first`` at position 0 .. k - 1 (ties go to the first position).
 Under torchrun each rank reduces a contiguous block of systems balanced by rows (``catalogue_shard_range``), the
 results are gathered and rank 0 writes the files; they are the same files as from one GPU.
 """
@@ -54,6 +60,9 @@ def build_parser():
     ap.add_argument("--uncertainty", action="store_true",
                     help="also split each trio row's predictive variance into aleatoric, between-model and within-model "
                          "parts")
+    ap.add_argument("--trios", action="store_true",
+                    help="also report, per trio row, how often that trio sets its system's instability time and its own "
+                         "posterior summary")
     return ap
 
 
@@ -104,12 +113,25 @@ def model_inputs(inputs, lo: int, hi: int, dev) -> torch.Tensor:
     return data_setup_kernel(torch.from_numpy(np.ascontiguousarray(inputs["masses"][lo:hi])).to(dev), ts)
 
 
+def weakest_trio_position(first: np.ndarray, counts: np.ndarray) -> dict:
+    """{str(k): [systems of k trios whose largest first-trio fraction is at position 0, 1, .., k - 1]} for every trio
+    count k >= 2 in the catalogue; ties go to the first position (numpy argmax)."""
+    off = np.concatenate([[0], np.cumsum(counts)])
+    res = {}
+    for k in np.unique(counts):
+        if k < 2:
+            continue
+        rows = off[:-1][counts == k][:, None] + np.arange(k)[None, :]
+        res[str(int(k))] = np.bincount(first[rows].argmax(1), minlength=int(k)).tolist()
+    return res
+
+
 def main(argv=None):
     """Returns the summary dict on rank 0 (None on the other ranks)."""
     import torch.distributed as dist
 
     from .multiswag import catalogue_shard_range, load_ensemble
-    from .posterior import STAT_NAMES, UNCERTAINTY_NAMES, survival_thresholds
+    from .posterior import STAT_NAMES, UNCERTAINTY_NAMES, check_trio_counts, survival_thresholds
 
     args = build_parser().parse_args(argv)
     if args.survival is not None:
@@ -117,6 +139,8 @@ def main(argv=None):
     if args.samples < 1:
         raise ValueError(f"--samples must be >= 1, got {args.samples}")
     counts, inputs = load_catalogue(args)
+    if args.trios:
+        check_trio_counts(counts, None)   # at most MAX_TRIOS_PER_SYSTEM trios per system
     N, R = counts.size, int(counts.sum())
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -125,15 +149,16 @@ def main(argv=None):
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     ens = load_ensemble(args.models, device=dev)
-    # summary, (with --survival) survival and (with --uncertainty) uncertainty come from one walk, in that order
+    # summary, (with --survival) survival, (with --uncertainty) uncertainty and (with --trios) the first-trio fractions
+    # and per-trio summary come from one walk, in that order
     if world > 1:
         T = (inputs["x"] if "x" in inputs else inputs["tseries"]).shape[1]
         _, _, lo, hi = catalogue_shard_range(counts, dist.get_rank(), world, ens.system_granule(T))
         outs = ens._reduce_sharded(model_inputs(inputs, lo, hi, dev), N, args.samples, counts, args.seed, args.scale,
-                                   thresholds=args.survival, uncertainty=args.uncertainty)
+                                   thresholds=args.survival, uncertainty=args.uncertainty, trios=args.trios)
     else:
         outs = ens._reduce(model_inputs(inputs, 0, R, dev), args.samples, counts, args.seed, args.scale,
-                           thresholds=args.survival, uncertainty=args.uncertainty)
+                           thresholds=args.survival, uncertainty=args.uncertainty, trios=args.trios)
     info = None
     if world == 1 or dist.get_rank() == 0:
         summary = outs[0].cpu().numpy()
@@ -149,7 +174,12 @@ def main(argv=None):
             arrays.update(survival=surv, thresholds=survival_thresholds(args.survival))
             info["survival_mean"] = [float(v) for v in surv.astype(np.float64).mean(0)]
         if args.uncertainty:
-            arrays.update(uncertainty=outs[-1].cpu().numpy(), uncertainty_names=np.array(UNCERTAINTY_NAMES))
+            arrays.update(uncertainty=outs[1 + (args.survival is not None)].cpu().numpy(),
+                          uncertainty_names=np.array(UNCERTAINTY_NAMES))
+        if args.trios:
+            first = outs[-2].cpu().numpy()
+            arrays.update(trio_first=first, trio_summary=outs[-1].cpu().numpy(), trio_stat_names=np.array(STAT_NAMES))
+            info["weakest_trio_position"] = weakest_trio_position(first, counts)
         os.makedirs(args.out, exist_ok=True)
         with open(os.path.join(args.out, "summary.json"), "w") as f:
             json.dump(info, f, indent=1)

@@ -318,6 +318,25 @@ int bnn_summarize_instability_ragged(const float* d_t, const float* d_pred, int6
 int bnn_survival_instability_ragged(const float* d_t, int64_t n_systems, const int64_t* d_row_offsets, int64_t n_units,
                                     const float* h_thresholds, int32_t n_thresholds, float* d_surv, void* stream);
 
+/* Which trio sets each system's instability time, from the sampled times d_t [rows, U] that bnn_sample_instability
+ * writes.  tmin[n,u] is the min over system n's trio rows exactly as bnn_summarize_instability takes it (fminf from
+ * +inf).  The winner at unit u is the FIRST of the system's rows r with t[r,u] == tmin[n,u] (ties go to the earlier
+ * trio; +inf is an ordinary value, so when every non-NaN draw is +inf the first +inf row wins); a unit whose draws are
+ * all NaN has no winner.  For each trio row r of system n:
+ *   d_first [rows]:  first[r] = #{u : r wins unit u} / U,
+ * the count exact, converted once as (float)((double)count / U); so sum_r first[r] = (U - #all-NaN units) / U.  Rows
+ * are system-major: system * n_trios + trio for the uniform entry, the offsets' rows for the ragged one (counted from
+ * d_row_offsets[0] as in bnn_survival_instability_ragged, so a slice of systems passes a view of the catalogue's
+ * offsets and its own d_t / d_first rows).  A system's result depends on its own rows only, and repeated calls are
+ * bit-identical.  At most 1024 trio rows per system: a ragged system with a larger count gets NaN rows, one with a count
+ * <= 0 owns no rows and nothing is written.  d_t and d_first need only 4-byte alignment.  BNN_E_ARG: null pointer,
+ * n_systems <= 0 or >= 2^31, n_units <= 0 or >= 2^32, n_trios < 1 or > 1024; BNN_E_ALIGN: d_t / d_first not 4-byte or
+ * d_row_offsets not 8-byte aligned; every check runs before the device is touched. */
+int bnn_first_trio_instability(const float* d_t, int64_t n_systems, int32_t n_trios, int64_t n_units, float* d_first,
+                               void* stream);
+int bnn_first_trio_instability_ragged(const float* d_t, int64_t n_systems, const int64_t* d_row_offsets, int64_t n_units,
+                                      float* d_first, void* stream);
+
 /* Variance decomposition of every row of the system-major block d_pred [n_rows, U, 2] (row = system * n_trios + trio).
  * Unit u = k * S + s is weight sample s of model k, S = units_per_model, M = U / S models; mu_{k,s} and sigma_{k,s} are
  * its predicted normal in log10 orbits.  With m_k = (1/S) sum_s mu_{k,s} and mean = (1/M) sum_k m_k, d_out [n_rows, 5]:
