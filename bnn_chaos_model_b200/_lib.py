@@ -139,6 +139,12 @@ SIGNATURES = {
     "bnn_decompose_uncertainty": (C.c_int, [c_f32p, C.c_int64, C.c_int64, C.c_int64, c_f32p, C.c_void_p]),
     "bnn_saliency": (C.c_int, [_CFG, C.c_int32, c_f32p, c_f32p, C.c_int64, c_f32p, C.c_uint64, c_f32p, c_f32p, c_f32p,
                                C.c_void_p, C.c_void_p]),
+    "bnn_posterior_saliency_workspace_bytes": (C.c_size_t, [_CFG, C.c_int32, C.c_int64]),
+    "bnn_posterior_saliency": (
+        C.c_int,
+        [_CFG, C.c_int32, c_f32p, C.c_int64, c_f32p, C.c_int64, C.c_int64, C.c_uint64, C.c_void_p, C.c_int32, C.c_int64,
+         c_f32p, c_f32p, c_f32p, C.c_void_p, C.c_void_p],
+    ),
 }
 
 # diagnostics declared in include/bnnchaos_diag.h (probes / timers; not part of the product ABI)

@@ -414,6 +414,136 @@ static int train_gradient(const char* who, bool state_ok, const char* state_name
     return BNN_OK;
 }
 
+// The saliency launch of the v3 kernel (no input noise, no summary noise, upstream gradient (1, 0)) shared by
+// bnn_saliency and bnn_posterior_saliency: n_models weight vectors [n_models, d] over B systems, grid (n_cta, n_models)
+// with n_cta = SMs / n_models CTAs per model (one wave), at most one per pair of systems.  The caller has checked the
+// arguments and the device.  Workspace: the CTAs' partials [n_models, n_cta, d + DPAD] (the saliency sums of squares
+// sit in the dlv_in slot), then the producer warps' input-tile scratch.
+static int64_t saliency_ctas(int32_t n_models, int64_t B) {
+    int64_t n_cta = sm_count() / n_models;
+    if (n_cta > (B + 1) / 2) n_cta = (B + 1) / 2;
+    if (n_cta < 1) n_cta = 1;
+    return n_cta;
+}
+// Sized for every call of at most n_models weight vectors and B systems, not just this one: n' * saliency_ctas(n', B')
+// is not monotone (9 units over 31 systems run 144 CTAs, 10 run 140), so a walk that sizes its workspace for its full
+// chunk and reuses it for a smaller remainder needs the bound.  n' * ctas <= max(n', SMs) (SMs / n' CTAs each up to SMs
+// units, one each beyond) and <= n' * ceil(B' / 2), both non-decreasing in n' and B'.
+static size_t saliency_workspace_floats(const bnn_model_config* cfg, int32_t n_models, int64_t B) {
+    const int64_t sms = sm_count();
+    int64_t n = n_models > sms ? n_models : sms;
+    if (n > (int64_t)n_models * ((B + 1) / 2)) n = (int64_t)n_models * ((B + 1) / 2);
+    return (size_t)n * (FlatLayout(cfg->n_features).d + DPAD) + 4 + (size_t)n * scratch_floats_per_cta(cfg);
+}
+static int saliency_launch(const bnn_model_config* cfg, int32_t n_models, const float* d_theta, const float* d_x, int64_t B,
+                           const float* d_eps12, uint64_t seed, float* d_grad_x, float* d_mu, void* d_workspace,
+                           cudaStream_t st, const float** partial_out, int* n_cta_out) {
+    const int F = cfg->n_features, T = cfg->n_times;
+    const FlatLayout fl(F);
+    const int64_t n_cta = saliency_ctas(n_models, B);
+    const int DP = fl.d + DPAD;
+    float* partial = (float*)d_workspace;
+    float* xprod = partial + (size_t)n_models * n_cta * DP;
+    xprod += (4 - ((uintptr_t)xprod / sizeof(float)) % 4) % 4;
+    Params prm;
+    prm.theta = d_theta; prm.X = d_x; prm.Y = nullptr; prm.batch_index = nullptr;
+    prm.eps_in = nullptr; prm.eps12 = d_eps12; prm.eps_sum = nullptr;
+    prm.partial = partial; prm.head_rec = nullptr; prm.xprod = xprod;
+    prm.B = (int)B; prm.T = T; prm.F = F; prm.FP = (F + 3) & ~3; prm.n_cta = (int)n_cta; prm.seed0 = 0;
+    prm.seed = seed; prm.step = 0; prm.zero_mask = cfg->zero_mask;
+    prm.hc = HeadConsts{cfg->lo_mu, cfg->hi_mu, cfg->lo_sd, cfg->hi_sd};
+    prm.beta_out = 0.f;
+    prm.saliency = 1; prm.gx_out = d_grad_x; prm.mu_out = d_mu;
+    static PerDeviceOnce attr_done;
+    if (attr_done.need()) {
+        BNN_CUDA(cudaFuncSetAttribute(train_fwd_bwd3_kernel<100, 41>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      227 * 1024));
+    }
+    const size_t smem3 = (size_t)Smem3(T, F).total * sizeof(float);
+    train_fwd_bwd3_kernel<100, 41><<<dim3((unsigned)n_cta, n_models), NTHR3, smem3, st>>>(prm);
+    BNN_CUDA(cudaGetLastError());
+    if (partial_out) *partial_out = partial;
+    if (n_cta_out) *n_cta_out = (int)n_cta;
+    return BNN_OK;
+}
+
+// ---- posterior attribution (bnn_posterior_saliency) ----
+constexpr int ATTR_ROUNDS = S2 / 4;   // float4 blocks of eps1 | eps2 per (unit, row)
+
+// eps12[u][r] = eps1 | eps2 of unit unit0 + u and row row0 + r, exactly the draws of the predictive kernel's Philox path
+// (predict_tc.cuh, tail_draw_eps): block blk of counter (blk, global unit, global row, STREAM_EPS) under the raw seed.
+__global__ void __launch_bounds__(256) attr_eps_kernel(int64_t n, int64_t rows, uint64_t seed, int64_t unit0, int64_t row0,
+                                                       float* __restrict__ eps12) {
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    const int64_t ur = i / ATTR_ROUNDS;
+    const int blk = (int)(i - ur * ATTR_ROUNDS);
+    const int64_t u = ur / rows, r = ur - u * rows;
+    reinterpret_cast<float4*>(eps12)[i] =
+        philox_normal4(seed, STREAM_EPS, (uint32_t)(unit0 + u), (uint32_t)(row0 + r), (uint32_t)blk);
+}
+
+// One (unit, row, column) per thread: part[u][r] = (sum_t g[t][c]^2 for c < F | sum_t g[t][c] | mu) in double, t in
+// increasing order.  A warp reads runs of consecutive columns of the same time step.
+__global__ void __launch_bounds__(256) attr_unit_sums_kernel(const float* __restrict__ g, const float* __restrict__ mu,
+                                                             int64_t n, int T, int F, double* __restrict__ part) {
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    const int64_t ur = i / F;
+    const int c = (int)(i - ur * F);
+    const float* p = g + ur * T * F + c;
+    double s2 = 0.0, s1 = 0.0;
+#pragma unroll 20
+    for (int t = 0; t < T; ++t) {
+        const double v = (double)__ldcs(p + (int64_t)t * F);
+        s2 = fma(v, v, s2);
+        s1 += v;
+    }
+    double* o = part + ur * (2 * F + 1);
+    o[c] = s2;
+    o[F + c] = s1;
+    if (c == 0) o[2 * F] = (double)mu[ur];
+}
+
+// acc[r][j] (+)= part[u][r][j] for u = 0 .. n_units - 1 in that order (first: acc starts at part[0][r][j]); with
+// finish_units > 0 the totals are divided in double and rounded once: attr[r][0][c] = acc / (U T), attr[r][1][c] = acc / U,
+// mu_mean[r] = acc / U.  One thread per (row, accumulator); no atomics.
+__global__ void __launch_bounds__(256) attr_accumulate_kernel(const double* __restrict__ part, int n_units, int64_t rows,
+                                                              int T, int F, int first, int64_t finish_units,
+                                                              double* __restrict__ acc, float* __restrict__ attr,
+                                                              float* __restrict__ mu_mean) {
+    const int W = 2 * F + 1;
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= rows * W) return;
+    const int64_t r = i / W;
+    const int j = (int)(i - r * W);
+    const int64_t ustride = rows * W;
+    double a = first ? part[i] : acc[i] + part[i];
+    for (int u = 1; u < n_units; ++u) a += part[u * ustride + i];
+    acc[i] = a;
+    if (finish_units > 0) {
+        const double U = (double)finish_units;
+        if (j < F) attr[r * 2 * F + j] = (float)(a / U / (double)T);
+        else if (j < 2 * F) attr[r * 2 * F + j] = (float)(a / U);
+        else mu_mean[r] = (float)(a / U);
+    }
+}
+
+// workspace of one bnn_posterior_saliency call (floats, each block a multiple of 4): eps12 | g | mu | part | saliency
+struct AttrWorkspace {
+    size_t eps12, g, mu, part, sal, total;
+    AttrWorkspace(const bnn_model_config* cfg, int32_t n_units, int64_t rows) {
+        const size_t ur = (size_t)n_units * rows, F = cfg->n_features;
+        size_t o = 0;
+        eps12 = o; o += ur * S2;
+        g = o; o += ur * cfg->n_times * F;
+        mu = o; o += (ur + 3) & ~(size_t)3;
+        part = o; o += (ur * (2 * F + 1) * 2 + 3) & ~(size_t)3;
+        sal = o; o += saliency_workspace_floats(cfg, n_units, rows);
+        total = o;
+    }
+};
+
 }  // namespace train
 }  // namespace bnn
 
@@ -501,34 +631,66 @@ int bnn_saliency(const bnn_model_config* cfg, int32_t n_models, const float* d_t
     BNN_REQUIRE(cfg->n_times == 100 && cfg->n_features == 41, BNN_E_CONFIG,
                 "bnn_saliency: compiled for T=100, F=41 (got T=%d, F=%d)", cfg->n_times, cfg->n_features);
     BNN_REQUIRE(aligned16(d_workspace) && (!d_eps12 || aligned16(d_eps12)), BNN_E_ALIGN, "bnn_saliency: alignment");
-    const int F = cfg->n_features, T = cfg->n_times;
-    const FlatLayout fl(F);
-    int64_t n_cta = train::sm_count() / n_models;
-    if (n_cta > (B + 1) / 2) n_cta = (B + 1) / 2;
-    if (n_cta < 1) n_cta = 1;
-    const int DP = fl.d + train::DPAD;
-    float* partial = (float*)d_workspace;
-    float* xprod = partial + (size_t)n_models * n_cta * DP;
-    xprod += (4 - ((uintptr_t)xprod / sizeof(float)) % 4) % 4;
-    train::Params prm;
-    prm.theta = d_theta; prm.X = d_x; prm.Y = nullptr; prm.batch_index = nullptr;
-    prm.eps_in = nullptr; prm.eps12 = d_eps12; prm.eps_sum = nullptr;
-    prm.partial = partial; prm.head_rec = nullptr; prm.xprod = xprod;
-    prm.B = (int)B; prm.T = T; prm.F = F; prm.FP = (F + 3) & ~3; prm.n_cta = (int)n_cta; prm.seed0 = 0;
-    prm.seed = seed; prm.step = 0; prm.zero_mask = cfg->zero_mask;
-    prm.hc = HeadConsts{cfg->lo_mu, cfg->hi_mu, cfg->lo_sd, cfg->hi_sd};
-    prm.beta_out = 0.f;
-    prm.saliency = 1; prm.gx_out = d_grad_x; prm.mu_out = d_mu;
-    static PerDeviceOnce attr_done;
-    if (attr_done.need()) {
-        BNN_CUDA(cudaFuncSetAttribute(train::train_fwd_bwd3_kernel<100, 41>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      227 * 1024));
-    }
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t smem3 = (size_t)train::Smem3(T, F).total * sizeof(float);
-    train::train_fwd_bwd3_kernel<100, 41><<<dim3((unsigned)n_cta, n_models), train::NTHR3, smem3, st>>>(prm);
+    const float* partial = nullptr;
+    int n_cta = 0;
+    rc = train::saliency_launch(cfg, n_models, d_theta, d_x, B, d_eps12, seed, d_grad_x, d_mu, d_workspace, st, &partial,
+                                &n_cta);
+    if (rc != BNN_OK) return rc;
+    train::saliency_finish_kernel<<<n_models, 64, 0, st>>>(partial, n_cta, FlatLayout(cfg->n_features).d, cfg->n_features,
+                                                           d_sumsq);
     BNN_CUDA(cudaGetLastError());
-    train::saliency_finish_kernel<<<n_models, 64, 0, st>>>(partial, (int)n_cta, fl.d, F, d_sumsq);
+    return BNN_OK;
+}
+
+size_t bnn_posterior_saliency_workspace_bytes(const bnn_model_config* cfg, int32_t n_units, int64_t rows) {
+    using namespace bnn;
+    if (validate_config(cfg) != BNN_OK || n_units < 1 || n_units > 65535 || rows < 1 || rows >= (1ll << 30)) return 0;
+    return train::AttrWorkspace(cfg, n_units, rows).total * sizeof(float);
+}
+
+int bnn_posterior_saliency(const bnn_model_config* cfg, int32_t n_units, const float* d_theta, int64_t unit0,
+                           const float* d_x, int64_t rows, int64_t row0, uint64_t seed, double* d_acc, int32_t first,
+                           int64_t finish_units, float* d_attr, float* d_mu_mean, float* d_mu_units, void* d_workspace,
+                           void* stream) {
+    using namespace bnn;
+    int rc = validate_config(cfg);
+    if (rc != BNN_OK) return rc;
+    const char* who = "bnn_posterior_saliency";
+    BNN_REQUIRE(d_theta && d_x && d_acc && d_workspace, BNN_E_ARG, "%s: null pointer", who);
+    BNN_REQUIRE(finish_units == 0 || (d_attr && d_mu_mean), BNN_E_ARG, "%s: finishing needs d_attr and d_mu_mean", who);
+    BNN_REQUIRE(n_units >= 1 && n_units <= 65535 && rows >= 1 && rows < (1ll << 30), BNN_E_ARG,
+                "%s: n_units=%d rows=%lld out of range", who, n_units, (long long)rows);
+    BNN_REQUIRE(unit0 >= 0 && unit0 + n_units <= (1ll << 32) && row0 >= 0 && row0 + rows <= (1ll << 32), BNN_E_ARG,
+                "%s: unit0=%lld row0=%lld: global unit and row indices must fit the 32-bit Philox counters", who,
+                (long long)unit0, (long long)row0);
+    BNN_REQUIRE(finish_units == 0 || (finish_units >= n_units && finish_units < (1ll << 32)), BNN_E_ARG,
+                "%s: finish_units=%lld (0, or the number of units accumulated, >= n_units)", who, (long long)finish_units);
+    BNN_REQUIRE(cfg->n_times == 100 && cfg->n_features == 41, BNN_E_CONFIG,
+                "%s: compiled for T=100, F=41 (got T=%d, F=%d)", who, cfg->n_times, cfg->n_features);
+    BNN_REQUIRE(aligned16(d_workspace) && ((uintptr_t)d_acc & 7u) == 0 && ((uintptr_t)d_x & 3u) == 0 &&
+                    ((uintptr_t)d_theta & 3u) == 0 && ((uintptr_t)d_attr & 3u) == 0 && ((uintptr_t)d_mu_mean & 3u) == 0 &&
+                    ((uintptr_t)d_mu_units & 3u) == 0,
+                BNN_E_ALIGN, "%s: d_workspace must be 16-byte, d_acc 8-byte and the float arrays 4-byte aligned", who);
+    if ((rc = check_device()) != BNN_OK) return rc;
+    const int F = cfg->n_features, T = cfg->n_times;
+    const train::AttrWorkspace wl(cfg, n_units, rows);
+    float* ws = (float*)d_workspace;
+    float* eps12 = ws + wl.eps12;
+    float* g = ws + wl.g;
+    float* mu = d_mu_units ? d_mu_units : ws + wl.mu;
+    double* part = reinterpret_cast<double*>(ws + wl.part);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t ur = (int64_t)n_units * rows;
+    const int64_t n_eps = ur * train::ATTR_ROUNDS, n_sums = ur * F, n_acc = rows * (2 * F + 1);
+    train::attr_eps_kernel<<<(unsigned)((n_eps + 255) / 256), 256, 0, st>>>(n_eps, rows, seed, unit0, row0, eps12);
+    BNN_CUDA(cudaGetLastError());
+    rc = train::saliency_launch(cfg, n_units, d_theta, d_x, rows, eps12, seed, g, mu, ws + wl.sal, st, nullptr, nullptr);
+    if (rc != BNN_OK) return rc;
+    train::attr_unit_sums_kernel<<<(unsigned)((n_sums + 255) / 256), 256, 0, st>>>(g, mu, n_sums, T, F, part);
+    BNN_CUDA(cudaGetLastError());
+    train::attr_accumulate_kernel<<<(unsigned)((n_acc + 255) / 256), 256, 0, st>>>(part, n_units, rows, T, F, first ? 1 : 0,
+                                                                                   finish_units, d_acc, d_attr, d_mu_mean);
     BNN_CUDA(cudaGetLastError());
     return BNN_OK;
 }

@@ -243,10 +243,14 @@ class MultiSWAG:
 
     # ------------------------------------------------------------------ batched path
     def sample_thetas(self, samples_per_model: int, seed: int, scale: float = 0.5, unit_model=None,
-                      unit_offset: int = 0, n_units: Optional[int] = None, z1=None, z2=None, want_flat=True):
+                      unit_offset: int = 0, n_units: Optional[int] = None, z1=None, z2=None, want_flat=True,
+                      want_packed=True):
         """(theta[U,d], theta_packed[U,P]).  Unit u = model*S + sample unless unit_model is given; units
         [unit_offset, unit_offset + n_units) of that numbering when a chunk is asked for (the Philox draws are keyed on
-        the global unit index).  ``want_flat=False``: only the packed layout is written (theta is None)."""
+        the global unit index).  ``want_flat=False``: only the packed layout is written (theta is None);
+        ``want_packed=False``: only the flat one (theta_packed is None)."""
+        if not want_flat and not want_packed:
+            raise ValueError("sample_thetas: ask for the flat or the packed layout (or both)")
         lib = _lib.load()
         cfg = self.config()
         M, d = self.w_avg.shape
@@ -254,7 +258,7 @@ class MultiSWAG:
         P = lib.bnn_packed_param_count(cfg)
         with torch.cuda.device(self.device), _lib.nvtx("bnn:K1 swag_sample"):
             theta = torch.empty((U, d), device=self.device) if want_flat else None
-            thp = torch.empty((U, P), device=self.device)
+            thp = torch.empty((U, P), device=self.device) if want_packed else None
             um = None
             if unit_model is not None:
                 um = torch.as_tensor(unit_model, dtype=torch.int32, device=self.device).contiguous()
@@ -263,7 +267,7 @@ class MultiSWAG:
                 lib.bnn_swag_sample(cfg, _lib.ptr(self.w_avg), _lib.ptr(self.w2_avg), _lib.ptr(self.pre_D), M, self.K,
                                     dp(um, "unit_model", torch.int32), U, unit_offset, max(int(samples_per_model), 1),
                                     float(scale), int(seed), dp(z1, "z1"), dp(z2, "z2"),
-                                    _lib.ptr(theta) if want_flat else None, _lib.ptr(thp),
+                                    _lib.ptr(theta), _lib.ptr(thp),
                                     _lib.current_stream_ptr()),
                 "bnn_swag_sample",
             )
@@ -551,9 +555,9 @@ class MultiSWAG:
 
     @staticmethod
     def _check_reduce(x: torch.Tensor, samples_per_model: int, n_trios, y=None, thresholds=None,
-                      uncertainty=False, trios=False):
-        """Argument checks of ``_reduce`` / ``_reduce_sharded``, before any device work.  Returns the thresholds as
-        ``posterior.survival_thresholds`` (or None)."""
+                      uncertainty=False, trios=False, attribution=False):
+        """Argument checks of ``_reduce`` / ``_reduce_sharded`` (and, with ``attribution``, of the attribution walk),
+        before any device work.  Returns the thresholds as ``posterior.survival_thresholds`` (or None)."""
         from . import posterior
 
         ragged = posterior.is_ragged(n_trios)   # a catalogue: its counts are checked here, its rows by the caller
@@ -565,7 +569,7 @@ class MultiSWAG:
             posterior.check_trio_counts(n_trios, None)
         if y is not None:
             MultiSWAG._check_labelled(x, y, samples_per_model)
-        if thresholds is None and not uncertainty and not trios and not ragged:
+        if thresholds is None and not uncertainty and not trios and not attribution and not ragged:
             return None
         if x.dim() != 3:
             raise ValueError(f"x must be [N*n_trios, T, F], got {tuple(x.shape)}")
@@ -573,6 +577,8 @@ class MultiSWAG:
             raise ValueError(f"{x.shape[0]} rows are not a multiple of {n_trios} trios")
         if int(samples_per_model) < 1:
             raise ValueError(f"samples_per_model must be >= 1, got {samples_per_model}")
+        if attribution and tuple(x.shape[1:]) != (100, 41):
+            raise ValueError(f"the attribution kernel takes [rows, 100, 41] inputs, got {tuple(x.shape)}")
         thr = posterior.survival_thresholds(thresholds) if thresholds is not None else None
         _lib.require_cuda(x, "x")
         return thr
@@ -832,6 +838,117 @@ class MultiSWAG:
         summary, first, trio_summary = self._reduce_sharded(x_local, n_total, samples_per_model, n_trios, seed, scale,
                                                             group, trios=True)
         return summary, first, trio_summary
+
+    def posterior_attribution(self, x: torch.Tensor, samples_per_model: int, n_trios=1, seed: int = 0, scale: float = 0.5,
+                              system_offset: int = 0, max_block_bytes: int = 1 << 30, unit_chunk: Optional[int] = None):
+        """Which inputs drive each row's prediction: x [N*n_trios, 100, 41] (as ``posterior_summary``) -> (attribution
+        [N, n_trios, 2, 41], mu [N, n_trios]).  For every row r and each of the U = n_models * samples_per_model units u,
+        g_u = d mu_u / d x_r [T, F] is the gradient of that unit's predicted mean, with the weights and summary draws
+        ``predict`` uses (no input or summary noise).  attribution[.., 0, c] (importance, ``posterior.ATTRIBUTION_NAMES``)
+        = (1/U) sum_u (1/T) sum_t g_u[t, c]^2: figures/feature_importance.py's measure for one row, averaged over the
+        posterior instead of taken at w_avg.  attribution[.., 1, c] (shift) = (1/U) sum_u sum_t g_u[t, c]: the signed
+        first-order change of mu when column c rises by one standard-scaler unit at every time step.  mu = (1/U) sum_u
+        mu_u, the mean the attribution belongs to (``posterior_uncertainty``'s mean_mu up to the kernels' rounding).
+        Summed in double unit after unit and rounded once, so the result depends neither on the chunking nor on a split
+        into shards with ``system_offset``.  Per-row outputs need no per-system pass: with per-system trio counts
+        ``n_trios`` (as in ``posterior_summary``, ``system_offset`` 0) they are [rows, 2, 41] and [rows] in x's row
+        order.  Units are walked ``unit_chunk`` at a time (default: one per SM, one wave of the saliency kernel), their
+        flat weights sampled once per chunk, and inside a unit chunk the rows in chunks whose gradients fit
+        ``max_block_bytes`` (16.4 kB per (unit, row))."""
+        from . import posterior
+
+        ragged = posterior.is_ragged(n_trios)
+        if ragged and system_offset:
+            raise ValueError("with per-system trio counts system_offset must be 0: split a catalogue with "
+                             "posterior_attribution_sharded")
+        self._check_attribution_walk(max_block_bytes, unit_chunk)
+        self._check_catalogue(x, n_trios)
+        self._check_reduce(x, samples_per_model, n_trios, attribution=True)
+        attr, mu = self._attribution(x, samples_per_model, 0 if ragged else int(system_offset) * int(n_trios), seed, scale,
+                                     max_block_bytes, unit_chunk)
+        if ragged:
+            return attr, mu
+        N = x.shape[0] // int(n_trios)
+        return attr.view(N, int(n_trios), 2, attr.shape[2]), mu.view(N, int(n_trios))
+
+    @staticmethod
+    def _check_attribution_walk(max_block_bytes, unit_chunk):
+        if int(max_block_bytes) < 1:
+            raise ValueError(f"max_block_bytes must be positive, got {max_block_bytes}")
+        if unit_chunk is not None and int(unit_chunk) < 1:
+            raise ValueError(f"unit_chunk must be >= 1, got {unit_chunk}")
+
+    def _attribution(self, x, samples_per_model, row0, seed, scale, max_block_bytes, unit_chunk):
+        """The walk of ``posterior_attribution`` over rows x whose first row is global row ``row0`` -> ([rows, 2, F],
+        [rows]).  Unit chunks in increasing order, each over all row chunks, into one float64 accumulator per row."""
+        from . import posterior
+
+        rows, T, F = x.shape
+        U = self.n_models * int(samples_per_model)
+        attr = torch.empty((rows, 2, F), device=self.device)
+        mu = torch.empty((rows,), device=self.device)
+        if rows == 0:
+            return attr, mu
+        with torch.cuda.device(self.device):
+            if unit_chunk is None:
+                unit_chunk = torch.cuda.get_device_properties(self.device).multi_processor_count
+            uc = min(int(unit_chunk), U, 65535)
+            per = min(rows, max(1, int(max_block_bytes) // (uc * T * F * 4)), (1 << 30) - 1)
+            x = x.contiguous().float()
+            cfg = self.config(T)
+            acc = torch.empty((rows, 2 * F + 1), device=self.device, dtype=torch.float64)
+            ws = posterior.attribution_workspace(cfg, uc, per, self.device)   # serves the smaller remainder chunks too
+            for u0 in range(0, U, uc):
+                u1 = min(u0 + uc, U)
+                theta, _ = self.sample_thetas(samples_per_model, seed, scale, unit_offset=u0, n_units=u1 - u0,
+                                              want_packed=False)
+                for a in range(0, rows, per):
+                    b = min(a + per, rows)
+                    posterior.accumulate_attribution(cfg, theta, u0, x[a:b], row0 + a, seed, acc[a:b], u0 == 0,
+                                                     U if u1 == U else 0, attr[a:b], mu[a:b], workspace=ws)
+                del theta
+        return attr, mu
+
+    def posterior_attribution_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int, n_trios=1,
+                                      seed: int = 0, scale: float = 0.5, group=None, max_block_bytes: int = 1 << 30,
+                                      unit_chunk: Optional[int] = None):
+        """``posterior_attribution`` with the rows split over ranks; ONE all_gather moves [rows, 2F + 1] (attribution |
+        mu).  An int ``n_trios``: systems are block-partitioned like ``posterior_summary_sharded`` (``shard_range``, no
+        granule: this path has no predictive kernel), and x_local holds the rows of the rank's systems.  Per-system trio
+        counts of the whole catalogue [n_total]: the attribution is per row, so the catalogue's rows themselves are
+        split with ``shard_range``, and x_local holds rank's rows.  Returns the same outputs as ``posterior_attribution``
+        on the whole x, on every rank."""
+        import torch.distributed as dist
+
+        from . import posterior
+
+        self._check_attribution_walk(max_block_bytes, unit_chunk)
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+        rank = dist.get_rank(group) if dist.is_initialized() else 0
+        ragged = posterior.is_ragged(n_trios)
+        if ragged:
+            off = posterior.row_offsets(n_trios, None)
+            if off.size - 1 != n_total:
+                raise ValueError(f"{off.size - 1} trio counts for a catalogue of n_total = {n_total} systems")
+            R_total, k = int(off[-1]), 1
+        else:
+            k = int(n_trios)
+            if k < 1 or x_local.shape[0] % k:
+                raise ValueError(f"{x_local.shape[0]} rows are not a multiple of {n_trios} trios")
+            R_total = int(n_total) * k
+        bounds = [tuple(k * v for v in shard_range(R_total // k, r, world)) for r in range(world)]
+        lo, hi = bounds[rank]
+        if x_local.shape[0] != hi - lo:
+            raise ValueError(f"rank {rank} owns rows [{lo}, {hi}) of {R_total} but was given {x_local.shape[0]} rows")
+        self._check_reduce(x_local, samples_per_model, n_trios, attribution=True)
+        attr, mu = self._attribution(x_local, samples_per_model, lo, seed, scale, max_block_bytes, unit_chunk)
+        F = x_local.shape[2]
+        if world > 1:
+            full = gather_system_shards(torch.cat([attr.view(-1, 2 * F), mu[:, None]], 1), R_total, group, bounds=bounds)
+            attr, mu = full[:, :2 * F].contiguous().view(R_total, 2, F), full[:, 2 * F].contiguous()
+        if ragged:
+            return attr, mu
+        return attr.view(int(n_total), k, 2, F), mu.view(int(n_total), k)
 
     def posterior_summary_sharded(self, x_local: torch.Tensor, n_total: int, samples_per_model: int, n_trios: int = 1,
                                   seed: int = 0, scale: float = 0.5, group=None):

@@ -6,6 +6,7 @@ resampling of draws >= 9 from the analytic prior, min over trios, per-system med
 device instead of the ``[N, U, 2]`` prediction block.  ``survival`` counts the same sampled times against thresholds:
 P(T_inst > t) per system.  ``uncertainty`` splits each row's predictive variance into aleatoric, between-model and
 within-model parts.  ``first_trio`` counts, per trio, how often it is the one that sets its system's min.
+``accumulate_attribution`` reduces each row's input gradients dmu / dx over the posterior's units (importance, shift).
 
 A catalogue of systems with different numbers of planets (P planets: P - 2 adjacent trios) is passed to ``summarize_instability``,
 ``survival`` and ``first_trio`` as per-system trio counts instead of one ``n_trios``: system n owns the next counts[n] rows, system-major
@@ -318,3 +319,35 @@ def uncertainty(pred: torch.Tensor, units_per_model: int):
         _lib.check(lib.bnn_decompose_uncertainty(_lib.ptr(pred), rows, U, S, _lib.ptr(out), _lib.current_stream_ptr()),
                    "bnn_decompose_uncertainty")
     return out
+
+
+ATTRIBUTION_NAMES = ("importance", "shift")
+
+
+def attribution_workspace(cfg, n_units: int, rows: int, device) -> torch.Tensor:
+    """Scratch for ``accumulate_attribution`` calls of up to n_units units x rows rows (16.4 kB of gradients per pair)."""
+    nbytes = _lib.load().bnn_posterior_saliency_workspace_bytes(cfg, int(n_units), int(rows))
+    if nbytes == 0:
+        raise ValueError(f"no attribution workspace for {n_units} units x {rows} rows")
+    return torch.empty(((nbytes + 3) // 4,), device=device, dtype=torch.float32)
+
+
+def accumulate_attribution(cfg, theta: torch.Tensor, unit0: int, x: torch.Tensor, row0: int, seed: int,
+                           acc: torch.Tensor, first: bool, finish_units: int = 0, attr=None, mu_mean=None, mu_units=None,
+                           workspace=None):
+    """One (unit chunk, row chunk) step of the posterior attribution (``bnn_posterior_saliency``): the flat weights theta
+    [Uc, d] of global units unit0 .. and the rows x [rows, T, F] of global rows row0 .. add their d mu / d x sums to the
+    float64 accumulators acc [rows, 2F + 1] (``first``: they start here).  ``finish_units`` = U on the call with the
+    walk's last units writes attr [rows, 2, F] (``ATTRIBUTION_NAMES``) and mu_mean [rows]; mu_units [Uc, rows] receives
+    each unit's mu."""
+    lib = _lib.load()
+    dev = x.device
+    if workspace is None:
+        workspace = attribution_workspace(cfg, theta.shape[0], x.shape[0], dev)
+    dp = lambda t, name, dt=None: _lib.dev_ptr(t, dev, name, dt)
+    with torch.cuda.device(dev), _lib.nvtx("bnn:K4 posterior_saliency"):
+        _lib.check(lib.bnn_posterior_saliency(cfg, theta.shape[0], dp(theta, "theta"), int(unit0), dp(x, "x"), x.shape[0],
+                                              int(row0), int(seed), dp(acc, "acc", torch.float64), int(bool(first)),
+                                              int(finish_units), dp(attr, "attr"), dp(mu_mean, "mu_mean"),
+                                              dp(mu_units, "mu_units"), dp(workspace, "workspace"),
+                                              _lib.current_stream_ptr()), "bnn_posterior_saliency")

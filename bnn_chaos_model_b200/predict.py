@@ -9,6 +9,7 @@ counts): per system the posterior summary [N, 8] (``posterior.STAT_NAMES``) of t
     python -m bnn_chaos_model_b200.predict --models DIR/*_output.pkl --data catalogue.npz --samples 100 --out OUT
     python -m bnn_chaos_model_b200.predict --models DIR/*_output.pkl --synthetic 2000 --survival 6 9 --uncertainty --out OUT
     python -m bnn_chaos_model_b200.predict --models DIR/*_output.pkl --data catalogue.npz --trios --out OUT
+    python -m bnn_chaos_model_b200.predict --models DIR/*_output.pkl --data catalogue.npz --trios --attribution --out OUT
     python -m torch.distributed.run --nproc-per-node 8 -m bnn_chaos_model_b200.predict --models ... --out OUT
 
 ``catalogue.npz`` holds ``n_trios`` [N] (trio rows per system, >= 1; system n owns the next n_trios[n] rows) and exactly
@@ -24,12 +25,16 @@ Writes to ``--out``:
     trio row (aleatoric, between-model and within-model parts of the predictive variance) and ``uncertainty_names``;
     with ``--trios`` ``trio_first`` [R], per trio row the fraction of the weight samples at which that trio sets its
     system's minimum (which trio goes unstable first), ``trio_summary`` [R, 8], the posterior summary of each trio on
-    its own, and ``trio_stat_names``;
+    its own, and ``trio_stat_names``; with ``--attribution`` ``attribution`` [R, 2, 41], per trio row and input column
+    the posterior mean of (1/T) sum_t (d mu / d x)^2 (importance) and of sum_t d mu / d x (shift), ``attribution_mu``
+    [R], the mean mu they belong to, and ``attribution_names`` (``MultiSWAG.posterior_attribution``);
   * ``summary.json``: the settings, the number of systems per trio count, with ``--survival`` ``survival_mean`` and,
     with ``--trios``, ``weakest_trio_position``: for each trio count k >= 2, how many of the systems of k trios have
-    their largest ``trio_first`` at position 0 .. k - 1 (ties go to the first position).
-Under torchrun each rank reduces a contiguous block of systems balanced by rows (``catalogue_shard_range``), the
-results are gathered and rank 0 writes the files; they are the same files as from one GPU.
+    their largest ``trio_first`` at position 0 .. k - 1 (ties go to the first position); with ``--attribution``
+    ``attribution_mean_importance`` [41], the importance averaged over the trio rows.
+Under torchrun each rank reduces a contiguous block of systems balanced by rows (``catalogue_shard_range``; the
+attribution, which is per row, splits the rows themselves), the results are gathered and rank 0 writes the files; they
+are the same files as from one GPU.
 """
 from __future__ import annotations
 
@@ -63,6 +68,9 @@ def build_parser():
     ap.add_argument("--trios", action="store_true",
                     help="also report, per trio row, how often that trio sets its system's instability time and its own "
                          "posterior summary")
+    ap.add_argument("--attribution", action="store_true",
+                    help="also attribute each trio row's predicted mean to the input columns (posterior mean of the "
+                         "squared and of the summed gradient d mu / d x)")
     return ap
 
 
@@ -130,8 +138,8 @@ def main(argv=None):
     """Returns the summary dict on rank 0 (None on the other ranks)."""
     import torch.distributed as dist
 
-    from .multiswag import catalogue_shard_range, load_ensemble
-    from .posterior import STAT_NAMES, UNCERTAINTY_NAMES, check_trio_counts, survival_thresholds
+    from .multiswag import catalogue_shard_range, load_ensemble, shard_range
+    from .posterior import ATTRIBUTION_NAMES, STAT_NAMES, UNCERTAINTY_NAMES, check_trio_counts, survival_thresholds
 
     args = build_parser().parse_args(argv)
     if args.survival is not None:
@@ -141,6 +149,8 @@ def main(argv=None):
     counts, inputs = load_catalogue(args)
     if args.trios:
         check_trio_counts(counts, None)   # at most MAX_TRIOS_PER_SYSTEM trios per system
+    if args.attribution and next(iter(inputs.values())).shape[1] != 100:
+        raise ValueError("--attribution needs T = 100 time steps per row")
     N, R = counts.size, int(counts.sum())
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -159,6 +169,10 @@ def main(argv=None):
     else:
         outs = ens._reduce(model_inputs(inputs, 0, R, dev), args.samples, counts, args.seed, args.scale,
                            thresholds=args.survival, uncertainty=args.uncertainty, trios=args.trios)
+    if args.attribution:   # per row: each rank takes a contiguous block of rows
+        lo, hi = shard_range(R, dist.get_rank(), world) if world > 1 else (0, R)
+        attr = ens.posterior_attribution_sharded(model_inputs(inputs, lo, hi, dev), N, args.samples, counts, args.seed,
+                                                 args.scale)
     info = None
     if world == 1 or dist.get_rank() == 0:
         summary = outs[0].cpu().numpy()
@@ -180,6 +194,10 @@ def main(argv=None):
             first = outs[-2].cpu().numpy()
             arrays.update(trio_first=first, trio_summary=outs[-1].cpu().numpy(), trio_stat_names=np.array(STAT_NAMES))
             info["weakest_trio_position"] = weakest_trio_position(first, counts)
+        if args.attribution:
+            a = attr[0].cpu().numpy()
+            arrays.update(attribution=a, attribution_mu=attr[1].cpu().numpy(), attribution_names=np.array(ATTRIBUTION_NAMES))
+            info["attribution_mean_importance"] = [float(v) for v in a[:, 0].astype(np.float64).mean(0)]
         os.makedirs(args.out, exist_ok=True)
         with open(os.path.join(args.out, "summary.json"), "w") as f:
             json.dump(info, f, indent=1)

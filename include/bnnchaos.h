@@ -219,6 +219,31 @@ int bnn_saliency(const bnn_model_config* cfg, int32_t n_models, const float* d_t
                  const float* d_eps12, uint64_t seed, float* d_grad_x, float* d_sumsq, float* d_mu, void* d_workspace,
                  void* stream);
 
+/* Posterior attribution: which inputs drive each row's predicted mean under the MultiSWAG posterior.  For the n_units
+ * sampled weight vectors d_theta [n_units, d] (flatten() order; global units unit0 ..) and the model-input rows d_x
+ * [rows, T, F] (global rows row0 ..): mu_u is unit u's predicted mean with the predictive kernel's own summary draws
+ * (eps1 | eps2 = Philox on (seed; unit0 + u, row0 + r), exactly bnn_predict's with d_eps NULL) and no input or summary
+ * noise, and g_u = d mu_u / d x_r [T, F] (the saliency kernel of bnn_saliency; the zeroed columns carry gradient too).
+ * Per row, into the caller's double accumulators d_acc [rows, 2F + 1]:
+ *   acc[r][c] += sum_t g_u[t][c]^2,  acc[r][F + c] += sum_t g_u[t][c],  acc[r][2F] += mu_u,
+ * unit after unit in increasing order (first != 0: the accumulators start at this call's first unit, unread), each
+ * (unit, row) summed over t in a fixed order; no atomics.  So a row's result depends only on its own inputs and the
+ * set of units: call the unit chunks in increasing order, each over any split of the rows, and the bits do not
+ * change.  finish_units > 0 (the total U of the walk, on the call with its last units): d_attr [rows, 2, F] =
+ * (importance = acc / (U T), shift = acc / U) and d_mu_mean [rows] = acc / U, divided in double and rounded to fp32
+ * once.  d_mu_units [n_units, rows] (may be NULL): each unit's mu.  The g block is transient workspace scratch (16.4 kB
+ * per (unit, row)): size the chunks with bnn_posterior_saliency_workspace_bytes(cfg, n_units, rows) (0 for bad
+ * arguments), which is non-decreasing in both counts: a workspace sized for (n_units, rows) serves every call of at most
+ * n_units units and rows rows (a walk's smaller remainder chunks included); it begins with this call's summary draws [n_units, rows, 2L], which bnn_predict reproduces bit for bit
+ * when given them as d_eps.  BNN_E_ARG: null pointer, n_units outside [1, 65535], rows outside [1, 2^30), unit or row indices past
+ * 2^32, finish_units neither 0 nor in [n_units, 2^32); BNN_E_CONFIG: T != 100 or F != 41; BNN_E_ALIGN: d_workspace not
+ * 16-byte, d_acc not 8-byte or a float array not 4-byte aligned; every check runs before the device is touched. */
+size_t bnn_posterior_saliency_workspace_bytes(const bnn_model_config* cfg, int32_t n_units, int64_t rows);
+int bnn_posterior_saliency(const bnn_model_config* cfg, int32_t n_units, const float* d_theta, int64_t unit0,
+                           const float* d_x, int64_t rows, int64_t row0, uint64_t seed, double* d_acc, int32_t first,
+                           int64_t finish_units, float* d_attr, float* d_mu_mean, float* d_mu_units, void* d_workspace,
+                           void* stream);
+
 /* The Philox draws bnn_train_step makes for (seed, step) when its eps pointers are NULL. */
 int bnn_train_noise(const bnn_model_config* cfg, int32_t n_seeds, int64_t B, uint64_t seed, uint64_t step,
                     float* d_eps_in, float* d_eps12, float* d_eps_sum, void* stream);
