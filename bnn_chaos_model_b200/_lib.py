@@ -109,6 +109,18 @@ SIGNATURES = {
         [_CFG, _HP, _ADAM, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, C.c_int64, c_f32p, c_f32p, c_f32p,
          C.c_uint64, C.c_uint64, c_f32p, c_f32p, C.c_void_p, C.c_void_p],
     ),
+    # per-seed hyperparameters: hp / adam are host arrays [n_seeds] (TrainHParams * n, AdamHParams * n), then plan_seeds
+    "bnn_train_workspace_bytes_seeds": (C.c_size_t, [_CFG, C.c_int64, C.c_int32, C.c_int32]),
+    "bnn_train_step_seeds": (
+        C.c_int,
+        [_CFG, _HP, C.c_int32, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, C.c_int64, c_f32p, c_f32p, c_f32p, C.c_uint64,
+         C.c_uint64, c_f32p, c_f32p, C.c_void_p, C.c_void_p],
+    ),
+    "bnn_train_step_adam_seeds": (
+        C.c_int,
+        [_CFG, _HP, _ADAM, C.c_int32, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, C.c_int64, c_f32p, c_f32p, c_f32p,
+         C.c_uint64, C.c_uint64, c_f32p, c_f32p, C.c_void_p, C.c_void_p],
+    ),
     "bnn_train_noise": (
         C.c_int,
         [_CFG, C.c_int32, C.c_int64, C.c_uint64, C.c_uint64, c_f32p, c_f32p, c_f32p, C.c_void_p],

@@ -36,6 +36,11 @@ namespace train {
 
 constexpr int DPAD = 8;            // metric slots appended to each gradient partial
 constexpr int SLOT_NLL = 0, SLOT_SKL = 1;
+// Per-seed hyperparameters travel in the kernels' parameters (no device copy, no allocation): a launch of the training
+// kernel carries the beta_out of at most TRAIN_SEED_CHUNK seeds, a launch of the reduce / update / metrics kernels the
+// scalars of at most SEED_CHUNK seeds; larger seed counts are split into launches of that many seeds.
+constexpr int TRAIN_SEED_CHUNK = 512;
+constexpr int SEED_CHUNK = 64;
 
 struct Params {
     const float* theta;        // [n_seeds, d]
@@ -56,7 +61,7 @@ struct Params {
     uint64_t seed, step;
     uint64_t zero_mask;
     HeadConsts hc;
-    float beta_out;
+    float beta_out[TRAIN_SEED_CHUNK];   // of seed seed0 + blockIdx.y (saliency: [0] = 0 for every model)
 };
 
 // Philox key of one seed-model's noise streams; counters: (block, batch position, step, stream)
@@ -71,21 +76,29 @@ __host__ __device__ inline uint64_t seed_key(uint64_t seed, int seed_index) {
 namespace bnn {
 namespace train {
 
-// grad[s][i] = sum_c partial[s][c][i] (fixed order) + analytic KL terms; per-block sum of squares.
+// The scalars of seed s0 + j, in entry j of a launch's SeedChunk (kernel parameters of the reduce / update / metrics
+// kernels).  kl_in_scale = beta_in * B and kl_sum_scale = beta_out * B are rounded on the host.
+struct SeedHp {
+    float lr, momentum, weight_decay, clip_norm, beta_in, beta_out;
+    float kl_in_scale, kl_sum_scale;
+};
+struct SeedChunk { SeedHp s[SEED_CHUNK]; };
+
+// grad[s][i] = sum_c partial[s][c][i] (fixed order) + analytic KL terms; per-block sum of squares.  s = s0 + blockIdx.y.
 __global__ void __launch_bounds__(256) train_reduce_kernel(const float* __restrict__ partial, const float* __restrict__ theta,
-                                                           int n_cta, int d, int F, float kl_in_scale, float kl_sum_scale,
+                                                           int n_cta, int d, int F, int s0, const SeedChunk hp,
                                                            float* __restrict__ grad, float* __restrict__ sq) {
     __shared__ float sh[256];
-    const int s = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+    const int s = s0 + (int)blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
     const int DP = d + DPAD;
     float g = 0.f;
     if (i < DP) {
         const float* p = partial + (int64_t)s * n_cta * DP + i;
         for (int c = 0; c < n_cta; ++c) g += p[(int64_t)c * DP];
         if (i < F) {  // input_kl * beta_in * B (:585-590, :726): d/dlv = (e^lv - 1)/2
-            g += kl_in_scale * 0.5f * (expf(theta[(int64_t)s * d + i]) - 1.0f);
+            g += hp.s[blockIdx.y].kl_in_scale * 0.5f * (expf(theta[(int64_t)s * d + i]) - 1.0f);
         } else if (i < F + S2) {  // summary_kl * beta_out, summed over the batch (:515-520, :727)
-            g += kl_sum_scale * 0.5f * (expf(theta[(int64_t)s * d + i]) - 1.0f);
+            g += hp.s[blockIdx.y].kl_sum_scale * 0.5f * (expf(theta[(int64_t)s * d + i]) - 1.0f);
         }
         grad[(int64_t)s * DP + i] = g;
     }
@@ -102,9 +115,9 @@ __global__ void __launch_bounds__(256) train_reduce_kernel(const float* __restri
 // when < 1), grad_out and the metric slots known from the gradient.  Returns the factor the gradient is scaled by
 // (min(1, coef)) and this thread's gradient element in gi (0 past d).
 __device__ __forceinline__ float clip_prologue(const float* __restrict__ grad, const float* __restrict__ sq, int n_blocks,
-                                               int d, int B, const bnn_train_hparams& hp, float* __restrict__ grad_out,
+                                               int d, int B, int s, const SeedHp& hp, float* __restrict__ grad_out,
                                                float* __restrict__ metrics, float& gi) {
-    const int s = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+    const int i = blockIdx.x * 256 + threadIdx.x;
     float ss = 0.f;
     for (int b = 0; b < n_blocks; ++b) ss += sq[s * n_blocks + b];
     const float norm = sqrtf(ss);
@@ -127,20 +140,22 @@ __device__ __forceinline__ float clip_prologue(const float* __restrict__ grad, c
     return clip;
 }
 
-// clip_grad_norm_ + torch.optim.SGD with momentum / weight decay.
+// clip_grad_norm_ + torch.optim.SGD with momentum / weight decay.  s = s0 + blockIdx.y.
 __global__ void __launch_bounds__(256) train_update_kernel(const float* __restrict__ grad, const float* __restrict__ sq,
-                                                           int n_blocks, int d, int B, bnn_train_hparams hp,
-                                                           float* __restrict__ theta, float* __restrict__ mom,
-                                                           float* __restrict__ grad_out, float* __restrict__ metrics) {
-    const int s = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+                                                           int n_blocks, int d, int B, int s0, const SeedChunk hps,
+                                                           int first_step, int apply_update, float* __restrict__ theta,
+                                                           float* __restrict__ mom, float* __restrict__ grad_out,
+                                                           float* __restrict__ metrics) {
+    const int s = s0 + (int)blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+    const SeedHp& hp = hps.s[blockIdx.y];
     float gi;
-    const float clip = clip_prologue(grad, sq, n_blocks, d, B, hp, grad_out, metrics, gi);
-    if (i < d && hp.apply_update) {
+    const float clip = clip_prologue(grad, sq, n_blocks, d, B, s, hp, grad_out, metrics, gi);
+    if (i < d && apply_update) {
         const int64_t o = (int64_t)s * d + i;
         const float th = theta[o];
         float dp = gi * clip;   // clip == 1 when not clipping: exact
         if (hp.weight_decay != 0.f) dp = fmaf(hp.weight_decay, th, dp);
-        const float buf = hp.first_step ? dp : fmaf(hp.momentum, mom[o], dp);
+        const float buf = first_step ? dp : fmaf(hp.momentum, mom[o], dp);
         mom[o] = buf;
         theta[o] = th - hp.lr * buf;
     }
@@ -155,18 +170,24 @@ struct AdamStep {
     float eps;
     int first;         // t == 1: both buffers are zero and are not read (a fresh optimizer; no memset needed)
 };
+struct AdamChunk { AdamStep a[SEED_CHUNK]; };
+// the Adam update kernel's parameters: both chunks, 7 pointers and 5 ints, within the 4 KB every launch may carry
+static_assert(sizeof(SeedChunk) + sizeof(AdamChunk) + 7 * 8 + 5 * 4 <= 4096, "SEED_CHUNK too large for the kernel parameters");
 
 // clip_grad_norm_ + torch.optim.Adam (amsgrad=False, maximize=False; weight decay is L2 added to the gradient, not AdamW):
 //   g += wd theta;  m = lerp(m, g, 1 - beta1);  v = beta2 v + (1 - beta2) g^2;  theta -= step_size m / (sqrt(v) / bc2_sqrt + eps)
 __global__ void __launch_bounds__(256) train_adam_update_kernel(const float* __restrict__ grad, const float* __restrict__ sq,
-                                                                int n_blocks, int d, int B, bnn_train_hparams hp, AdamStep a,
+                                                                int n_blocks, int d, int B, int s0, const SeedChunk hps,
+                                                                const AdamChunk as, int apply_update,
                                                                 float* __restrict__ theta, float* __restrict__ exp_avg,
                                                                 float* __restrict__ exp_avg_sq, float* __restrict__ grad_out,
                                                                 float* __restrict__ metrics) {
-    const int s = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+    const int s = s0 + (int)blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+    const SeedHp& hp = hps.s[blockIdx.y];
+    const AdamStep& a = as.a[blockIdx.y];
     float gi;
-    const float clip = clip_prologue(grad, sq, n_blocks, d, B, hp, grad_out, metrics, gi);
-    if (i < d && hp.apply_update) {
+    const float clip = clip_prologue(grad, sq, n_blocks, d, B, s, hp, grad_out, metrics, gi);
+    if (i < d && apply_update) {
         const int64_t o = (int64_t)s * d + i;
         const float th = theta[o];
         float g = gi * clip;
@@ -181,11 +202,13 @@ __global__ void __launch_bounds__(256) train_adam_update_kernel(const float* __r
     }
 }
 
-// input_kl * beta_in * B / B and the total, from the weights the step was evaluated at (runs BEFORE the update kernel)
+// input_kl * beta_in * B / B and the total, from the weights the step was evaluated at (runs BEFORE the update kernel).
+// s = s0 + blockIdx.x.
 __global__ void train_metrics_kernel(const float* __restrict__ theta, const float* __restrict__ grad, int d, int F, int B,
-                                     bnn_train_hparams hp, float* __restrict__ metrics) {
-    const int s = blockIdx.x;
+                                     int s0, const SeedChunk hps, float* __restrict__ metrics) {
+    const int s = s0 + (int)blockIdx.x;
     if (threadIdx.x != 0) return;
+    const SeedHp& hp = hps.s[blockIdx.x];
     float kl = 0.f;
     for (int c = 0; c < F; ++c) {
         const float lv = theta[(int64_t)s * d + c];
@@ -333,33 +356,91 @@ static SeedPlan pick_plan(const bnn_model_config* cfg, int64_t B, int n_seeds) {
     }
     return best;
 }
-static int pick_n_cta(const bnn_model_config* cfg, int64_t B, int n_seeds) { return pick_plan(cfg, B, n_seeds).n_cta; }
 
-// Everything of a training step before the optimizer's update, shared by bnn_train_step (SGD) and bnn_train_step_adam:
-// the argument checks (`who` names the entry in messages; `state_ok`: the optimizer's state buffers are given, required
-// when hp->apply_update), the seed-group launches of the training kernel, the fixed-order reduce and the logged metrics.
-// On BNN_OK the reduced gradient and its per-block sums of squares are enqueued on st for the update kernel.
-struct Gradient { const float* grad; const float* sq; int nb, d; };
-static int train_gradient(const char* who, bool state_ok, const char* state_name, const bnn_model_config* cfg,
-                          const bnn_train_hparams* hp, int32_t n_seeds, const float* d_theta, const float* d_x,
-                          const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
-                          const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_metrics,
-                          void* d_workspace, cudaStream_t st, Gradient* out) {
-    int rc = validate_config(cfg);
-    if (rc != BNN_OK) return rc;
-    if ((rc = check_device()) != BNN_OK) return rc;
-    BNN_REQUIRE(hp && d_theta && d_x && d_y && d_workspace, BNN_E_ARG, "%s: null pointer", who);
+// bytes of the workspace of a step of n_seeds seeds at n_cta CTAs per seed: partial | grad | sq | pad | head records (v3)
+// | input-tile scratch
+static size_t workspace_bytes(const bnn_model_config* cfg, int64_t B, int32_t n_seeds, int n_cta) {
+    const size_t DP = FlatLayout(cfg->n_features).d + DPAD;
+    const size_t nb = (DP + 255) / 256;
+    return ((size_t)n_seeds * n_cta * DP + (size_t)n_seeds * DP + (size_t)n_seeds * nb + 64 + (size_t)n_seeds * B * REC + 4 +
+            (size_t)n_seeds * n_cta * scratch_floats_per_cta(cfg)) * sizeof(float);
+}
+
+static SeedChunk seed_chunk(const bnn_train_hparams* hp, int hp_stride, int s0, int n, int64_t B) {
+    SeedChunk c{};
+    for (int j = 0; j < n; ++j) {
+        const bnn_train_hparams& h = hp[(size_t)(s0 + j) * hp_stride];
+        c.s[j] = SeedHp{h.lr, h.momentum, h.weight_decay, h.clip_norm, h.beta_in, h.beta_out, h.beta_in * (float)B,
+                        h.beta_out * (float)B};
+    }
+    return c;
+}
+
+// The torch.optim.Adam scalars of one step, the bias corrections as torch computes them from Python floats (double),
+// with this step's beta1
+static AdamStep adam_step(const bnn_train_hparams& hp, const bnn_adam_hparams& adam) {
+    const double t = (double)adam.step;
+    AdamStep a;
+    a.step_size = (float)((double)hp.lr / (1.0 - pow(adam.beta1, t)));
+    a.bc2_sqrt = (float)sqrt(1.0 - pow(adam.beta2, t));
+    a.w1 = (float)(1.0 - adam.beta1);
+    a.beta2 = (float)adam.beta2;
+    a.w2 = (float)(1.0 - adam.beta2);
+    a.eps = (float)adam.eps;
+    a.first = adam.step == 1;
+    return a;
+}
+
+// One training step of n_seeds models, shared by the four entries: SGD (adam == null) or Adam.  Seed s's scalars are
+// hp[s * hp_stride] (and adam[s * hp_stride]): stride 0 repeats one struct (bnn_train_step, bnn_train_step_adam),
+// stride 1 reads one per seed (the _seeds entries); first_step and apply_update must be the same for every seed.  Every
+// argument check runs before the device is touched.  Then the seed-group launches of the training kernel and, per chunk
+// of SEED_CHUNK seeds, the fixed-order reduce, the logged metrics and the update.  `who` names the entry in messages;
+// d_state0 / d_state1: the momentum buffer (SGD) or exp_avg / exp_avg_sq (Adam), required when apply_update.
+// plan_seeds > 0: the seed groups and CTAs per seed are pick_plan's for plan_seeds seeds, whatever n_seeds is (0: for
+// n_seeds); a seed's bits depend on its CTA count, so a fixed plan_seeds makes them independent of how many seeds share
+// the call.
+static int train_step(const char* who, const bnn_model_config* cfg, const bnn_train_hparams* hp,
+                      const bnn_adam_hparams* adam, bool is_adam, int hp_stride, int32_t n_seeds, int32_t plan_seeds,
+                      float* d_theta,
+                      float* d_state0, float* d_state1, const float* d_x, const float* d_y, const int32_t* d_batch_index,
+                      int64_t B, const float* d_eps_in, const float* d_eps12, const float* d_eps_sum, uint64_t seed,
+                      uint64_t step, float* d_grad_out, float* d_metrics, void* d_workspace, cudaStream_t st) {
+    BNN_REQUIRE(hp && (!is_adam || adam), BNN_E_ARG, "%s: null pointer", who);
     BNN_REQUIRE(n_seeds >= 1 && n_seeds <= 65535 && B >= 1 && B < (1ll << 30), BNN_E_ARG,
                 "%s: n_seeds=%d B=%lld out of range", who, n_seeds, (long long)B);
-    BNN_REQUIRE(!hp->apply_update || state_ok, BNN_E_ARG, "%s: %s required to update", who, state_name);
+    BNN_REQUIRE(plan_seeds >= 0 && plan_seeds <= 65535, BNN_E_ARG, "%s: plan_seeds=%d (0, or 1..65535)", who, plan_seeds);
+    for (int s = 0; s < n_seeds; ++s) {
+        const bnn_train_hparams& h = hp[(size_t)s * hp_stride];
+        char at[32] = "";
+        if (hp_stride) snprintf(at, sizeof(at), " (seed %d)", s);
+        BNN_REQUIRE(h.first_step == hp[0].first_step && h.apply_update == hp[0].apply_update, BNN_E_ARG,
+                    "%s: first_step and apply_update must be the same for every seed (seed %d differs from seed 0)", who, s);
+        if (!is_adam) continue;
+        // torch.optim.Adam's constructor checks, written so that NaN fails them too
+        const bnn_adam_hparams& a = adam[(size_t)s * hp_stride];
+        BNN_REQUIRE(h.lr >= 0.f, BNN_E_ARG, "%s: invalid learning rate %g%s", who, (double)h.lr, at);
+        BNN_REQUIRE(h.weight_decay >= 0.f, BNN_E_ARG, "%s: invalid weight_decay %g%s", who, (double)h.weight_decay, at);
+        BNN_REQUIRE(a.beta1 >= 0.0 && a.beta1 < 1.0, BNN_E_ARG, "%s: invalid beta1 %g (need [0, 1))%s", who, a.beta1, at);
+        BNN_REQUIRE(a.beta2 >= 0.0 && a.beta2 < 1.0, BNN_E_ARG, "%s: invalid beta2 %g (need [0, 1))%s", who, a.beta2, at);
+        BNN_REQUIRE(a.eps >= 0.0, BNN_E_ARG, "%s: invalid eps %g%s", who, a.eps, at);
+        BNN_REQUIRE(a.step >= 1, BNN_E_ARG, "%s: step %lld (t is 1-based)%s", who, (long long)a.step, at);
+    }
+    const int first_step = hp[0].first_step, apply_update = hp[0].apply_update;
+    int rc = validate_config(cfg);
+    if (rc != BNN_OK) return rc;
+    BNN_REQUIRE(d_theta && d_x && d_y && d_workspace, BNN_E_ARG, "%s: null pointer", who);
+    BNN_REQUIRE(!apply_update || (d_state0 && (!is_adam || d_state1)), BNN_E_ARG, "%s: %s required to update", who,
+                is_adam ? "exp_avg and exp_avg_sq" : "momentum buffer");
     const bool any = d_eps_in || d_eps12 || d_eps_sum, all = d_eps_in && d_eps12 && d_eps_sum;
     BNN_REQUIRE(!any || all, BNN_E_ARG, "%s: give all of eps_in, eps12, eps_sum or none", who);
     BNN_REQUIRE(aligned16(d_workspace) && (!d_eps12 || (aligned16(d_eps12) && aligned16(d_eps_sum))), BNN_E_ALIGN,
                 "%s: workspace / eps12 / eps_sum must be 16-byte aligned", who);
     const int F = cfg->n_features, T = cfg->n_times, FP = (F + 3) & ~3;
     BNN_REQUIRE(shape_ok(cfg), BNN_E_CONFIG, "%s: compiled for the reference's shape T=100, F=41 (got T=%d, F=%d)", who, T, F);
+    if ((rc = check_device()) != BNN_OK) return rc;
     const FlatLayout fl(F);
-    const SeedPlan plan = pick_plan(cfg, B, n_seeds);
+    const SeedPlan plan = pick_plan(cfg, B, plan_seeds ? plan_seeds : n_seeds);
     const int n_cta = plan.n_cta;
     const int DP = fl.d + DPAD, nb = (DP + 255) / 256;
     float* partial = (float*)d_workspace;
@@ -377,40 +458,56 @@ static int train_gradient(const char* who, bool state_ok, const char* state_name
     prm.B = (int)B; prm.T = T; prm.F = F; prm.FP = FP; prm.n_cta = n_cta; prm.seed0 = 0;
     prm.seed = seed; prm.step = step; prm.zero_mask = cfg->zero_mask;
     prm.hc = HeadConsts{cfg->lo_mu, cfg->hi_mu, cfg->lo_sd, cfg->hi_sd};
-    prm.beta_out = hp->beta_out;
     prm.saliency = 0; prm.gx_out = nullptr; prm.mu_out = nullptr;
-    if (use_tc(cfg, B)) {
-        const size_t smem_tc = (size_t)tcx::SmemTC(cfg->zero_mask).total * sizeof(float);
+    const bool tc = use_tc(cfg, B);
+    const size_t smem = tc ? (size_t)tcx::SmemTC(cfg->zero_mask).total * sizeof(float) : (size_t)Smem3(T, F).total * sizeof(float);
+    if (tc) {
         static PerDeviceOnce attr_tc_done;
         if (attr_tc_done.need()) {
             BNN_CUDA(cudaFuncSetAttribute(train_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         }
-        for (int s0 = 0; s0 < n_seeds; s0 += plan.per) {   // seed groups (pick_plan); every buffer is indexed by the global seed
-            prm.seed0 = s0;
-            train_tc_kernel<<<dim3(n_cta, n_seeds - s0 < plan.per ? n_seeds - s0 : plan.per), tcx::NTHR_TC, smem_tc, st>>>(prm);
-        }
     } else {
-        const size_t smem3 = (size_t)Smem3(T, F).total * sizeof(float);
         static PerDeviceOnce attr3_done;
         if (attr3_done.need()) {
             BNN_CUDA(cudaFuncSetAttribute(train_fwd_bwd3_kernel<100, 41>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           227 * 1024));
         }
-        for (int s0 = 0; s0 < n_seeds; s0 += plan.per) {
+    }
+    // A group of more than TRAIN_SEED_CHUNK seeds runs one CTA per seed (pick_plan) and so more CTAs than SMs: it is
+    // split into launches of a whole number of waves, which take as many waves in all as the group in one launch.
+    const int sms = sm_count();
+    const int sub = sms <= TRAIN_SEED_CHUNK ? TRAIN_SEED_CHUNK / sms * sms : TRAIN_SEED_CHUNK;
+    for (int g0 = 0; g0 < n_seeds; g0 += plan.per) {   // seed groups (pick_plan); every buffer is indexed by the global seed
+        const int g1 = n_seeds < g0 + plan.per ? n_seeds : g0 + plan.per;
+        for (int s0 = g0; s0 < g1; s0 += sub) {
+            const int n = g1 - s0 < sub ? g1 - s0 : sub;
             prm.seed0 = s0;
-            train_fwd_bwd3_kernel<100, 41><<<dim3(n_cta, n_seeds - s0 < plan.per ? n_seeds - s0 : plan.per), NTHR3, smem3, st>>>(
-                prm);
+            for (int j = 0; j < n; ++j) prm.beta_out[j] = hp[(size_t)(s0 + j) * hp_stride].beta_out;
+            if (tc) train_tc_kernel<<<dim3(n_cta, n), tcx::NTHR_TC, smem, st>>>(prm);
+            else train_fwd_bwd3_kernel<100, 41><<<dim3(n_cta, n), NTHR3, smem, st>>>(prm);
         }
     }
     BNN_CUDA(cudaGetLastError());
-    train_reduce_kernel<<<dim3(nb, n_seeds), 256, 0, st>>>(partial, d_theta, n_cta, fl.d, F, hp->beta_in * (float)B,
-                                                          hp->beta_out * (float)B, grad, sq);
-    BNN_CUDA(cudaGetLastError());
-    if (d_metrics) {
-        train_metrics_kernel<<<n_seeds, 32, 0, st>>>(d_theta, grad, fl.d, F, (int)B, *hp, d_metrics);
+    for (int s0 = 0; s0 < n_seeds; s0 += SEED_CHUNK) {   // seeds are independent from here on: chunk after chunk
+        const int n = n_seeds - s0 < SEED_CHUNK ? n_seeds - s0 : SEED_CHUNK;
+        const SeedChunk hc = seed_chunk(hp, hp_stride, s0, n, B);
+        train_reduce_kernel<<<dim3(nb, n), 256, 0, st>>>(partial, d_theta, n_cta, fl.d, F, s0, hc, grad, sq);
+        BNN_CUDA(cudaGetLastError());
+        if (d_metrics) {
+            train_metrics_kernel<<<n, 32, 0, st>>>(d_theta, grad, fl.d, F, (int)B, s0, hc, d_metrics);
+            BNN_CUDA(cudaGetLastError());
+        }
+        if (is_adam) {
+            AdamChunk ac{};
+            for (int j = 0; j < n; ++j) ac.a[j] = adam_step(hp[(size_t)(s0 + j) * hp_stride], adam[(size_t)(s0 + j) * hp_stride]);
+            train_adam_update_kernel<<<dim3(nb, n), 256, 0, st>>>(grad, sq, nb, fl.d, (int)B, s0, hc, ac, apply_update,
+                                                                  d_theta, d_state0, d_state1, d_grad_out, d_metrics);
+        } else {
+            train_update_kernel<<<dim3(nb, n), 256, 0, st>>>(grad, sq, nb, fl.d, (int)B, s0, hc, first_step, apply_update,
+                                                             d_theta, d_state0, d_grad_out, d_metrics);
+        }
         BNN_CUDA(cudaGetLastError());
     }
-    *out = Gradient{grad, sq, nb, fl.d};
     return BNN_OK;
 }
 
@@ -452,7 +549,7 @@ static int saliency_launch(const bnn_model_config* cfg, int32_t n_models, const 
     prm.B = (int)B; prm.T = T; prm.F = F; prm.FP = (F + 3) & ~3; prm.n_cta = (int)n_cta; prm.seed0 = 0;
     prm.seed = seed; prm.step = 0; prm.zero_mask = cfg->zero_mask;
     prm.hc = HeadConsts{cfg->lo_mu, cfg->hi_mu, cfg->lo_sd, cfg->hi_sd};
-    prm.beta_out = 0.f;
+    prm.beta_out[0] = 0.f;   // every model reads entry 0 (train_v3.cuh)
     prm.saliency = 1; prm.gx_out = d_grad_x; prm.mu_out = d_mu;
     static PerDeviceOnce attr_done;
     if (attr_done.need()) {
@@ -552,31 +649,31 @@ extern "C" {
 size_t bnn_train_workspace_bytes(const bnn_model_config* cfg, int64_t B, int32_t n_seeds) {
     using namespace bnn;
     if (validate_config(cfg) != BNN_OK || B <= 0 || n_seeds <= 0) return 0;
-    const int d = FlatLayout(cfg->n_features).d;
-    const int n_cta = train::pick_n_cta(cfg, B, n_seeds);
-    const size_t DP = d + train::DPAD;
-    const size_t nb = (DP + 255) / 256;
-    // partial | grad | sq | pad | head records (v3)
-    return ((size_t)n_seeds * n_cta * DP + (size_t)n_seeds * DP + (size_t)n_seeds * nb + 64 +
-            (size_t)n_seeds * B * train::REC + 4 +
-            (size_t)n_seeds * n_cta * train::scratch_floats_per_cta(cfg)) * sizeof(float);
+    return train::workspace_bytes(cfg, B, n_seeds, train::pick_plan(cfg, B, n_seeds).n_cta);
+}
+
+size_t bnn_train_workspace_bytes_seeds(const bnn_model_config* cfg, int64_t B, int32_t n_seeds, int32_t plan_seeds) {
+    using namespace bnn;
+    if (validate_config(cfg) != BNN_OK || B <= 0 || n_seeds <= 0 || plan_seeds < 0 || plan_seeds > 65535) return 0;
+    return train::workspace_bytes(cfg, B, n_seeds, train::pick_plan(cfg, B, plan_seeds ? plan_seeds : n_seeds).n_cta);
 }
 
 int bnn_train_step(const bnn_model_config* cfg, const bnn_train_hparams* hp, int32_t n_seeds, float* d_theta,
                    float* d_momentum, const float* d_x, const float* d_y, const int32_t* d_batch_index, int64_t B,
                    const float* d_eps_in, const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
                    float* d_grad_out, float* d_metrics, void* d_workspace, void* stream) {
-    using namespace bnn;
-    cudaStream_t st = (cudaStream_t)stream;
-    train::Gradient gr;
-    const int rc = train::train_gradient("bnn_train_step", d_momentum, "momentum buffer", cfg, hp, n_seeds, d_theta, d_x, d_y,
-                                        d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step, d_metrics, d_workspace,
-                                        st, &gr);
-    if (rc != BNN_OK) return rc;
-    train::train_update_kernel<<<dim3(gr.nb, n_seeds), 256, 0, st>>>(gr.grad, gr.sq, gr.nb, gr.d, (int)B, *hp, d_theta,
-                                                                    d_momentum, d_grad_out, d_metrics);
-    BNN_CUDA(cudaGetLastError());
-    return BNN_OK;
+    return bnn::train::train_step("bnn_train_step", cfg, hp, nullptr, false, 0, n_seeds, 0, d_theta, d_momentum, nullptr, d_x,
+                                  d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step, d_grad_out, d_metrics,
+                                  d_workspace, (cudaStream_t)stream);
+}
+
+int bnn_train_step_seeds(const bnn_model_config* cfg, const bnn_train_hparams* hp, int32_t n_seeds, int32_t plan_seeds,
+                         float* d_theta, float* d_momentum, const float* d_x, const float* d_y, const int32_t* d_batch_index, int64_t B,
+                         const float* d_eps_in, const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
+                         float* d_grad_out, float* d_metrics, void* d_workspace, void* stream) {
+    return bnn::train::train_step("bnn_train_step_seeds", cfg, hp, nullptr, false, 1, n_seeds, plan_seeds, d_theta, d_momentum, nullptr,
+                                  d_x, d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step, d_grad_out,
+                                  d_metrics, d_workspace, (cudaStream_t)stream);
 }
 
 int bnn_train_step_adam(const bnn_model_config* cfg, const bnn_train_hparams* hp, const bnn_adam_hparams* adam,
@@ -584,38 +681,19 @@ int bnn_train_step_adam(const bnn_model_config* cfg, const bnn_train_hparams* hp
                         const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
                         const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_grad_out,
                         float* d_metrics, void* d_workspace, void* stream) {
-    using namespace bnn;
-    // torch.optim.Adam's constructor checks, written so that NaN fails them too
-    BNN_REQUIRE(hp && adam, BNN_E_ARG, "bnn_train_step_adam: null pointer");
-    BNN_REQUIRE(hp->lr >= 0.f, BNN_E_ARG, "bnn_train_step_adam: invalid learning rate %g", (double)hp->lr);
-    BNN_REQUIRE(hp->weight_decay >= 0.f, BNN_E_ARG, "bnn_train_step_adam: invalid weight_decay %g", (double)hp->weight_decay);
-    BNN_REQUIRE(adam->beta1 >= 0.0 && adam->beta1 < 1.0, BNN_E_ARG, "bnn_train_step_adam: invalid beta1 %g (need [0, 1))",
-                adam->beta1);
-    BNN_REQUIRE(adam->beta2 >= 0.0 && adam->beta2 < 1.0, BNN_E_ARG, "bnn_train_step_adam: invalid beta2 %g (need [0, 1))",
-                adam->beta2);
-    BNN_REQUIRE(adam->eps >= 0.0, BNN_E_ARG, "bnn_train_step_adam: invalid eps %g", adam->eps);
-    BNN_REQUIRE(adam->step >= 1, BNN_E_ARG, "bnn_train_step_adam: step %lld (t is 1-based)", (long long)adam->step);
-    cudaStream_t st = (cudaStream_t)stream;
-    train::Gradient gr;
-    const int rc = train::train_gradient("bnn_train_step_adam", d_exp_avg && d_exp_avg_sq, "exp_avg and exp_avg_sq", cfg, hp,
-                                        n_seeds, d_theta, d_x, d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step,
-                                        d_metrics, d_workspace, st, &gr);
-    if (rc != BNN_OK) return rc;
-    // bias corrections as torch computes them from Python floats, with this step's beta1
-    const double t = (double)adam->step;
-    train::AdamStep a;
-    a.step_size = (float)((double)hp->lr / (1.0 - pow(adam->beta1, t)));
-    a.bc2_sqrt = (float)sqrt(1.0 - pow(adam->beta2, t));
-    a.w1 = (float)(1.0 - adam->beta1);
-    a.beta2 = (float)adam->beta2;
-    a.w2 = (float)(1.0 - adam->beta2);
-    a.eps = (float)adam->eps;
-    a.first = adam->step == 1;
-    train::train_adam_update_kernel<<<dim3(gr.nb, n_seeds), 256, 0, st>>>(gr.grad, gr.sq, gr.nb, gr.d, (int)B, *hp, a,
-                                                                         d_theta, d_exp_avg, d_exp_avg_sq, d_grad_out,
-                                                                         d_metrics);
-    BNN_CUDA(cudaGetLastError());
-    return BNN_OK;
+    return bnn::train::train_step("bnn_train_step_adam", cfg, hp, adam, true, 0, n_seeds, 0, d_theta, d_exp_avg, d_exp_avg_sq,
+                                  d_x, d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step, d_grad_out,
+                                  d_metrics, d_workspace, (cudaStream_t)stream);
+}
+
+int bnn_train_step_adam_seeds(const bnn_model_config* cfg, const bnn_train_hparams* hp, const bnn_adam_hparams* adam,
+                              int32_t n_seeds, int32_t plan_seeds, float* d_theta, float* d_exp_avg, float* d_exp_avg_sq, const float* d_x,
+                              const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
+                              const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_grad_out,
+                              float* d_metrics, void* d_workspace, void* stream) {
+    return bnn::train::train_step("bnn_train_step_adam_seeds", cfg, hp, adam, true, 1, n_seeds, plan_seeds, d_theta, d_exp_avg,
+                                  d_exp_avg_sq, d_x, d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step,
+                                  d_grad_out, d_metrics, d_workspace, (cudaStream_t)stream);
 }
 
 int bnn_saliency(const bnn_model_config* cfg, int32_t n_models, const float* d_theta, const float* d_x, int64_t B,

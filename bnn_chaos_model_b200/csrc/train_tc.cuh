@@ -870,7 +870,7 @@ __global__ void __launch_bounds__(tcx::NTHR_TC, 1) train_tc_kernel(const Params 
                 if (lane < 10) {
                     const float g = (a + a1) + a2;
                     rec[R_DLVS + hj] = g * (0.5f * (sv[V3_ESN + hj] * cst[C3_ELVH + hj]));   // ds'/dlv = eps e^{lv/2} / 2
-                    sv[V3_GS + hj] = g + prm.beta_out * sv[V3_S + hj];
+                    sv[V3_GS + hj] = g + prm.beta_out[blockIdx.y] * sv[V3_S + hj];
                 }
                 // the record of the deferred head outer products: s', r1, r2, g_a1h, g_a2h (complete since the last barrier)
                 for (int i = lt; i < R_DLVS; i += 128) rec[i] = sv[V3_REC0 + i];

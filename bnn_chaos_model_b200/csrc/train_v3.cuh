@@ -981,7 +981,7 @@ __global__ void __launch_bounds__(NTHR3, 1) train_fwd_bwd3_kernel(const Params p
             a += __shfl_xor_sync(0xffffffffu, a, 2);
             if (part == 0) {
                 if (act && !prm.saliency) rec[R_DLVS + k] = a * (0.5f * (sv[V3_ESN + k] * cst[C3_ELVH + k]));  // ds'/dlv = eps e^{lv/2} / 2
-                sv[V3_GS + k] = a + (act ? prm.beta_out * sv[V3_S + k] : 0.f);
+                sv[V3_GS + k] = a + (act ? prm.beta_out[prm.saliency ? 0 : blockIdx.y] * sv[V3_S + k] : 0.f);
             }
         } else if (act && !prm.saliency) {
             // the other warp of the half writes the record (s', r1, r2, g_a1, g_a2 are complete)

@@ -62,9 +62,10 @@ def default_hparams(args, seed: int, swa_steps: int, epochs: int) -> dict:
     }
 
 
-def gather_seed_statistics(trainer: MultiSeedSWAGTrainer, n_seeds: int, group=None):
+def gather_seed_statistics(trainer: MultiSeedSWAGTrainer, n_seeds: int, group=None, extra: Optional[torch.Tensor] = None):
     """The job's only collective: every rank's (theta, w_avg, w2_avg, pre_D [d, K], n_models, n_cols) for its seeds,
-    padded to the largest seed group, all-gathered once.  Returns per-seed tensors in seed order (on every rank)."""
+    padded to the largest seed group, all-gathered once.  Returns per-seed tensors in seed order (on every rank).
+    ``extra`` [S, k] (optional): k more floats per seed, gathered in the same collective and returned as "extra"."""
     import torch.distributed as dist
 
     world = dist.get_world_size(group) if dist.is_initialized() else 1
@@ -72,14 +73,17 @@ def gather_seed_statistics(trainer: MultiSeedSWAGTrainer, n_seeds: int, group=No
     smax, S = max(counts), trainer.S
     d, K = trainer.theta.shape[1], trainer.K
     dev = trainer.theta.device
-    per = 3 * d + d * K + 2
+    k = 0 if extra is None else extra.shape[1]
+    per = 3 * d + d * K + 2 + k
     send = torch.zeros((smax, per), device=dev)
     send[:S, :d] = trainer.theta
     send[:S, d:2 * d] = trainer.w_avg
     send[:S, 2 * d:3 * d] = trainer.w2_avg
     send[:S, 3 * d:3 * d + d * K] = trainer.pre_D.reshape(S, d * K)
-    send[:S, -2] = trainer.n_models.float()
-    send[:S, -1] = trainer.n_cols.float()
+    send[:S, 3 * d + d * K] = trainer.n_models.float()
+    send[:S, 3 * d + d * K + 1] = trainer.n_cols.float()
+    if k:
+        send[:S, per - k:] = extra
     if world > 1:
         recv = torch.empty((world * smax, per), device=dev)
         dist.all_gather_into_tensor(recv, send, group=group)
@@ -87,8 +91,12 @@ def gather_seed_statistics(trainer: MultiSeedSWAGTrainer, n_seeds: int, group=No
     else:
         rows = send[:S]
     assert rows.shape[0] == n_seeds
-    return {"theta": rows[:, :d], "w_avg": rows[:, d:2 * d], "w2_avg": rows[:, 2 * d:3 * d],
-            "pre_D": rows[:, 3 * d:3 * d + d * K].reshape(n_seeds, d, K), "n_models": rows[:, -2].long(), "n_cols": rows[:, -1].long()}
+    out = {"theta": rows[:, :d], "w_avg": rows[:, d:2 * d], "w2_avg": rows[:, 2 * d:3 * d],
+           "pre_D": rows[:, 3 * d:3 * d + d * K].reshape(n_seeds, d, K), "n_models": rows[:, 3 * d + d * K].long(),
+           "n_cols": rows[:, 3 * d + d * K + 1].long()}
+    if k:
+        out["extra"] = rows[:, per - k:]
+    return out
 
 
 def write_outputs(stats: dict, models_hparams: Sequence[dict], swa_params: dict, names: Sequence[str], out_dir: str,
@@ -162,8 +170,21 @@ def build_parser():
     return ap
 
 
-def main(argv=None):
+def load_data(args):
+    """(X_train, y_train, X_val, y_val) from --data, else from the synthetic generator (--synthetic)."""
     import numpy as np
+
+    if args.data:
+        z = np.load(args.data)
+        return tuple(torch.from_numpy(z[k]) for k in ("X_train", "y_train", "X_val", "y_val"))
+    from . import synth
+
+    nt, nv = args.synthetic
+    return (torch.from_numpy(synth.make_systems(nt, seed=1)), torch.from_numpy(synth.make_labels(nt, seed=1)),
+            torch.from_numpy(synth.make_systems(nv, seed=2)), torch.from_numpy(synth.make_labels(nv, seed=2)))
+
+
+def main(argv=None):
     import torch.distributed as dist
 
     args = build_parser().parse_args(argv)
@@ -172,16 +193,7 @@ def main(argv=None):
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    if args.data:
-        z = np.load(args.data)
-        Xt, yt, Xv, yv = (torch.from_numpy(z[k]) for k in ("X_train", "y_train", "X_val", "y_val"))
-    else:
-        from . import synth
-
-        nt, nv = args.synthetic
-        Xt, yt = torch.from_numpy(synth.make_systems(nt, seed=1)), torch.from_numpy(synth.make_labels(nt, seed=1))
-        Xv, yv = torch.from_numpy(synth.make_systems(nv, seed=2)), torch.from_numpy(synth.make_labels(nv, seed=2))
-    paths, trainer, logs = run(args, Xt, yt, Xv, yv, args.out)
+    paths, trainer, logs = run(args, *load_data(args), args.out)
     if paths is not None:
         last = logs[-1] if logs else {}
         print(f"wrote {len(paths)} SWAG checkpoints to {args.out}; epochs {trainer.current_epoch}, steps {trainer.global_step}; "

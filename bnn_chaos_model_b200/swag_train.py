@@ -31,6 +31,24 @@ def seeds_of_rank(n_seeds: int, rank: int, world: int):
     return list(range(lo, hi))
 
 
+GOLDEN = 0x9E3779B97F4A7C15   # the step of the per-seed Philox keys (csrc/train.cu seed_key)
+
+
+def run_key(seed: int, run: int) -> int:
+    """The seed argument under which index 0 of a fused call gets the Philox key of index ``run`` (seed_key(seed, i) =
+    seed + GOLDEN (i + 1) mod 2^64, so a call's index i then draws what index run + i draws under ``seed``)."""
+    return (int(seed) + GOLDEN * int(run)) % (1 << 64)
+
+
+def check_shared(models, key: str, get):
+    """ValueError naming ``key`` unless ``get(model)`` is the same for every model: a value one fused job cannot give
+    each seed its own of (the run's length, the batch, the collection start, the validation mode)."""
+    vals = [get(m) for m in models]
+    if any(v != vals[0] for v in vals[1:]):
+        raise ValueError(f"{key} must be the same for every seed model of one trainer, got {vals}")
+    return vals[0]
+
+
 def check_optimizer(optimizer: str, betas, eps):
     """The optimizer name and torch.optim.Adam's checks of betas / eps, as ValueError.  Returns (beta1, beta2, eps)."""
     if optimizer not in ("sgd", "adam"):
@@ -57,16 +75,40 @@ class MultiSeedSWAGTrainer:
     ``optimizer`` -- "sgd" (the reference's SGD with hparams['momentum']) or "adam": torch.optim.Adam with ``betas`` and
     ``eps`` (amsgrad off, L2 weight decay hparams['weight_decay']) on the same clipped gradient; per seed it keeps
     ``exp_avg`` / ``exp_avg_sq`` and counts its steps in ``adam_step``.  Validation, ``collect`` and ``export`` do not
-    depend on the choice."""
+    depend on the choice.
+
+    Each seed trains with its own model's scalars: swa_params['swa_lr'] and ['swa_recording_lr_factor'],
+    hparams['momentum'] and ['weight_decay'], beta_in and beta_out (one ``bnn_train_step_seeds`` call carries them all;
+    ``seed_hparams`` lists them per step), so a grid of configs x seeds trains as one job.  Before, every seed silently
+    trained with the first model's values.  What one fused job cannot vary -- hparams['swa_start'] and noisy_val when
+    not given here, swa_params['swa_start'] with ``lr_milestone`` -- raises ValueError naming the key when the models
+    differ.  ``lr``, ``lr_factor`` and ``hp`` hold the first seed's values.
+
+    ``first_run`` -- the global index of seed 0 when one job's runs are split over ranks (the sweep driver): seed i's
+    Philox keys, batch shuffle and validation draws then depend on (seed, first_run + i) alone, so a run draws the same
+    numbers on whichever rank it lands.  Default: keyed on the local index with one shuffle generator, as before.
+    ``plan_seeds`` -- plan the fused step's seed groups and CTAs per seed for that many seeds rather than for this
+    trainer's count (``bnn_train_step_seeds``): a seed's bits depend on its CTA count, so with ``first_run`` and a fixed
+    ``plan_seeds`` a run trains to the same bits however the runs are split over ranks."""
 
     def __init__(self, models: Sequence[SWAGModel], X_train, y_train, X_val=None, y_val=None, batch_size=2000,
                  device=None, seed=0, swa_start: Optional[int] = None, noisy_val: Optional[bool] = None,
-                 lr_milestone: bool = True, optimizer: str = "sgd", betas=(0.9, 0.999), eps: float = 1e-8):
+                 lr_milestone: bool = True, optimizer: str = "sgd", betas=(0.9, 0.999), eps: float = 1e-8,
+                 first_run: Optional[int] = None, plan_seeds: Optional[int] = None):
         beta1, beta2, eps = check_optimizer(optimizer, betas, eps)   # before anything touches a device
+        if plan_seeds is not None and not 1 <= int(plan_seeds) <= 65535:
+            raise ValueError(f"plan_seeds must be in [1, 65535], got {plan_seeds}")
+        self.plan_seeds = 0 if plan_seeds is None else int(plan_seeds)
         self.optimizer, self.betas, self.eps = optimizer, (beta1, beta2), eps
         if len(models) == 0:
             raise ValueError("no seed models")
         self.models: List[SWAGModel] = list(models)
+        if noisy_val is None:
+            check_shared(self.models, "noisy_val", lambda m: bool(m.hparams.get("noisy_val", True)))
+        if swa_start is None:
+            check_shared(self.models, "swa_start", lambda m: int(m.hparams["swa_start"]))
+        if lr_milestone:
+            check_shared(self.models, "swa_params['swa_start']", lambda m: (getattr(m, "swa_params", None) or {}).get("swa_start"))
         self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
         if self.device.type != "cuda":
             raise BnnChaosError("MultiSeedSWAGTrainer needs a CUDA device: there is no CPU fallback")
@@ -107,45 +149,71 @@ class MultiSeedSWAGTrainer:
         self.first_step = True
         self._ws = None
         self._ws_val = None
-        self._gen = torch.Generator(device=dev)
-        self._gen.manual_seed(self.seed)
-        self.lr = float(m0.swa_params["swa_lr"])
-        self.hp = dict(momentum=float(m0.hparams["momentum"]), weight_decay=float(m0.hparams["weight_decay"]),
-                       clip_norm=0.1 * d, beta_in=float(m0.beta_in), beta_out=float(m0.beta_out))  # run_swag.py:61
+        self.first_run = None if first_run is None else int(first_run)
+        if self.first_run is None:
+            self._gen = torch.Generator(device=dev)
+            self._gen.manual_seed(self.seed)
+        else:
+            self._gens = [torch.Generator(device=dev) for _ in range(self.S)]
+            for i, g in enumerate(self._gens):
+                g.manual_seed(run_key(self.seed, self.first_run + i) % (1 << 63))
+        self.seed_hp = [dict(lr=float(m.swa_params["swa_lr"]),
+                             lr_factor=float((getattr(m, "swa_params", None) or {}).get("swa_recording_lr_factor", 0.5)),
+                             momentum=float(m.hparams["momentum"]), weight_decay=float(m.hparams["weight_decay"]),
+                             clip_norm=0.1 * d, beta_in=float(m.beta_in), beta_out=float(m.beta_out))  # run_swag.py:61
+                        for m in self.models]
+        self.lr = self.seed_hp[0]["lr"]
+        self.hp = {k: v for k, v in self.seed_hp[0].items() if k not in ("lr", "lr_factor")}
 
     # ------------------------------------------------------------------ one optimisation step, all seeds
     def train_step(self, batch_index: Optional[torch.Tensor], B: int, lr: Optional[float] = None):
+        """One fused optimizer step of every seed, each with its own scalars (``seed_hparams``); ``lr`` given: that
+        learning rate for every seed."""
         lib = _lib.load()
         cfg = self.models[0].config(self.X.shape[1])
-        hp = TrainHParams(lr=self.step_lr() if lr is None else float(lr), first_step=int(self.first_step), apply_update=1,
-                          **self.step_hparams())
+        per_seed = self.seed_hparams()
+        hp = (TrainHParams * self.S)(*(
+            TrainHParams(lr=h["lr"] if lr is None else float(lr), momentum=h["momentum"], weight_decay=h["weight_decay"],
+                         clip_norm=h["clip_norm"], beta_in=h["beta_in"], beta_out=h["beta_out"],
+                         first_step=int(self.first_step), apply_update=1) for h in per_seed))
         with torch.cuda.device(self.device), _lib.nvtx("bnn:K4 train_step"):
-            nbytes = lib.bnn_train_workspace_bytes(cfg, B, self.S)
+            nbytes = lib.bnn_train_workspace_bytes_seeds(cfg, B, self.S, self.plan_seeds)
             if self._ws is None or self._ws.numel() * 4 < nbytes:
                 self._ws = torch.empty((nbytes + 3) // 4, device=self.device, dtype=torch.float32)
-            rest = (_lib.ptr(self.X), _lib.ptr(self.y), _lib.ptr(batch_index), B, None, None, None, self.seed, self.global_step,
+            seed = self.seed if self.first_run is None else run_key(self.seed, self.first_run)
+            rest = (_lib.ptr(self.X), _lib.ptr(self.y), _lib.ptr(batch_index), B, None, None, None, seed, self.global_step,
                     None, _lib.ptr(self.metrics), _lib.ptr(self._ws), _lib.current_stream_ptr())
             if self.optimizer == "adam":
-                adam = AdamHParams(beta1=self.step_beta1(), beta2=self.betas[1], eps=self.eps, step=self.adam_step + 1)
-                _lib.check(lib.bnn_train_step_adam(cfg, hp, adam, self.S, _lib.ptr(self.theta), _lib.ptr(self.exp_avg),
-                                                   _lib.ptr(self.exp_avg_sq), *rest), "bnn_train_step_adam")
+                adam = (AdamHParams * self.S)(*(AdamHParams(beta1=h["beta1"], beta2=self.betas[1], eps=self.eps,
+                                                            step=self.adam_step + 1) for h in per_seed))
+                _lib.check(lib.bnn_train_step_adam_seeds(cfg, hp, adam, self.S, self.plan_seeds, _lib.ptr(self.theta),
+                                                         _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq), *rest),
+                           "bnn_train_step_adam_seeds")
                 self.adam_step += 1
             else:
-                _lib.check(lib.bnn_train_step(cfg, hp, self.S, _lib.ptr(self.theta), _lib.ptr(self.momentum), *rest),
-                           "bnn_train_step")
+                _lib.check(lib.bnn_train_step_seeds(cfg, hp, self.S, self.plan_seeds, _lib.ptr(self.theta),
+                                                    _lib.ptr(self.momentum), *rest), "bnn_train_step_seeds")
         self.first_step = False
         self.global_step += 1
 
+    def seed_hparams(self, step: Optional[int] = None) -> List[dict]:
+        """Per seed, the scalars of optimizer step ``step`` (default: the coming one): lr, momentum, weight_decay,
+        clip_norm, beta_in, beta_out and Adam's beta1 -- what ``train_step`` hands the fused step for that seed."""
+        g = self.global_step if step is None else int(step)
+        milestone = self.lr_milestone is not None and g >= self.lr_milestone
+        return [dict(lr=h["lr"] * h["lr_factor"] if milestone else h["lr"], momentum=h["momentum"],
+                     weight_decay=h["weight_decay"], clip_norm=h["clip_norm"], beta_in=h["beta_in"], beta_out=h["beta_out"],
+                     beta1=self.betas[0]) for h in self.seed_hp]
+
     def step_lr(self, step: Optional[int] = None) -> float:
         """Learning rate of optimizer step ``step`` (default: the coming one): swa_lr, times swa_recording_lr_factor from
-        step swa_params['swa_start'] on (torch MultiStepLR stepped once per optimizer step, :709-720)."""
-        g = self.global_step if step is None else int(step)
-        if self.lr_milestone is not None and g >= self.lr_milestone:
-            return self.lr * self.lr_factor
-        return self.lr
+        step swa_params['swa_start'] on (torch MultiStepLR stepped once per optimizer step, :709-720).  The first seed's;
+        every seed's: ``seed_hparams``."""
+        return self.seed_hparams(step)[0]["lr"]
 
     def step_hparams(self):
-        """momentum, weight decay, clip and KL weights of the coming step (constant in the SWAG phase, :722-732)."""
+        """momentum, weight decay, clip and KL weights of the coming step (constant in the SWAG phase, :722-732), the
+        first seed's; every seed's: ``seed_hparams``."""
         return self.hp
 
     def step_beta1(self) -> float:
@@ -155,7 +223,8 @@ class MultiSeedSWAGTrainer:
     def epoch_batches(self):
         """Per-seed shuffles of the training set (DataLoader(shuffle=True), :276): [n_batches] of ([S,B] int32, B)."""
         n = self.X.shape[0]
-        perms = torch.stack([torch.randperm(n, device=self.device, generator=self._gen) for _ in range(self.S)])
+        gens = [self._gen] * self.S if self.first_run is None else self._gens
+        perms = torch.stack([torch.randperm(n, device=self.device, generator=g) for g in gens])
         perms = perms.to(torch.int32)
         out = []
         for lo in range(0, n, self.batch_size):  # the last batch is ragged, like DataLoader without drop_last
@@ -174,12 +243,24 @@ class MultiSeedSWAGTrainer:
         current weights and at w_avg (the current weights where nothing has been collected yet), in one launch.
         noisy_val=False: K2 + the per-unit NLL sum (bnn_eval_loss; eps1, eps2 from Philox).  noisy_val=True: the
         training kernel's noisy forward without update (bnn_train_step, apply_update=0: input noise, eps1, eps2 and
-        summary noise from Philox keyed on (seed ^ 0x5EED; unit, system, epoch)); metrics[:, 0] * B is the summed loss."""
+        summary noise from Philox keyed on (seed ^ 0x5EED; unit, system, epoch)); metrics[:, 0] * B is the summed loss.
+        With ``first_run``, each seed's weight sets are a call of their own under the run's key."""
+        have_avg = bool((self.n_models > 0).all())
+        thetas = torch.cat([self.theta, self.w_avg]) if have_avg else self.theta
+        if self.first_run is None:
+            loss = self._unit_losses(thetas.contiguous(), self.seed ^ 0x5EED)
+        else:
+            per_run = [self._unit_losses(thetas[i::self.S].contiguous(), run_key(self.seed ^ 0x5EED, 2 * (self.first_run + i)))
+                       for i in range(self.S)]
+            loss = torch.cat([torch.stack([u[j] for u in per_run]) for j in range(thetas.shape[0] // self.S)])
+        loss = loss / float(self.test_len)
+        return (loss[: self.S], loss[self.S:] if have_avg else loss[: self.S])
+
+    def _unit_losses(self, thetas, seed: int):
+        """Summed validation loss [U] of the weight vectors thetas [U, d] under the Philox seed ``seed``."""
         lib = _lib.load()
         m0 = self.models[0]
         cfg = m0.config(self.Xv.shape[1])
-        have_avg = bool((self.n_models > 0).all())
-        thetas = (torch.cat([self.theta, self.w_avg]) if have_avg else self.theta).contiguous()
         U, B = thetas.shape[0], self.Xv.shape[0]
         with torch.cuda.device(self.device):
             if self.noisy_val:
@@ -191,7 +272,7 @@ class MultiSeedSWAGTrainer:
                 met = torch.empty((U, 8), device=self.device)
                 _lib.check(
                     lib.bnn_train_step(cfg, hp, U, _lib.ptr(thetas), None, _lib.ptr(self.Xv), _lib.ptr(self.yv), None, B,
-                                       None, None, None, self.seed ^ 0x5EED, self.current_epoch, None, _lib.ptr(met),
+                                       None, None, None, seed, self.current_epoch, None, _lib.ptr(met),
                                        _lib.ptr(self._ws_val), _lib.current_stream_ptr()),
                     "bnn_train_step (noisy validation)",
                 )
@@ -202,11 +283,10 @@ class MultiSeedSWAGTrainer:
                 loss = torch.empty(U, device=self.device)
                 _lib.check(
                     lib.bnn_eval_loss(cfg, _lib.ptr(self.Xv), _lib.ptr(self.yv), B, _lib.ptr(thp), U, None,
-                                      self.seed ^ 0x5EED, _lib.ptr(out), _lib.ptr(loss), None, _lib.current_stream_ptr()),
+                                      seed, _lib.ptr(out), _lib.ptr(loss), None, _lib.current_stream_ptr()),
                     "bnn_eval_loss",
                 )
-        loss = loss / float(self.test_len)
-        return (loss[: self.S], loss[self.S:] if have_avg else loss[: self.S])
+        return loss
 
     def collect(self):
         """aggregate_model (:763-785) for every seed."""
@@ -268,39 +348,58 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
       (ModelCheckpoint, find_minima.py:67,82);
     * the run ends when the scheduler is stepped past its total -- the reference's ValueError
       (:137-139, caught at find_minima.py:79-82) -- after which every seed is reset to its best checkpoint.
+
+    Each seed's one-cycle peak is its own model's ``lr`` and its KL weights anneal towards its own ``beta_in`` /
+    ``beta_out``, with its own weight_decay; the cycled momentum (Adam's beta1) is the same for all.  Before, every
+    seed trained with the first model's values.  ``steps``, ``batch_size`` (when not given here) and noisy_val (when not
+    given here) must be the same for every model, else ValueError naming the key.
     """
 
     def __init__(self, models: Sequence[VarModel], X_train, y_train, X_val=None, y_val=None, batch_size=None,
                  device=None, seed=0, noisy_val: Optional[bool] = None, optimizer: str = "sgd", betas=(0.9, 0.999),
-                 eps: float = 1e-8):
+                 eps: float = 1e-8, first_run: Optional[int] = None, plan_seeds: Optional[int] = None):
+        if len(models) == 0:
+            raise ValueError("no seed models")
         m0 = models[0]
+        check_shared(models, "steps", lambda m: int(m.steps))
+        if batch_size is None:
+            check_shared(models, "batch_size", lambda m: int(m.batch_size))
         for m in models:  # the SWAG bookkeeping of the base class reads these; unused here
             if not hasattr(m, "K"):
                 m.K, m.c, m.swa_params = 1, 1, {"swa_lr": m.lr}
         super().__init__(models, X_train, y_train, X_val, y_val, batch_size=batch_size or m0.batch_size, device=device,
                          seed=seed, swa_start=1 << 62, noisy_val=noisy_val, lr_milestone=False, optimizer=optimizer,
-                         betas=betas, eps=eps)
+                         betas=betas, eps=eps, first_run=first_run, plan_seeds=plan_seeds)
         self.steps = int(m0.steps)
-        self.max_lr = float(m0.lr)
+        self.max_lrs = [float(m.lr) for m in self.models]
+        self.max_lr = self.max_lrs[0]
         self.total_sched = int(0.9 * self.steps)
         self.best_val = torch.full((self.S,), float("inf"), device=self.device)
         self.best_theta = self.theta.clone()
         self.finished = False
 
     def schedule(self, step: Optional[int] = None):
-        """(lr, momentum, beta_in, beta_out) of optimizer step ``step`` (default: the coming one)."""
+        """(lr, momentum, beta_in, beta_out) of optimizer step ``step`` (default: the coming one), the first seed's;
+        every seed's: ``seed_hparams``."""
+        h = self.seed_hparams(step)[0]
+        return h["lr"], h["momentum"], h["beta_in"], h["beta_out"]
+
+    def seed_hparams(self, step: Optional[int] = None) -> List[dict]:
+        """Per seed: the one-cycle lr towards the seed's own peak, the shared cycled momentum (Adam's beta1), and the
+        KL weights annealed towards the seed's own.  Raises ScheduleFinished (a ValueError) past the schedule's end,
+        like scheduler.step()."""
         g = self.global_step if step is None else int(step)
-        lr, mom = one_cycle_lr_momentum(g, self.max_lr, self.total_sched)
         f = min([1, (g / self.steps) / 0.3])
-        return lr, mom, f * self.hp["beta_in"], f * self.hp["beta_out"]
+        out = []
+        for h, max_lr in zip(self.seed_hp, self.max_lrs):
+            lr, mom = one_cycle_lr_momentum(g, max_lr, self.total_sched)
+            out.append(dict(h, lr=lr, momentum=mom, beta_in=f * h["beta_in"], beta_out=f * h["beta_out"], beta1=mom))
+            del out[-1]["lr_factor"]
+        return out
 
     def step_lr(self, step: Optional[int] = None) -> float:
-        """Learning rate of optimizer step ``step`` (default: the coming one): swa_lr, times swa_recording_lr_factor from
-        step swa_params['swa_start'] on (torch MultiStepLR stepped once per optimizer step, :709-720)."""
-        g = self.global_step if step is None else int(step)
-        if self.lr_milestone is not None and g >= self.lr_milestone:
-            return self.lr * self.lr_factor
-        return self.lr
+        """Learning rate of optimizer step ``step`` (default: the coming one), the first seed's one-cycle value."""
+        return self.schedule(step)[0]
 
     def step_hparams(self):
         _, mom, b_in, b_out = self.schedule()
@@ -309,11 +408,6 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
     def step_beta1(self) -> float:
         """The one-cycle momentum of the coming step, Adam's beta1 (CustomOneCycleLR with use_beta1)."""
         return self.schedule()[1]
-
-    def train_step(self, batch_index, B, lr=None):
-        if lr is None:
-            lr = self.schedule()[0]  # raises ScheduleFinished (a ValueError) past the schedule's end, like scheduler.step()
-        super().train_step(batch_index, B, lr)
 
     def fit(self, epochs: Optional[int] = None, validate: bool = True, check_nan_every: int = 1):
         """Trainer.fit of find_minima.py: epochs = 1 + steps / steps_per_epoch unless given; stops at the schedule's end."""

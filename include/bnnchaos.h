@@ -208,6 +208,33 @@ int bnn_train_step_adam(const bnn_model_config* cfg, const bnn_train_hparams* hp
                         const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
                         const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
                         float* d_grad_out, float* d_metrics, void* d_workspace, void* stream);
+
+/* Per-seed hyperparameters (hyperparameter sweeps in one fused job): bnn_train_step / bnn_train_step_adam with HOST
+ * arrays hp [n_seeds] (and adam [n_seeds]).  Seed s uses hp[s] for lr, momentum, weight_decay, clip_norm, beta_in and
+ * beta_out -- in the summary-KL term of its gradient, its KL scales, its clip, its update and its logged metrics -- and
+ * adam[s] for beta1, beta2, eps and t (bias corrections in double per seed, as bnn_train_step_adam computes them).
+ * first_step and apply_update must be equal across seeds.  The values travel in the kernels' parameters: no allocation,
+ * no copy, no synchronisation.  With all entries equal the results are those of the single-struct entry bit for bit, and
+ * seed s's results are those of a call in which every seed carries hp[s] (same plan, same Philox key).  Every other
+ * argument and the workspace (bnn_train_workspace_bytes) as the single-struct entry.  BNN_E_ARG: a null hp / adam, mixed
+ * first_step or apply_update, and (Adam) a seed's lr < 0, weight_decay < 0, beta outside [0, 1), eps < 0 or t < 1, the
+ * message naming the seed; every check runs before the device is touched.
+ * plan_seeds: 0 plans the seed groups and the CTAs per seed for n_seeds, as the single-struct entry does; > 0 plans them
+ * for plan_seeds seeds whatever n_seeds is (n_seeds seeds run in groups of that plan's size, each seed on that plan's
+ * CTAs).  A seed's bits depend on its CTA count, so a fixed plan_seeds gives a seed the same result whichever and
+ * however many seeds share the call: a job split over any number of GPUs trains each run identically.  The workspace is
+ * bnn_train_workspace_bytes_seeds(cfg, B, n_seeds, plan_seeds) bytes (plan_seeds = 0: bnn_train_workspace_bytes). */
+size_t bnn_train_workspace_bytes_seeds(const bnn_model_config* cfg, int64_t B, int32_t n_seeds, int32_t plan_seeds);
+int bnn_train_step_seeds(const bnn_model_config* cfg, const bnn_train_hparams* hp, int32_t n_seeds, int32_t plan_seeds,
+                         float* d_theta, float* d_momentum, const float* d_x, const float* d_y,
+                         const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
+                         const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
+                         float* d_grad_out, float* d_metrics, void* d_workspace, void* stream);
+int bnn_train_step_adam_seeds(const bnn_model_config* cfg, const bnn_train_hparams* hp, const bnn_adam_hparams* adam,
+                              int32_t n_seeds, int32_t plan_seeds, float* d_theta, float* d_exp_avg, float* d_exp_avg_sq, const float* d_x,
+                              const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
+                              const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
+                              float* d_grad_out, float* d_metrics, void* d_workspace, void* stream);
 /* Saliency (figures/feature_importance.py:93-131, gradforward): for each of n_models weight vectors d_theta[m]
  * (flatten() order; the script uses w_avg) and each system b: mu_b = predict_instability(compute_summary_stats(
  * mask(x_b)))[0] and g = d mu_b / d x (all F columns of the masked input; no input noise, no summary noise).
