@@ -121,6 +121,17 @@ SIGNATURES = {
         [_CFG, _HP, _ADAM, C.c_int32, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, C.c_int64, c_f32p, c_f32p, c_f32p,
          C.c_uint64, C.c_uint64, c_f32p, c_f32p, C.c_void_p, C.c_void_p],
     ),
+    # per-seed halt: the _seeds arguments, then d_halted_at [n_seeds] int64 before the stream
+    "bnn_train_step_seeds_halt": (
+        C.c_int,
+        [_CFG, _HP, C.c_int32, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, C.c_int64, c_f32p, c_f32p, c_f32p, C.c_uint64,
+         C.c_uint64, c_f32p, c_f32p, C.c_void_p, C.c_void_p, C.c_void_p],
+    ),
+    "bnn_train_step_adam_seeds_halt": (
+        C.c_int,
+        [_CFG, _HP, _ADAM, C.c_int32, C.c_int32, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, C.c_int64, c_f32p, c_f32p, c_f32p,
+         C.c_uint64, C.c_uint64, c_f32p, c_f32p, C.c_void_p, C.c_void_p, C.c_void_p],
+    ),
     "bnn_train_noise": (
         C.c_int,
         [_CFG, C.c_int32, C.c_int64, C.c_uint64, C.c_uint64, c_f32p, c_f32p, c_f32p, C.c_void_p],
@@ -134,6 +145,11 @@ SIGNATURES = {
         C.c_int,
         [c_f32p, C.c_int64, C.c_int32, C.c_int32, c_f32p, c_f32p, c_f32p, c_i32p, c_i32p, C.c_int32, C.c_int32,
          C.c_void_p],
+    ),
+    "bnn_swag_collect_halt": (
+        C.c_int,
+        [c_f32p, C.c_int64, C.c_int32, C.c_int32, c_f32p, c_f32p, c_f32p, c_i32p, c_i32p, C.c_int32, C.c_int32,
+         C.c_void_p, C.c_void_p],
     ),
     "bnn_pack_inputs": (C.c_int, [c_f32p, c_f32p, c_f32p, c_f32p, C.c_int64, C.c_int32, c_f32p, C.c_void_p]),
     "bnn_sample_instability": (

@@ -11,13 +11,15 @@
 
 namespace bnn {
 
+// halted_at (may be null): a seed with halted_at[s] >= 0 (bnn_train_step_seeds_halt) is left untouched, here and in
+// swag_bump_kernel.
 __global__ void swag_collect_kernel(const float* __restrict__ w, int64_t d, int K, float* __restrict__ w_avg,
                                     float* __restrict__ w2_avg, float* __restrict__ pre_D,
                                     const int32_t* __restrict__ n_models, const int32_t* __restrict__ n_cols,
-                                    int current_epoch, int c) {
+                                    int current_epoch, int c, const int64_t* __restrict__ halted_at) {
     const int s = blockIdx.y;
     const int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (j >= d) return;
+    if (j >= d || (halted_at && halted_at[s] >= 0)) return;
     const int n = n_models[s];
     const int nc = n_cols[s];
     const int64_t o = (int64_t)s * d + j;
@@ -43,12 +45,34 @@ __global__ void swag_collect_kernel(const float* __restrict__ w, int64_t d, int 
     }
 }
 
-__global__ void swag_bump_kernel(int32_t* n_models, int32_t* n_cols, int n_seeds, int K, int current_epoch, int c) {
+__global__ void swag_bump_kernel(int32_t* n_models, int32_t* n_cols, int n_seeds, int K, int current_epoch, int c,
+                                 const int64_t* __restrict__ halted_at) {
     const int s = threadIdx.x + blockIdx.x * blockDim.x;
-    if (s >= n_seeds) return;
+    if (s >= n_seeds || (halted_at && halted_at[s] >= 0)) return;
     const int nc = n_cols[s];
     if ((nc == 0) || (current_epoch % c == 0)) n_cols[s] = min(nc + 1, K);
     n_models[s] += 1;
+}
+
+// bnn_swag_collect (halted_at null) and bnn_swag_collect_halt; every argument check runs before the device is touched
+static int swag_collect(const char* who, const float* d_w, int64_t d, int32_t n_seeds, int32_t K, float* d_w_avg,
+                        float* d_w2_avg, float* d_pre_D, int32_t* d_n_models, int32_t* d_n_cols, int32_t current_epoch,
+                        int32_t c, bool halt, const int64_t* d_halted_at, cudaStream_t st) {
+    BNN_REQUIRE(d_w && d_w_avg && d_w2_avg && d_pre_D && d_n_models && d_n_cols && (!halt || d_halted_at), BNN_E_ARG,
+                "%s: null pointer", who);
+    BNN_REQUIRE(d > 0 && n_seeds > 0 && n_seeds < 65536 && K >= 1 && c >= 1, BNN_E_ARG,
+                "%s: bad sizes (d=%lld seeds=%d K=%d c=%d)", who, (long long)d, n_seeds, K, c);
+    BNN_REQUIRE(((uintptr_t)d_halted_at & 7u) == 0, BNN_E_ALIGN, "%s: d_halted_at must be 8-byte aligned", who);
+    int rc = check_device();
+    if (rc != BNN_OK) return rc;
+    const int threads = 256;
+    dim3 grid((unsigned)((d + threads - 1) / threads), (unsigned)n_seeds);
+    swag_collect_kernel<<<grid, threads, 0, st>>>(d_w, d, K, d_w_avg, d_w2_avg, d_pre_D, d_n_models, d_n_cols,
+                                                  current_epoch, c, d_halted_at);
+    BNN_CUDA(cudaGetLastError());
+    swag_bump_kernel<<<(n_seeds + 127) / 128, 128, 0, st>>>(d_n_models, d_n_cols, n_seeds, K, current_epoch, c, d_halted_at);
+    BNN_CUDA(cudaGetLastError());
+    return BNN_OK;
 }
 
 }  // namespace bnn
@@ -56,22 +80,15 @@ __global__ void swag_bump_kernel(int32_t* n_models, int32_t* n_cols, int n_seeds
 extern "C" int bnn_swag_collect(const float* d_w, int64_t d, int32_t n_seeds, int32_t K, float* d_w_avg,
                                 float* d_w2_avg, float* d_pre_D, int32_t* d_n_models, int32_t* d_n_cols,
                                 int32_t current_epoch, int32_t c, void* stream) {
-    using namespace bnn;
-    int rc = check_device();
-    if (rc != BNN_OK) return rc;
-    BNN_REQUIRE(d_w && d_w_avg && d_w2_avg && d_pre_D && d_n_models && d_n_cols, BNN_E_ARG,
-                "bnn_swag_collect: null pointer");
-    BNN_REQUIRE(d > 0 && n_seeds > 0 && n_seeds < 65536 && K >= 1 && c >= 1, BNN_E_ARG,
-                "bnn_swag_collect: bad sizes (d=%lld seeds=%d K=%d c=%d)", (long long)d, n_seeds, K, c);
-    cudaStream_t st = (cudaStream_t)stream;
-    const int threads = 256;
-    dim3 grid((unsigned)((d + threads - 1) / threads), (unsigned)n_seeds);
-    swag_collect_kernel<<<grid, threads, 0, st>>>(d_w, d, K, d_w_avg, d_w2_avg, d_pre_D, d_n_models, d_n_cols,
-                                                  current_epoch, c);
-    BNN_CUDA(cudaGetLastError());
-    swag_bump_kernel<<<(n_seeds + 127) / 128, 128, 0, st>>>(d_n_models, d_n_cols, n_seeds, K, current_epoch, c);
-    BNN_CUDA(cudaGetLastError());
-    return BNN_OK;
+    return bnn::swag_collect("bnn_swag_collect", d_w, d, n_seeds, K, d_w_avg, d_w2_avg, d_pre_D, d_n_models, d_n_cols,
+                             current_epoch, c, false, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int bnn_swag_collect_halt(const float* d_w, int64_t d, int32_t n_seeds, int32_t K, float* d_w_avg,
+                                     float* d_w2_avg, float* d_pre_D, int32_t* d_n_models, int32_t* d_n_cols,
+                                     int32_t current_epoch, int32_t c, const int64_t* d_halted_at, void* stream) {
+    return bnn::swag_collect("bnn_swag_collect_halt", d_w, d, n_seeds, K, d_w_avg, d_w2_avg, d_pre_D, d_n_models,
+                             d_n_cols, current_epoch, c, true, d_halted_at, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------------------

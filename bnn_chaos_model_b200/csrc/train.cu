@@ -114,9 +114,16 @@ __global__ void __launch_bounds__(256) train_reduce_kernel(const float* __restri
 // Prologue of both update kernels: clip_grad_norm_ over seed s's whole gradient (coef = clip / (norm + 1e-6), applied
 // when < 1), grad_out and the metric slots known from the gradient.  Returns the factor the gradient is scaled by
 // (min(1, coef)) and this thread's gradient element in gi (0 past d).
+// Per-seed halt (halted_at non-null, the _halt entries): skip is set when seed s is already halted (halted_at[s] >= 0)
+// or this step is bad -- nll + skl + norm not finite, the condition of metrics column 6 -- and the thread that writes the
+// metrics (the last block's last thread, also when metrics is null) latches halted_at[s] = step when the seed was live.  Every thread of the seed computes the same norm and reads
+// the same two metric slots, so it reaches the same decision whichever block runs first: a block that still reads -1
+// sees the bad step itself, one that reads the latched word sees a halted seed, and both mean skip.  So the latch needs
+// no second kernel and no ordering between blocks.  With halted_at null, skip is false and nothing else changes.
 __device__ __forceinline__ float clip_prologue(const float* __restrict__ grad, const float* __restrict__ sq, int n_blocks,
                                                int d, int B, int s, const SeedHp& hp, float* __restrict__ grad_out,
-                                               float* __restrict__ metrics, float& gi) {
+                                               float* __restrict__ metrics, int64_t* halted_at, int64_t step,
+                                               float& gi, bool& skip) {
     const int i = blockIdx.x * 256 + threadIdx.x;
     float ss = 0.f;
     for (int b = 0; b < n_blocks; ++b) ss += sq[s * n_blocks + b];
@@ -126,16 +133,27 @@ __device__ __forceinline__ float clip_prologue(const float* __restrict__ grad, c
     const float* g = grad + (int64_t)s * (d + DPAD);
     gi = i < d ? g[i] : 0.f;
     if (grad_out && i < d) grad_out[(int64_t)s * d + i] = gi;
-    if (metrics && blockIdx.x == gridDim.x - 1 && threadIdx.x == 255) {
-        float* m = metrics + s * 8;
+    const bool last = blockIdx.x == gridDim.x - 1 && threadIdx.x == 255;
+    skip = false;
+    if ((metrics && last) || halted_at) {
         const float nll = g[d + SLOT_NLL], skl = g[d + SLOT_SKL] * hp.beta_out;
-        m[0] = nll / (float)B;
-        m[3] = skl / (float)B;
-        m[4] = norm;
-        m[5] = clip;
-        m[6] = isfinite(nll + skl + norm) ? 0.f : 1.f;
-        m[7] = 0.f;
-        // m[1] (loss with reg) and m[2] (input_kl) are completed by train_metrics_kernel, which reads lv_in before the update
+        const bool bad = !isfinite(nll + skl + norm);
+        if (metrics && last) {
+            float* m = metrics + s * 8;
+            m[0] = nll / (float)B;
+            m[3] = skl / (float)B;
+            m[4] = norm;
+            m[5] = clip;
+            m[6] = bad ? 1.f : 0.f;
+            m[7] = 0.f;
+            // m[1] (loss with reg) and m[2] (input_kl) are completed by train_metrics_kernel, which reads lv_in before the
+            // update
+        }
+        if (halted_at) {
+            const bool was = halted_at[s] >= 0;
+            skip = was || bad;
+            if (last && bad && !was) halted_at[s] = step;
+        }
     }
     return clip;
 }
@@ -145,12 +163,13 @@ __global__ void __launch_bounds__(256) train_update_kernel(const float* __restri
                                                            int n_blocks, int d, int B, int s0, const SeedChunk hps,
                                                            int first_step, int apply_update, float* __restrict__ theta,
                                                            float* __restrict__ mom, float* __restrict__ grad_out,
-                                                           float* __restrict__ metrics) {
+                                                           float* __restrict__ metrics, int64_t* halted_at, int64_t step) {
     const int s = s0 + (int)blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
     const SeedHp& hp = hps.s[blockIdx.y];
     float gi;
-    const float clip = clip_prologue(grad, sq, n_blocks, d, B, s, hp, grad_out, metrics, gi);
-    if (i < d && apply_update) {
+    bool skip;
+    const float clip = clip_prologue(grad, sq, n_blocks, d, B, s, hp, grad_out, metrics, halted_at, step, gi, skip);
+    if (i < d && apply_update && !skip) {
         const int64_t o = (int64_t)s * d + i;
         const float th = theta[o];
         float dp = gi * clip;   // clip == 1 when not clipping: exact
@@ -171,8 +190,8 @@ struct AdamStep {
     int first;         // t == 1: both buffers are zero and are not read (a fresh optimizer; no memset needed)
 };
 struct AdamChunk { AdamStep a[SEED_CHUNK]; };
-// the Adam update kernel's parameters: both chunks, 7 pointers and 5 ints, within the 4 KB every launch may carry
-static_assert(sizeof(SeedChunk) + sizeof(AdamChunk) + 7 * 8 + 5 * 4 <= 4096, "SEED_CHUNK too large for the kernel parameters");
+// the Adam update kernel's parameters: both chunks, 8 pointers, 5 ints and the step, within the 4 KB every launch may carry
+static_assert(sizeof(SeedChunk) + sizeof(AdamChunk) + 8 * 8 + 5 * 4 + 8 <= 4096, "SEED_CHUNK too large for the kernel parameters");
 
 // clip_grad_norm_ + torch.optim.Adam (amsgrad=False, maximize=False; weight decay is L2 added to the gradient, not AdamW):
 //   g += wd theta;  m = lerp(m, g, 1 - beta1);  v = beta2 v + (1 - beta2) g^2;  theta -= step_size m / (sqrt(v) / bc2_sqrt + eps)
@@ -181,13 +200,14 @@ __global__ void __launch_bounds__(256) train_adam_update_kernel(const float* __r
                                                                 const AdamChunk as, int apply_update,
                                                                 float* __restrict__ theta, float* __restrict__ exp_avg,
                                                                 float* __restrict__ exp_avg_sq, float* __restrict__ grad_out,
-                                                                float* __restrict__ metrics) {
+                                                                float* __restrict__ metrics, int64_t* halted_at, int64_t step) {
     const int s = s0 + (int)blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
     const SeedHp& hp = hps.s[blockIdx.y];
     const AdamStep& a = as.a[blockIdx.y];
     float gi;
-    const float clip = clip_prologue(grad, sq, n_blocks, d, B, s, hp, grad_out, metrics, gi);
-    if (i < d && apply_update) {
+    bool skip;
+    const float clip = clip_prologue(grad, sq, n_blocks, d, B, s, hp, grad_out, metrics, halted_at, step, gi, skip);
+    if (i < d && apply_update && !skip) {
         const int64_t o = (int64_t)s * d + i;
         const float th = theta[o];
         float g = gi * clip;
@@ -399,10 +419,11 @@ static AdamStep adam_step(const bnn_train_hparams& hp, const bnn_adam_hparams& a
 // d_state0 / d_state1: the momentum buffer (SGD) or exp_avg / exp_avg_sq (Adam), required when apply_update.
 // plan_seeds > 0: the seed groups and CTAs per seed are pick_plan's for plan_seeds seeds, whatever n_seeds is (0: for
 // n_seeds); a seed's bits depend on its CTA count, so a fixed plan_seeds makes them independent of how many seeds share
-// the call.
+// the call.  halt: the _halt entries, whose d_halted_at [n_seeds] (int64, 8-byte aligned) is required; the other entries
+// pass null and the update kernels then compute what they did before the halt word existed.
 static int train_step(const char* who, const bnn_model_config* cfg, const bnn_train_hparams* hp,
                       const bnn_adam_hparams* adam, bool is_adam, int hp_stride, int32_t n_seeds, int32_t plan_seeds,
-                      float* d_theta,
+                      bool halt, int64_t* d_halted_at, float* d_theta,
                       float* d_state0, float* d_state1, const float* d_x, const float* d_y, const int32_t* d_batch_index,
                       int64_t B, const float* d_eps_in, const float* d_eps12, const float* d_eps_sum, uint64_t seed,
                       uint64_t step, float* d_grad_out, float* d_metrics, void* d_workspace, cudaStream_t st) {
@@ -410,6 +431,12 @@ static int train_step(const char* who, const bnn_model_config* cfg, const bnn_tr
     BNN_REQUIRE(n_seeds >= 1 && n_seeds <= 65535 && B >= 1 && B < (1ll << 30), BNN_E_ARG,
                 "%s: n_seeds=%d B=%lld out of range", who, n_seeds, (long long)B);
     BNN_REQUIRE(plan_seeds >= 0 && plan_seeds <= 65535, BNN_E_ARG, "%s: plan_seeds=%d (0, or 1..65535)", who, plan_seeds);
+    if (halt) {
+        BNN_REQUIRE(d_halted_at, BNN_E_ARG, "%s: null d_halted_at", who);
+        BNN_REQUIRE(step < (1ull << 63), BNN_E_ARG, "%s: step %llu does not fit the int64 halt word", who,
+                    (unsigned long long)step);
+        BNN_REQUIRE(((uintptr_t)d_halted_at & 7u) == 0, BNN_E_ALIGN, "%s: d_halted_at must be 8-byte aligned", who);
+    }
     for (int s = 0; s < n_seeds; ++s) {
         const bnn_train_hparams& h = hp[(size_t)s * hp_stride];
         char at[32] = "";
@@ -501,10 +528,12 @@ static int train_step(const char* who, const bnn_model_config* cfg, const bnn_tr
             AdamChunk ac{};
             for (int j = 0; j < n; ++j) ac.a[j] = adam_step(hp[(size_t)(s0 + j) * hp_stride], adam[(size_t)(s0 + j) * hp_stride]);
             train_adam_update_kernel<<<dim3(nb, n), 256, 0, st>>>(grad, sq, nb, fl.d, (int)B, s0, hc, ac, apply_update,
-                                                                  d_theta, d_state0, d_state1, d_grad_out, d_metrics);
+                                                                  d_theta, d_state0, d_state1, d_grad_out, d_metrics,
+                                                                  d_halted_at, (int64_t)step);
         } else {
             train_update_kernel<<<dim3(nb, n), 256, 0, st>>>(grad, sq, nb, fl.d, (int)B, s0, hc, first_step, apply_update,
-                                                             d_theta, d_state0, d_grad_out, d_metrics);
+                                                             d_theta, d_state0, d_grad_out, d_metrics, d_halted_at,
+                                                             (int64_t)step);
         }
         BNN_CUDA(cudaGetLastError());
     }
@@ -662,7 +691,8 @@ int bnn_train_step(const bnn_model_config* cfg, const bnn_train_hparams* hp, int
                    float* d_momentum, const float* d_x, const float* d_y, const int32_t* d_batch_index, int64_t B,
                    const float* d_eps_in, const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
                    float* d_grad_out, float* d_metrics, void* d_workspace, void* stream) {
-    return bnn::train::train_step("bnn_train_step", cfg, hp, nullptr, false, 0, n_seeds, 0, d_theta, d_momentum, nullptr, d_x,
+    return bnn::train::train_step("bnn_train_step", cfg, hp, nullptr, false, 0, n_seeds, 0, false, nullptr, d_theta,
+                                  d_momentum, nullptr, d_x,
                                   d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step, d_grad_out, d_metrics,
                                   d_workspace, (cudaStream_t)stream);
 }
@@ -671,7 +701,8 @@ int bnn_train_step_seeds(const bnn_model_config* cfg, const bnn_train_hparams* h
                          float* d_theta, float* d_momentum, const float* d_x, const float* d_y, const int32_t* d_batch_index, int64_t B,
                          const float* d_eps_in, const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
                          float* d_grad_out, float* d_metrics, void* d_workspace, void* stream) {
-    return bnn::train::train_step("bnn_train_step_seeds", cfg, hp, nullptr, false, 1, n_seeds, plan_seeds, d_theta, d_momentum, nullptr,
+    return bnn::train::train_step("bnn_train_step_seeds", cfg, hp, nullptr, false, 1, n_seeds, plan_seeds, false, nullptr,
+                                  d_theta, d_momentum, nullptr,
                                   d_x, d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step, d_grad_out,
                                   d_metrics, d_workspace, (cudaStream_t)stream);
 }
@@ -681,7 +712,8 @@ int bnn_train_step_adam(const bnn_model_config* cfg, const bnn_train_hparams* hp
                         const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
                         const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_grad_out,
                         float* d_metrics, void* d_workspace, void* stream) {
-    return bnn::train::train_step("bnn_train_step_adam", cfg, hp, adam, true, 0, n_seeds, 0, d_theta, d_exp_avg, d_exp_avg_sq,
+    return bnn::train::train_step("bnn_train_step_adam", cfg, hp, adam, true, 0, n_seeds, 0, false, nullptr, d_theta,
+                                  d_exp_avg, d_exp_avg_sq,
                                   d_x, d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step, d_grad_out,
                                   d_metrics, d_workspace, (cudaStream_t)stream);
 }
@@ -691,9 +723,31 @@ int bnn_train_step_adam_seeds(const bnn_model_config* cfg, const bnn_train_hpara
                               const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
                               const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_grad_out,
                               float* d_metrics, void* d_workspace, void* stream) {
-    return bnn::train::train_step("bnn_train_step_adam_seeds", cfg, hp, adam, true, 1, n_seeds, plan_seeds, d_theta, d_exp_avg,
+    return bnn::train::train_step("bnn_train_step_adam_seeds", cfg, hp, adam, true, 1, n_seeds, plan_seeds, false, nullptr,
+                                  d_theta, d_exp_avg,
                                   d_exp_avg_sq, d_x, d_y, d_batch_index, B, d_eps_in, d_eps12, d_eps_sum, seed, step,
                                   d_grad_out, d_metrics, d_workspace, (cudaStream_t)stream);
+}
+
+int bnn_train_step_seeds_halt(const bnn_model_config* cfg, const bnn_train_hparams* hp, int32_t n_seeds, int32_t plan_seeds,
+                              float* d_theta, float* d_momentum, const float* d_x, const float* d_y,
+                              const int32_t* d_batch_index, int64_t B, const float* d_eps_in, const float* d_eps12,
+                              const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_grad_out, float* d_metrics,
+                              void* d_workspace, int64_t* d_halted_at, void* stream) {
+    return bnn::train::train_step("bnn_train_step_seeds_halt", cfg, hp, nullptr, false, 1, n_seeds, plan_seeds, true,
+                                  d_halted_at, d_theta, d_momentum, nullptr, d_x, d_y, d_batch_index, B, d_eps_in, d_eps12,
+                                  d_eps_sum, seed, step, d_grad_out, d_metrics, d_workspace, (cudaStream_t)stream);
+}
+
+int bnn_train_step_adam_seeds_halt(const bnn_model_config* cfg, const bnn_train_hparams* hp, const bnn_adam_hparams* adam,
+                                   int32_t n_seeds, int32_t plan_seeds, float* d_theta, float* d_exp_avg,
+                                   float* d_exp_avg_sq, const float* d_x, const float* d_y, const int32_t* d_batch_index,
+                                   int64_t B, const float* d_eps_in, const float* d_eps12, const float* d_eps_sum,
+                                   uint64_t seed, uint64_t step, float* d_grad_out, float* d_metrics, void* d_workspace,
+                                   int64_t* d_halted_at, void* stream) {
+    return bnn::train::train_step("bnn_train_step_adam_seeds_halt", cfg, hp, adam, true, 1, n_seeds, plan_seeds, true,
+                                  d_halted_at, d_theta, d_exp_avg, d_exp_avg_sq, d_x, d_y, d_batch_index, B, d_eps_in,
+                                  d_eps12, d_eps_sum, seed, step, d_grad_out, d_metrics, d_workspace, (cudaStream_t)stream);
 }
 
 int bnn_saliency(const bnn_model_config* cfg, int32_t n_models, const float* d_theta, const float* d_x, int64_t B,

@@ -15,10 +15,16 @@ The reference reads its training set from data files that are not in the reposit
 come from ``--data file.npz`` (X_train, y_train, X_val, y_val, already normalised like get_data does) or, by default,
 from the synthetic generator.  Start weights: ``--init DIR`` with one ``*_<seed>.pt`` flat weight vector per seed (the
 output of the pre-training phase, ``MultiSeedPretrainer.export``), else the seed's own random initialisation.
+
+``--on_nan halt`` lets a diverging seed stop alone (``MultiSeedSWAGTrainer(on_nan="halt")``) instead of ending the whole
+job with ValueError (the default, ``raise``): the files above are written for the seeds that completed only -- the
+reference's driver exits without output for a run that hit terminate_on_nan -- and ``OUT/halted.json`` lists every seed's
+name and ``halted_at_step`` (null = completed).
 """
 from __future__ import annotations
 
 import argparse
+import json
 import os
 import pickle
 from typing import List, Optional, Sequence
@@ -121,6 +127,30 @@ def write_outputs(stats: dict, models_hparams: Sequence[dict], swa_params: dict,
     return paths
 
 
+# the halt step travels as one float column of the gathered statistics: fp32 holds every integer below 2^24 exactly
+MAX_GATHERED_STEP = 1 << 24
+
+
+def halted_column(trainer: MultiSeedSWAGTrainer) -> torch.Tensor:
+    """``trainer.halted_at`` as an [S, 1] float column for ``gather_seed_statistics``'s ``extra``."""
+    assert max(trainer.halted_at) < MAX_GATHERED_STEP, "a halt step past 2^24 would not survive the fp32 gather"
+    return torch.tensor(trainer.halted_at, dtype=torch.float32, device=trainer.theta.device)[:, None]
+
+
+def halted_steps(column) -> List[Optional[int]]:
+    """The gathered halt column as per-seed steps, None for a seed that completed."""
+    return [None if v < 0 else int(v) for v in column.tolist()]
+
+
+def write_halted(out_dir: str, names: Sequence[str], steps: Sequence[Optional[int]]) -> str:
+    """OUT/halted.json: per seed its checkpoint name and halted_at_step (null = completed)."""
+    os.makedirs(out_dir, exist_ok=True)
+    path = os.path.join(out_dir, "halted.json")
+    with open(path, "w") as f:
+        json.dump({"seeds": [{"name": n, "halted_at_step": h} for n, h in zip(names, steps)]}, f, indent=1)
+    return path
+
+
 def run(args, X_train, y_train, X_val, y_val, out_dir: Optional[str] = None, group=None):
     """Train this rank's seeds, gather, write (rank 0).  Returns (paths or None, trainer, logs)."""
     import torch.distributed as dist
@@ -140,14 +170,30 @@ def run(args, X_train, y_train, X_val, y_val, out_dir: Optional[str] = None, gro
             m.load(torch.load(os.path.join(args.init, checkpoint_filename(args, s) + ".pt"), map_location=dev, weights_only=True))
         models.append(m)
     trainer = MultiSeedSWAGTrainer(models, X_train, y_train, X_val, y_val, batch_size=args.batch_size, device=dev,
-                                   seed=args.noise_seed + 1000003 * rank, swa_start=swa["swa_start"], optimizer=args.optimizer)
+                                   seed=args.noise_seed + 1000003 * rank, swa_start=swa["swa_start"], optimizer=args.optimizer,
+                                   on_nan=args.on_nan)
     logs = trainer.fit(epochs, validate=X_val is not None)
-    stats = gather_seed_statistics(trainer, args.n_seeds, group)
+    halt = args.on_nan == "halt"
+    stats = gather_seed_statistics(trainer, args.n_seeds, group, extra=halted_column(trainer) if halt else None)
     paths = None
     if rank == 0 and out_dir:
-        names = [checkpoint_filename(args, s) for s in range(args.n_seeds)]
-        paths = write_outputs(stats, all_hp, swa, names, out_dir, trainer.global_step, trainer.current_epoch)
+        paths = write_run(args, stats, all_hp, swa, out_dir, trainer.global_step, trainer.current_epoch)
     return paths, trainer, logs
+
+
+def write_run(args, stats: dict, all_hp: Sequence[dict], swa: dict, out_dir: str, global_step: int,
+              current_epoch: int) -> List[str]:
+    """Rank 0's files: every seed's outputs, or with --on_nan halt (the halt column in stats["extra"]) the completed
+    seeds' outputs and OUT/halted.json."""
+    names = [checkpoint_filename(args, s) for s in range(args.n_seeds)]
+    if args.on_nan == "halt":
+        steps = halted_steps(stats["extra"][:, 0])
+        write_halted(out_dir, names, steps)
+        done = [s for s in range(args.n_seeds) if steps[s] is None]
+        keep = torch.tensor(done, dtype=torch.long, device=stats["theta"].device)
+        stats = {k: v[keep] for k, v in stats.items() if k != "extra"}
+        all_hp, names = [all_hp[s] for s in done], [names[s] for s in done]
+    return write_outputs(stats, all_hp, swa, names, out_dir, global_step, current_epoch)
 
 
 def build_parser():
@@ -163,6 +209,9 @@ def build_parser():
     ap.add_argument("--noise_seed", type=int, default=0)
     ap.add_argument("--optimizer", choices=("sgd", "adam"), default="sgd",
                     help="sgd: the reference's SGD with momentum; adam: torch.optim.Adam (betas 0.9, 0.999, eps 1e-8)")
+    ap.add_argument("--on_nan", choices=("raise", "halt"), default="raise",
+                    help="raise: a non-finite training step ends the job (ValueError); halt: that seed stops alone and "
+                         "only the completed seeds are written (OUT/halted.json lists which halted, and at which step)")
     ap.add_argument("--data", default=None, help="npz with X_train, y_train, X_val, y_val (normalised)")
     ap.add_argument("--synthetic", type=int, nargs=2, default=(8000, 1000), metavar=("N_TRAIN", "N_VAL"))
     ap.add_argument("--init", default=None, help="directory of <checkpoint_filename>.pt flat weight vectors")

@@ -49,6 +49,20 @@ def check_shared(models, key: str, get):
     return vals[0]
 
 
+ON_NAN = ("raise", "halt")
+
+
+def halted_nan(x: torch.Tensor, halted: torch.Tensor) -> torch.Tensor:
+    """x [S] with NaN for every seed whose halt word (``halted`` [S] int64, -1 = live) is set."""
+    return torch.where(halted >= 0, torch.full_like(x, float("nan")), x)
+
+
+def best_epoch_weights(theta: torch.Tensor, best_val: torch.Tensor, best_theta: torch.Tensor) -> torch.Tensor:
+    """Per seed: the best epoch's weights where the seed has a finite best validation loss, else its current weights
+    (a seed that halted before any finite validation keeps what it has)."""
+    return torch.where(torch.isfinite(best_val)[:, None], best_theta, theta)
+
+
 def check_optimizer(optimizer: str, betas, eps):
     """The optimizer name and torch.optim.Adam's checks of betas / eps, as ValueError.  Returns (beta1, beta2, eps)."""
     if optimizer not in ("sgd", "adam"):
@@ -89,13 +103,25 @@ class MultiSeedSWAGTrainer:
     numbers on whichever rank it lands.  Default: keyed on the local index with one shuffle generator, as before.
     ``plan_seeds`` -- plan the fused step's seed groups and CTAs per seed for that many seeds rather than for this
     trainer's count (``bnn_train_step_seeds``): a seed's bits depend on its CTA count, so with ``first_run`` and a fixed
-    ``plan_seeds`` a run trains to the same bits however the runs are split over ranks."""
+    ``plan_seeds`` a run trains to the same bits however the runs are split over ranks.
+
+    ``on_nan`` -- what a non-finite training step does.  "raise" (default): ValueError at the end of the epoch in which
+    any seed's metrics flag a non-finite step (terminate_on_nan, run_swag.py:78), which ends every seed of the job.
+    "halt": each seed stops alone, on the device, at its first bad step (``bnn_train_step_seeds_halt``): that step and
+    every later one leave its weights and optimizer state untouched, and ``collect`` skips it from then on
+    (``bnn_swag_collect_halt``).  The other seeds train to the same bits as without the halted one.  The device word is
+    read once per epoch, where "raise" reads the flag; ``halted_at`` holds it per seed (-1 = completed, else the global
+    step that halted the seed), and the log entries carry NaN validation losses for a seed from the epoch it halted in.
+    A halted seed still runs its forward / backward: the launch's time is set by the seeds that share it."""
 
     def __init__(self, models: Sequence[SWAGModel], X_train, y_train, X_val=None, y_val=None, batch_size=2000,
                  device=None, seed=0, swa_start: Optional[int] = None, noisy_val: Optional[bool] = None,
                  lr_milestone: bool = True, optimizer: str = "sgd", betas=(0.9, 0.999), eps: float = 1e-8,
-                 first_run: Optional[int] = None, plan_seeds: Optional[int] = None):
+                 first_run: Optional[int] = None, plan_seeds: Optional[int] = None, on_nan: str = "raise"):
         beta1, beta2, eps = check_optimizer(optimizer, betas, eps)   # before anything touches a device
+        if on_nan not in ON_NAN:
+            raise ValueError(f"on_nan must be 'raise' or 'halt', got {on_nan!r}")
+        self.on_nan = on_nan
         if plan_seeds is not None and not 1 <= int(plan_seeds) <= 65535:
             raise ValueError(f"plan_seeds must be in [1, 65535], got {plan_seeds}")
         self.plan_seeds = 0 if plan_seeds is None else int(plan_seeds)
@@ -144,6 +170,8 @@ class MultiSeedSWAGTrainer:
         self.n_models = torch.zeros(self.S, dtype=torch.int32, device=dev)
         self.n_cols = torch.zeros(self.S, dtype=torch.int32, device=dev)
         self.metrics = torch.zeros((self.S, 8), device=dev)
+        self._halted = torch.full((self.S,), -1, dtype=torch.int64, device=dev) if on_nan == "halt" else None
+        self.halted_at = [-1] * self.S
         self.global_step = 0
         self.current_epoch = 0
         self.first_step = True
@@ -182,17 +210,20 @@ class MultiSeedSWAGTrainer:
                 self._ws = torch.empty((nbytes + 3) // 4, device=self.device, dtype=torch.float32)
             seed = self.seed if self.first_run is None else run_key(self.seed, self.first_run)
             rest = (_lib.ptr(self.X), _lib.ptr(self.y), _lib.ptr(batch_index), B, None, None, None, seed, self.global_step,
-                    None, _lib.ptr(self.metrics), _lib.ptr(self._ws), _lib.current_stream_ptr())
+                    None, _lib.ptr(self.metrics), _lib.ptr(self._ws))
+            halt = self._halted is not None
+            rest += (_lib.ptr(self._halted), _lib.current_stream_ptr()) if halt else (_lib.current_stream_ptr(),)
             if self.optimizer == "adam":
                 adam = (AdamHParams * self.S)(*(AdamHParams(beta1=h["beta1"], beta2=self.betas[1], eps=self.eps,
                                                             step=self.adam_step + 1) for h in per_seed))
-                _lib.check(lib.bnn_train_step_adam_seeds(cfg, hp, adam, self.S, self.plan_seeds, _lib.ptr(self.theta),
-                                                         _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq), *rest),
-                           "bnn_train_step_adam_seeds")
+                name = "bnn_train_step_adam_seeds_halt" if halt else "bnn_train_step_adam_seeds"
+                _lib.check(getattr(lib, name)(cfg, hp, adam, self.S, self.plan_seeds, _lib.ptr(self.theta),
+                                              _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq), *rest), name)
                 self.adam_step += 1
             else:
-                _lib.check(lib.bnn_train_step_seeds(cfg, hp, self.S, self.plan_seeds, _lib.ptr(self.theta),
-                                                    _lib.ptr(self.momentum), *rest), "bnn_train_step_seeds")
+                name = "bnn_train_step_seeds_halt" if halt else "bnn_train_step_seeds"
+                _lib.check(getattr(lib, name)(cfg, hp, self.S, self.plan_seeds, _lib.ptr(self.theta),
+                                              _lib.ptr(self.momentum), *rest), name)
         self.first_step = False
         self.global_step += 1
 
@@ -244,8 +275,12 @@ class MultiSeedSWAGTrainer:
         noisy_val=False: K2 + the per-unit NLL sum (bnn_eval_loss; eps1, eps2 from Philox).  noisy_val=True: the
         training kernel's noisy forward without update (bnn_train_step, apply_update=0: input noise, eps1, eps2 and
         summary noise from Philox keyed on (seed ^ 0x5EED; unit, system, epoch)); metrics[:, 0] * B is the summed loss.
-        With ``first_run``, each seed's weight sets are a call of their own under the run's key."""
-        have_avg = bool((self.n_models > 0).all())
+        With ``first_run``, each seed's weight sets are a call of their own under the run's key.  A halted seed does not
+        hold back the others' w_avg losses when it halted before its first collection."""
+        collected = self.n_models > 0
+        if self._halted is not None:
+            collected |= self._halted >= 0
+        have_avg = bool(collected.all())
         thetas = torch.cat([self.theta, self.w_avg]) if have_avg else self.theta
         if self.first_run is None:
             loss = self._unit_losses(thetas.contiguous(), self.seed ^ 0x5EED)
@@ -293,12 +328,24 @@ class MultiSeedSWAGTrainer:
         lib = _lib.load()
         d = self.theta.shape[1]
         with torch.cuda.device(self.device), _lib.nvtx("bnn:K5 swag_collect"):
-            _lib.check(
-                lib.bnn_swag_collect(_lib.ptr(self.theta), d, self.S, self.K, _lib.ptr(self.w_avg), _lib.ptr(self.w2_avg),
-                                     _lib.ptr(self.pre_D), _lib.ptr(self.n_models), _lib.ptr(self.n_cols),
-                                     int(self.current_epoch), int(self.c), _lib.current_stream_ptr()),
-                "bnn_swag_collect",
-            )
+            args = (_lib.ptr(self.theta), d, self.S, self.K, _lib.ptr(self.w_avg), _lib.ptr(self.w2_avg),
+                    _lib.ptr(self.pre_D), _lib.ptr(self.n_models), _lib.ptr(self.n_cols), int(self.current_epoch), int(self.c))
+            if self._halted is None:
+                _lib.check(lib.bnn_swag_collect(*args, _lib.current_stream_ptr()), "bnn_swag_collect")
+            else:
+                _lib.check(lib.bnn_swag_collect_halt(*args, _lib.ptr(self._halted), _lib.current_stream_ptr()),
+                           "bnn_swag_collect_halt")
+
+    def _check_nan(self, check_nan_every: int):
+        """End of an epoch: "halt" reads the halt words into ``halted_at``; "raise" raises on the non-finite flag."""
+        if self._halted is not None:
+            self.halted_at = self._halted.tolist()
+        elif check_nan_every and (self.current_epoch % check_nan_every == 0):
+            if bool((self.metrics[:, 6] != 0).any()):  # terminate_on_nan (run_swag.py:78), once per epoch
+                raise ValueError(f"non-finite training loss at epoch {self.current_epoch}")
+
+    def _halted_nan(self, x):
+        return x if self._halted is None else halted_nan(x, self._halted)
 
     def fit(self, epochs: int, validate: bool = True, check_nan_every: int = 1):
         """Trainer.fit (run_swag.py:74-82): epochs of training, validation, and collection after swa_start."""
@@ -308,12 +355,10 @@ class MultiSeedSWAGTrainer:
             entry = {"epoch": self.current_epoch, "global_step": self.global_step}
             if validate and self.Xv is not None:
                 v, s = self.validation_losses()
-                entry["val_loss_no_reg"], entry["swa_loss_no_reg"] = v.cpu(), s.cpu()
+                entry["val_loss_no_reg"], entry["swa_loss_no_reg"] = self._halted_nan(v).cpu(), self._halted_nan(s).cpu()
             if self.global_step > self.swa_start:  # :808
                 self.collect()
-            if check_nan_every and (self.current_epoch % check_nan_every == 0):
-                if bool((self.metrics[:, 6] != 0).any()):  # terminate_on_nan (run_swag.py:78), once per epoch
-                    raise ValueError(f"non-finite training loss at epoch {self.current_epoch}")
+            self._check_nan(check_nan_every)
             logs.append(entry)
             self.current_epoch += 1
         return logs
@@ -349,6 +394,12 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
     * the run ends when the scheduler is stepped past its total -- the reference's ValueError
       (:137-139, caught at find_minima.py:79-82) -- after which every seed is reset to its best checkpoint.
 
+    With ``on_nan="halt"`` a halted seed's best-epoch record stops updating in the epoch it halts (its validation loss
+    reads NaN from then on, so frozen weights cannot become "best" through validation noise), and at the schedule's end
+    each seed with a finite best is restored to it on its own -- the reference's ``except ValueError`` reloads the best
+    checkpoint after terminate_on_nan as after the schedule's end (find_minima.py:80-86).  With "raise" the restore is
+    all or nothing, as before.
+
     Each seed's one-cycle peak is its own model's ``lr`` and its KL weights anneal towards its own ``beta_in`` /
     ``beta_out``, with its own weight_decay; the cycled momentum (Adam's beta1) is the same for all.  Before, every
     seed trained with the first model's values.  ``steps``, ``batch_size`` (when not given here) and noisy_val (when not
@@ -357,7 +408,8 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
 
     def __init__(self, models: Sequence[VarModel], X_train, y_train, X_val=None, y_val=None, batch_size=None,
                  device=None, seed=0, noisy_val: Optional[bool] = None, optimizer: str = "sgd", betas=(0.9, 0.999),
-                 eps: float = 1e-8, first_run: Optional[int] = None, plan_seeds: Optional[int] = None):
+                 eps: float = 1e-8, first_run: Optional[int] = None, plan_seeds: Optional[int] = None,
+                 on_nan: str = "raise"):
         if len(models) == 0:
             raise ValueError("no seed models")
         m0 = models[0]
@@ -369,7 +421,7 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
                 m.K, m.c, m.swa_params = 1, 1, {"swa_lr": m.lr}
         super().__init__(models, X_train, y_train, X_val, y_val, batch_size=batch_size or m0.batch_size, device=device,
                          seed=seed, swa_start=1 << 62, noisy_val=noisy_val, lr_milestone=False, optimizer=optimizer,
-                         betas=betas, eps=eps, first_run=first_run, plan_seeds=plan_seeds)
+                         betas=betas, eps=eps, first_run=first_run, plan_seeds=plan_seeds, on_nan=on_nan)
         self.steps = int(m0.steps)
         self.max_lrs = [float(m.lr) for m in self.models]
         self.max_lr = self.max_lrs[0]
@@ -421,18 +473,22 @@ class MultiSeedPretrainer(MultiSeedSWAGTrainer):
                 self.finished = True
             entry = {"epoch": self.current_epoch, "global_step": self.global_step}
             if not self.finished and validate and self.Xv is not None:
-                v, _ = self.validation_losses()
-                better = v < self.best_val
+                v = self._halted_nan(self.validation_losses()[0])
+                better = v < self.best_val   # NaN (a halted seed) is never better
                 self.best_val = torch.where(better, v, self.best_val)
                 self.best_theta = torch.where(better[:, None], self.theta, self.best_theta)
                 entry["val_loss_no_reg"] = v.cpu()
-            if check_nan_every and bool((self.metrics[:, 6] != 0).any()):
+            if self._halted is not None:
+                self.halted_at = self._halted.tolist()
+            elif check_nan_every and bool((self.metrics[:, 6] != 0).any()):
                 raise ValueError(f"non-finite training loss at epoch {self.current_epoch}")
             logs.append(entry)
             self.current_epoch += 1
             if self.finished:
-                if self.Xv is not None and bool(torch.isfinite(self.best_val).all()):
-                    self.theta.copy_(self.best_theta)  # load_state_dict(best_model_path), find_minima.py:82
+                if self.Xv is not None and self._halted is not None:   # load_state_dict(best_model_path), find_minima.py:82
+                    self.theta.copy_(best_epoch_weights(self.theta, self.best_val, self.best_theta))
+                elif self.Xv is not None and bool(torch.isfinite(self.best_val).all()):
+                    self.theta.copy_(self.best_theta)
                 break
         return logs
 

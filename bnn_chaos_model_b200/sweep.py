@@ -27,6 +27,13 @@ config with the highest lpd (swag), else the lowest mean SWA (swag) or best-epoc
 validation set therefore picks both the pre-training checkpoints and the config: judge the chosen config on data it
 has not seen.
 
+``--on_nan halt`` (run_swag's flag; default ``raise``, where one diverging run ends the job) lets each run stop alone at
+its first non-finite step, which a sweep over learning rates is bound to meet.  Each config entry then gets
+``halted_at_step`` per seed (null = completed) and a halted seed's losses are null.  Pretrain writes a halted seed's
+``.pt`` when it had a finite best epoch, and nothing otherwise; swag writes and scores only a config's completed seeds
+(``lpd`` over their ensemble, null when none completed).  ``best`` only considers configs with a completed run (pretrain:
+one with a finite best) and is null when there is none.  With ``raise`` sweep.json has no ``halted_at_step``.
+
 Results do not depend on the number of ranks, bit for bit.  A run's noise, batch shuffles and validation draws are
 keyed on its global index j (``first_run``), so it draws the same numbers on whichever rank it lands; and every rank
 plans its fused step for ``--plan_seeds`` seeds (default 4) whatever number of runs it holds, so every run's gradient is
@@ -46,7 +53,7 @@ from typing import Dict, List, Sequence
 import torch
 
 from . import run_swag
-from .swag_train import MultiSeedPretrainer, MultiSeedSWAGTrainer, seeds_of_rank
+from .swag_train import MultiSeedPretrainer, MultiSeedSWAGTrainer, best_epoch_weights, seeds_of_rank
 
 GRID_KEYS = {
     "pretrain": ("lr", "weight_decay", "beta_in", "beta_out"),
@@ -125,17 +132,19 @@ def run(args, configs: Sequence[Dict[str, float]], X_train, y_train, X_val, y_va
                 m.load(torch.load(os.path.join(args.init, name), map_location=dev, weights_only=True))
         models.append(m)
     kw = dict(batch_size=args.batch_size, device=dev, seed=args.noise_seed, optimizer=args.optimizer, first_run=runs[0],
-              plan_seeds=args.plan_seeds)
+              plan_seeds=args.plan_seeds, on_nan=args.on_nan)
     if phase == "pretrain":
         trainer = MultiSeedPretrainer(models, X_train, y_train, X_val, y_val, **kw)
         trainer.fit(args.epochs or None)
         # the best epoch's weights also when --epochs ends the run before the schedule does (fit restores them only then)
-        trainer.theta.copy_(torch.where(torch.isfinite(trainer.best_val)[:, None], trainer.best_theta, trainer.theta))
+        trainer.theta.copy_(best_epoch_weights(trainer.theta, trainer.best_val, trainer.best_theta))
         extra = trainer.best_val[:, None]
     else:
         trainer = MultiSeedSWAGTrainer(models, X_train, y_train, X_val, y_val, swa_start=run_hp[0][1]["swa_start"], **kw)
         last = trainer.fit(epochs)[-1]
         extra = torch.stack([last["val_loss_no_reg"], last["swa_loss_no_reg"]], dim=1).to(dev)
+    if args.on_nan == "halt":   # the last extra column
+        extra = torch.cat([extra, run_swag.halted_column(trainer)], dim=1)
     stats = run_swag.gather_seed_statistics(trainer, n_runs, group, extra=extra.float())
     if rank != 0:
         return None
@@ -148,36 +157,54 @@ def write_sweep(args, configs, stats, run_hp, trainer, X_val, y_val, out_dir: st
     spc, phase = args.seeds_per_config, args.phase
     names = [run_swag.checkpoint_filename(args, s) for s in range(spc)]
     xv, yv = X_val.to(trainer.device).contiguous().float(), y_val.to(trainer.device).contiguous().float()
-    # sampling needs all K deviation columns; every run of the job collects on the same epochs, so all have them or none
-    scored = phase == "swag" and bool((stats["n_cols"] >= trainer.K).all())
+    halt = args.on_nan == "halt"
+    steps = run_swag.halted_steps(stats["extra"][:, -1]) if halt else [None] * stats["theta"].shape[0]
+    done = [j for j, h in enumerate(steps) if h is None]
+    # sampling needs all K deviation columns; every completed run of the job collects on the same epochs, so all have
+    # them or none
+    scored = phase == "swag" and bool(done) and bool((stats["n_cols"][done] >= trainer.K).all())
+
+    def losses(col, lo, hi):
+        return [None if steps[j] is not None else float(stats["extra"][j, col]) for j in range(lo, hi)]
+
     entries = []
     for k, ov in enumerate(configs):
         lo, hi = k * spc, (k + 1) * spc
         d = config_dir(out_dir, k)
-        e = {"config": k, "dir": os.path.basename(d), "overrides": ov,
-             "val_loss": [float(v) for v in stats["extra"][lo:hi, 0]]}
+        e = {"config": k, "dir": os.path.basename(d), "overrides": ov, "val_loss": losses(0, lo, hi)}
+        if halt:
+            e["halted_at_step"] = steps[lo:hi]
         if phase == "pretrain":
             os.makedirs(d, exist_ok=True)
-            for s in range(spc):
-                torch.save(stats["theta"][lo + s].cpu().clone(), os.path.join(d, names[s] + ".pt"))
+            for s in range(spc):   # a halted seed's best epoch, when it had a finite one
+                if steps[lo + s] is None or math.isfinite(float(stats["extra"][lo + s, 0])):
+                    torch.save(stats["theta"][lo + s].cpu().clone(), os.path.join(d, names[s] + ".pt"))
         else:
-            sub = {key: v[lo:hi] for key, v in stats.items()}
-            paths = run_swag.write_outputs(sub, [run_hp[j][0] for j in range(lo, hi)], run_hp[lo][1], names, d,
+            ok = [s for s in range(spc) if steps[lo + s] is None]
+            idx = torch.tensor([lo + s for s in ok], dtype=torch.long, device=stats["theta"].device)
+            sub = {key: v[idx] for key, v in stats.items()}
+            paths = run_swag.write_outputs(sub, [run_hp[lo + s][0] for s in ok], run_hp[lo][1], [names[s] for s in ok], d,
                                            trainer.global_step, trainer.current_epoch)
-            e["swa_val_loss"] = [float(v) for v in stats["extra"][lo:hi, 1]]
+            e["swa_val_loss"] = losses(1, lo, hi)
             e["lpd"] = e["mean_nll"] = None
-            if scored:
+            if scored and paths:
                 _, score = load_ensemble(paths, device=trainer.device).evaluate(xv, yv, args.eval_samples,
                                                                                 seed=args.noise_seed)
                 e["lpd"], e["mean_nll"] = float(score[:, 0].double().mean()), float(score[:, 1].double().mean())
         entries.append(e)
-    if scored:
-        best, best_by = max(range(len(entries)), key=lambda k: entries[k]["lpd"]), "lpd (highest)"
-    else:
+
+    def mean_loss(e):   # over the completed runs with a finite loss (pretrain: a finite best); None without one
         key = "val_loss" if phase == "pretrain" else "swa_val_loss"
-        best = min(range(len(entries)), key=lambda k: sum(entries[k][key]) / spc)
+        vals = [v for v in e[key] if v is not None and math.isfinite(v)]
+        return sum(vals) / len(vals) if vals else None
+
+    if scored:
+        ranked, best_by = [(k, -e["lpd"]) for k, e in enumerate(entries) if e["lpd"] is not None], "lpd (highest)"
+    else:
+        ranked = [(k, mean_loss(e)) for k, e in enumerate(entries) if mean_loss(e) is not None]
         best_by = ("mean validation loss (lowest)" if phase == "pretrain" else
                    "mean SWA validation loss (lowest): fewer than K deviation columns collected, so no lpd")
+    best = min(ranked, key=lambda kv: kv[1])[0] if ranked else None
     result = {"phase": phase, "seeds_per_config": spc, "configs": entries, "best": best, "best_by": best_by}
     with open(os.path.join(out_dir, "sweep.json"), "w") as f:
         json.dump(result, f, indent=1)
@@ -227,8 +254,9 @@ def main(argv=None):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     result = run(args, configs, *run_swag.load_data(args), args.out)
     if result is not None:
-        print(f"wrote {len(configs)} configs x {args.seeds_per_config} seeds to {args.out}; best config {result['best']} "
-              f"{result['configs'][result['best']]['overrides']}")
+        best = result["best"]
+        print(f"wrote {len(configs)} configs x {args.seeds_per_config} seeds to {args.out}; best config {best} "
+              f"{None if best is None else result['configs'][best]['overrides']}")
     if world > 1:
         dist.destroy_process_group()
 

@@ -235,6 +235,31 @@ int bnn_train_step_adam_seeds(const bnn_model_config* cfg, const bnn_train_hpara
                               const float* d_y, const int32_t* d_batch_index, int64_t B, const float* d_eps_in,
                               const float* d_eps12, const float* d_eps_sum, uint64_t seed, uint64_t step,
                               float* d_grad_out, float* d_metrics, void* d_workspace, void* stream);
+/* Per-seed halt on a non-finite step: bnn_train_step_seeds / bnn_train_step_adam_seeds plus d_halted_at [n_seeds], a
+ * caller-owned device int64 per seed: -1 while the seed's run is live, else the `step` argument of the call at which it
+ * halted.  Step k is bad for seed s when nll + skl + norm is not finite -- the batch NLL sum, the summary-KL term times
+ * beta_out and the L2 norm of the unclipped gradient, the condition of metrics column 6 (input-KL overflow reaches it
+ * through its gradient).  When seed s is already halted, or step k is bad for it, the update of s is not applied: theta,
+ * the momentum buffer and exp_avg / exp_avg_sq of s stay bit for bit what they were before the call; a live seed
+ * latches d_halted_at[s] = k.  So the offending step is not applied.  (Whether the reference's terminate_on_nan checked
+ * before or after optimizer.step() is unverified: its Lightning 1.1 source is not available.)  d_grad_out and d_metrics
+ * are written for every seed as by the _seeds entry, and a halted seed's forward / backward still runs.  Seeds are
+ * independent: a live seed's bits do not depend on whether another seed halted, and with every word -1 and no bad step
+ * the results are the _seeds entry's bit for bit.  The decision is made on the device at the step itself; the caller
+ * reads the words whenever it synchronises anyway.  The _seeds entries are these with no halt word.  BNN_E_ARG: a null
+ * d_halted_at, a step >= 2^63 (it must fit the word); BNN_E_ALIGN: d_halted_at not 8-byte aligned; both come back
+ * before the device is touched, with the _seeds entry's own checks. */
+int bnn_train_step_seeds_halt(const bnn_model_config* cfg, const bnn_train_hparams* hp, int32_t n_seeds, int32_t plan_seeds,
+                              float* d_theta, float* d_momentum, const float* d_x, const float* d_y,
+                              const int32_t* d_batch_index, int64_t B, const float* d_eps_in, const float* d_eps12,
+                              const float* d_eps_sum, uint64_t seed, uint64_t step, float* d_grad_out, float* d_metrics,
+                              void* d_workspace, int64_t* d_halted_at, void* stream);
+int bnn_train_step_adam_seeds_halt(const bnn_model_config* cfg, const bnn_train_hparams* hp, const bnn_adam_hparams* adam,
+                                   int32_t n_seeds, int32_t plan_seeds, float* d_theta, float* d_exp_avg,
+                                   float* d_exp_avg_sq, const float* d_x, const float* d_y, const int32_t* d_batch_index,
+                                   int64_t B, const float* d_eps_in, const float* d_eps12, const float* d_eps_sum,
+                                   uint64_t seed, uint64_t step, float* d_grad_out, float* d_metrics, void* d_workspace,
+                                   int64_t* d_halted_at, void* stream);
 /* Saliency (figures/feature_importance.py:93-131, gradforward): for each of n_models weight vectors d_theta[m]
  * (flatten() order; the script uses w_avg) and each system b: mu_b = predict_instability(compute_summary_stats(
  * mask(x_b)))[0] and g = d mu_b / d x (all F columns of the masked input; no input noise, no summary noise).
@@ -295,6 +320,15 @@ int bnn_eval_loss(const bnn_model_config* cfg, const float* d_x, const float* d_
 int bnn_swag_collect(const float* d_w, int64_t d, int32_t n_seeds, int32_t K, float* d_w_avg,
                      float* d_w2_avg, float* d_pre_D, int32_t* d_n_models, int32_t* d_n_cols,
                      int32_t current_epoch, int32_t c, void* stream);
+
+/* bnn_swag_collect that leaves halted seeds untouched: a seed with d_halted_at[s] >= 0 (the word of
+ * bnn_train_step_seeds_halt) keeps its w_avg, w2_avg, pre_D, n_models and n_cols; the other seeds collect as with
+ * bnn_swag_collect, which is this entry with no halt word.  A seed that halts during an epoch is therefore not collected
+ * at the end of it, like a reference run that ended mid-epoch.  BNN_E_ARG: a null pointer or bad size; BNN_E_ALIGN:
+ * d_halted_at not 8-byte aligned; both before the device is touched. */
+int bnn_swag_collect_halt(const float* d_w, int64_t d, int32_t n_seeds, int32_t K, float* d_w_avg,
+                          float* d_w2_avg, float* d_pre_D, int32_t* d_n_models, int32_t* d_n_cols,
+                          int32_t current_epoch, int32_t c, const int64_t* d_halted_at, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Input packing, the step upstream of bnn_predict: data_setup_kernel (figures/spock/regression.py:183-213)
