@@ -173,6 +173,8 @@ SIGNATURES = {
         [_CFG, C.c_int32, c_f32p, C.c_int64, c_f32p, C.c_int64, C.c_int64, C.c_uint64, C.c_void_p, C.c_int32, C.c_int64,
          c_f32p, c_f32p, c_f32p, C.c_void_p, C.c_void_p],
     ),
+    "bnn_integrate_orbits": (
+        C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 # diagnostics declared in include/bnnchaos_diag.h (probes / timers; not part of the product ABI)

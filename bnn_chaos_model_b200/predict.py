@@ -16,7 +16,13 @@ counts): per system the posterior summary [N, 8] (``posterior.STAT_NAMES``) of t
 one of
   * ``x`` [R, T, 41] float32 model inputs, normalised like run_swag's X (R = sum of n_trios);
   * ``tseries`` [R, T, 26] and ``masses`` [R, 3], the raw float64 series and masses of each trio, packed and normalised
-    on the device with the v50 scaler (``inputs.data_setup_kernel``).
+    on the device with the v50 scaler (``inputs.data_setup_kernel``);
+or, instead of all of these, ``n_planets`` [N] (3..8) and ``orbits`` [sum n_planets, 7], each system's initial orbits
+(``nbody.integrate_orbits``; n_trios = n_planets - 2): the systems are integrated for ``--n_orbits`` inner orbits on the
+device first.  That path needs an ensemble whose flags zero input columns 1-7, which the integration does not compute.
+A system that goes unstable during the integration has a known instability time t = log10_t_unstable: its summary
+columns 0-5 are t and 6-7 NaN, its survival is 1.0 where t > T and 0.0 otherwise, and its rows of uncertainty,
+trio_first, trio_summary and attribution are NaN (``nbody.override_unstable``).
 Without ``--data``, ``--synthetic N`` draws N trio counts uniformly from 1..5 and the rows from the synthetic generator.
 
 Writes to ``--out``:
@@ -28,7 +34,9 @@ Writes to ``--out``:
     its own, and ``trio_stat_names``; with ``--attribution`` ``attribution`` [R, 2, 41], per trio row and input column
     the posterior mean of (1/T) sum_t (d mu / d x)^2 (importance) and of sum_t d mu / d x (shift), ``attribution_mu``
     [R], the mean mu they belong to, and ``attribution_names`` (``MultiSWAG.posterior_attribution``);
-  * ``summary.json``: the settings, the number of systems per trio count, with ``--survival`` ``survival_mean`` and,
+    an orbit catalogue adds ``log10_t_unstable`` [N] (NaN for a system that survives the integration);
+  * ``summary.json``: the settings, the number of systems per trio count (an orbit catalogue adds
+    ``n_unstable_in_integration``, ``n_orbits`` and ``dt_frac``), with ``--survival`` ``survival_mean`` and,
     with ``--trios``, ``weakest_trio_position``: for each trio count k >= 2, how many of the systems of k trios have
     their largest ``trio_first`` at position 0 .. k - 1 (ties go to the first position); with ``--attribution``
     ``attribution_mean_importance`` [41], the importance averaged over the trio rows.
@@ -68,6 +76,10 @@ def build_parser():
     ap.add_argument("--trios", action="store_true",
                     help="also report, per trio row, how often that trio sets its system's instability time and its own "
                          "posterior summary")
+    ap.add_argument("--n_orbits", type=float, default=1e4,
+                    help="orbit catalogues: integrate this many inner orbits (outputs span 990/999 of them)")
+    ap.add_argument("--dt_frac", type=float, default=0.05,
+                    help="orbit catalogues: time step as a fraction of the shortest pericentre-scaled period")
     ap.add_argument("--attribution", action="store_true",
                     help="also attribute each trio row's predicted mean to the input columns (posterior mean of the "
                          "squared and of the summed gradient d mu / d x)")
@@ -75,12 +87,15 @@ def build_parser():
 
 
 def load_catalogue(args):
-    """(n_trios int64 [N], inputs) with inputs {"x": [R, T, 41] float32} or {"tseries": [R, T, 26], "masses": [R, 3]}
-    (float64), as CPU arrays.  Raises ValueError on a malformed catalogue, before any device work."""
+    """(n_trios int64 [N], inputs) with inputs {"x": [R, T, 41] float32}, {"tseries": [R, T, 26], "masses": [R, 3]}
+    (float64) or {"orbits": [sum P, 7] float64, "n_planets": [N] int64}, as CPU arrays.  Raises ValueError on a malformed
+    catalogue, before any device work."""
     from .posterior import row_offsets
 
     if args.data:
         z = np.load(args.data)
+        if "orbits" in z.files or "n_planets" in z.files:
+            return load_orbit_catalogue(args.data, z)
         if "n_trios" not in z.files:
             raise ValueError(f"{args.data} has no n_trios (trio rows per system)")
         has_x, has_raw = "x" in z.files, ("tseries" in z.files or "masses" in z.files)
@@ -111,6 +126,44 @@ def load_catalogue(args):
     return counts.astype(np.int64), inputs
 
 
+def load_orbit_catalogue(path, z):
+    """The orbit form of catalogue.npz: (n_trios = n_planets - 2, {"orbits", "n_planets"}), checked like
+    ``nbody.integrate_orbits`` checks its input."""
+    from . import nbody
+
+    others = sorted(set(z.files) & {"x", "tseries", "masses"})
+    if others:
+        raise ValueError(f"{path}: orbits and n_planets exclude {others}")
+    if "orbits" not in z.files or "n_planets" not in z.files:
+        raise ValueError(f"{path} must hold both orbits [sum n_planets, 7] and n_planets [N]")
+    orbits = np.asarray(z["orbits"], np.float64)
+    if orbits.ndim != 2 or orbits.shape[1] != 7:
+        raise ValueError(f"orbits must be [sum n_planets, 7], got {orbits.shape}")
+    counts = nbody.planet_counts(np.asarray(z["n_planets"]), orbits.shape[0])
+    nbody.check_elements(orbits, counts)
+    if "n_trios" in z.files and not np.array_equal(np.asarray(z["n_trios"]), counts - 2):
+        raise ValueError(f"{path}: n_trios must equal n_planets - 2")
+    return counts - 2, {"orbits": orbits, "n_planets": counts}
+
+
+def integrate_rows(inputs, counts, lo: int, hi: int, args, dev):
+    """Integrate the systems that own trio rows [lo, hi) of an orbit catalogue.  Returns (tseries, masses) of those
+    rows on `dev` and (sys_lo, log10_t_unstable of systems sys_lo ..) as a numpy array."""
+    from .nbody import integrate_orbits
+
+    off = np.concatenate([[0], np.cumsum(counts)])
+    s_lo = int(np.searchsorted(off[1:], lo, side="right"))
+    s_hi = int(np.searchsorted(off[:-1], hi, side="left"))
+    if hi <= lo or s_hi <= s_lo:
+        empty = torch.empty((0, 100, 26), dtype=torch.float64, device=dev)
+        return empty, torch.empty((0, 3), dtype=torch.float64, device=dev), (s_lo, np.empty(0))
+    poff = np.concatenate([[0], np.cumsum(inputs["n_planets"])])
+    ts, ms, lt = integrate_orbits(inputs["orbits"][poff[s_lo]:poff[s_hi]], inputs["n_planets"][s_lo:s_hi], args.n_orbits,
+                                  args.dt_frac, device=dev)
+    a, b = lo - int(off[s_lo]), hi - int(off[s_lo])
+    return ts[a:b].contiguous(), ms[a:b].contiguous(), (s_lo, lt.cpu().numpy())
+
+
 def model_inputs(inputs, lo: int, hi: int, dev) -> torch.Tensor:
     """Rows [lo, hi) of the catalogue as model inputs on `dev` (raw series are packed there)."""
     if "x" in inputs:
@@ -134,6 +187,26 @@ def weakest_trio_position(first: np.ndarray, counts: np.ndarray) -> dict:
     return res
 
 
+def orbit_outputs(arrays, info, lt, counts, args):
+    """An orbit catalogue's outputs: the known instability times of systems unstable in the integration override the
+    posterior (``nbody.override_unstable``); the means in ``info`` and ``weakest_trio_position`` leave those systems
+    out."""
+    from .nbody import override_unstable
+
+    hit = np.isfinite(lt)
+    out = override_unstable(arrays, lt, counts)
+    out["log10_t_unstable"] = lt
+    info.update(n_unstable_in_integration=int(hit.sum()), n_orbits=float(args.n_orbits), dt_frac=float(args.dt_frac))
+    if "survival" in out:
+        info["survival_mean"] = [float(v) for v in out["survival"].astype(np.float64).mean(0)]
+    if "trio_first" in out:
+        keep = ~np.repeat(hit, counts)
+        info["weakest_trio_position"] = weakest_trio_position(arrays["trio_first"][keep], counts[~hit])
+    if "attribution" in out:
+        info["attribution_mean_importance"] = [float(v) for v in np.nanmean(out["attribution"][:, 0].astype(np.float64), 0)]
+    return out
+
+
 def main(argv=None):
     """Returns the summary dict on rank 0 (None on the other ranks)."""
     import torch.distributed as dist
@@ -147,9 +220,14 @@ def main(argv=None):
     if args.samples < 1:
         raise ValueError(f"--samples must be >= 1, got {args.samples}")
     counts, inputs = load_catalogue(args)
+    orbit_form = "orbits" in inputs
+    if orbit_form:
+        from .nbody import check_run
+
+        check_run(args.n_orbits, args.dt_frac)
     if args.trios:
         check_trio_counts(counts, None)   # at most MAX_TRIOS_PER_SYSTEM trios per system
-    if args.attribution and next(iter(inputs.values())).shape[1] != 100:
+    if args.attribution and not orbit_form and next(iter(inputs.values())).shape[1] != 100:
         raise ValueError("--attribution needs T = 100 time steps per row")
     N, R = counts.size, int(counts.sum())
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -159,20 +237,43 @@ def main(argv=None):
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     ens = load_ensemble(args.models, device=dev)
+    lt_parts = []   # (sys_lo, log10_t_unstable of systems sys_lo ..) of every integration on this rank
+    if orbit_form:
+        from .nbody import check_zero_mask
+
+        check_zero_mask(ens.models)
+
+    def rows_input(lo, hi):
+        if not orbit_form:
+            return model_inputs(inputs, lo, hi, dev)
+        from .inputs import data_setup_kernel
+
+        ts, ms, part = integrate_rows(inputs, counts, lo, hi, args, dev)
+        lt_parts.append(part)
+        return data_setup_kernel(ms, ts)
+
     # summary, (with --survival) survival, (with --uncertainty) uncertainty and (with --trios) the first-trio fractions
     # and per-trio summary come from one walk, in that order
     if world > 1:
-        T = (inputs["x"] if "x" in inputs else inputs["tseries"]).shape[1]
+        T = 100 if orbit_form else (inputs["x"] if "x" in inputs else inputs["tseries"]).shape[1]
         _, _, lo, hi = catalogue_shard_range(counts, dist.get_rank(), world, ens.system_granule(T))
-        outs = ens._reduce_sharded(model_inputs(inputs, lo, hi, dev), N, args.samples, counts, args.seed, args.scale,
+        outs = ens._reduce_sharded(rows_input(lo, hi), N, args.samples, counts, args.seed, args.scale,
                                    thresholds=args.survival, uncertainty=args.uncertainty, trios=args.trios)
     else:
-        outs = ens._reduce(model_inputs(inputs, 0, R, dev), args.samples, counts, args.seed, args.scale,
+        outs = ens._reduce(rows_input(0, R), args.samples, counts, args.seed, args.scale,
                            thresholds=args.survival, uncertainty=args.uncertainty, trios=args.trios)
     if args.attribution:   # per row: each rank takes a contiguous block of rows
         lo, hi = shard_range(R, dist.get_rank(), world) if world > 1 else (0, R)
-        attr = ens.posterior_attribution_sharded(model_inputs(inputs, lo, hi, dev), N, args.samples, counts, args.seed,
+        attr = ens.posterior_attribution_sharded(rows_input(lo, hi), N, args.samples, counts, args.seed,
                                                  args.scale)
+    if orbit_form:   # every system is integrated by at least one rank; its bits do not depend on which
+        if world > 1:
+            gathered = [None] * world
+            dist.all_gather_object(gathered, lt_parts)
+            lt_parts = [p for parts in gathered for p in parts]
+        lt_full = np.full(N, np.nan)
+        for s_lo, part in lt_parts:
+            lt_full[s_lo:s_lo + part.size] = part
     info = None
     if world == 1 or dist.get_rank() == 0:
         summary = outs[0].cpu().numpy()
@@ -198,6 +299,8 @@ def main(argv=None):
             a = attr[0].cpu().numpy()
             arrays.update(attribution=a, attribution_mu=attr[1].cpu().numpy(), attribution_names=np.array(ATTRIBUTION_NAMES))
             info["attribution_mean_importance"] = [float(v) for v in a[:, 0].astype(np.float64).mean(0)]
+        if orbit_form:
+            arrays = orbit_outputs(arrays, info, lt_full, counts, args)
         os.makedirs(args.out, exist_ok=True)
         with open(os.path.join(args.out, "summary.json"), "w") as f:
             json.dump(info, f, indent=1)

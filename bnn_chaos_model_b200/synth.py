@@ -91,3 +91,31 @@ def make_labels(n: int, seed: int = 0) -> np.ndarray:
     """fp32 [n, 2] log10 instability times; >= 9 is the censored ('stable') branch."""
     rng = np.random.default_rng(seed + 7919)
     return rng.uniform(4.0, 10.0, (n, 2)).astype(np.float32)
+
+
+def initial_orbits(n: int, n_planets, seed: int = 0, spacing=(5.0, 20.0), e_max: float = 0.05,
+                   inc_max: float = 0.05) -> np.ndarray:
+    """Initial orbits for ``nbody.integrate_orbits``: [n, P, 7] for an int ``n_planets``, or [sum P, 7] for per-system
+    counts [n].  Per planet (m, a, e, inc, Omega, varpi, lambda): m = 10^U(-7, -4.3) (the masses of ``raw_systems``),
+    a1 = 1 and each next a spaced U(spacing) mutual Hill radii out, e ~ U(0, e_max), inc ~ U(0, inc_max), angles
+    U(0, 2 pi).  Systems in the range the v50 ensembles were trained on, some of them unstable within 10^4 orbits; of
+    those that survive, a few (under 2 % of 3-planet systems) have a planet scattered out of that range by a close
+    approach that stops short of Hill-sphere overlap."""
+    rng = np.random.default_rng(seed)
+    counts = np.full(n, int(n_planets)) if np.ndim(n_planets) == 0 else np.asarray(n_planets, dtype=np.int64)
+    if counts.size != n:
+        raise ValueError(f"{counts.size} planet counts for {n} systems")
+    el = np.empty((int(counts.sum()), 7))
+    el[:, 0] = 10.0 ** rng.uniform(-7.0, -4.3, el.shape[0])
+    el[:, 2] = rng.uniform(0.0, e_max, el.shape[0])
+    el[:, 3] = rng.uniform(0.0, inc_max, el.shape[0])
+    el[:, 4:7] = rng.uniform(0.0, 2 * np.pi, (el.shape[0], 3))
+    delta = rng.uniform(spacing[0], spacing[1], el.shape[0])
+    first = np.concatenate([[0], np.cumsum(counts)[:-1]])
+    # a_{p+1} = a_p (1 + k) / (1 - k), k = delta ((m_p + m_{p+1}) / 3)^(1/3) / 2: the planets delta mutual Hill radii apart
+    k = delta[1:] * ((el[:-1, 0] + el[1:, 0]) / 3.0) ** (1.0 / 3.0) / 2.0
+    log_ratio = np.concatenate([[0.0], np.log((1.0 + k) / (1.0 - k))])
+    log_ratio[first] = 0.0
+    cum = np.cumsum(log_ratio)
+    el[:, 1] = np.exp(cum - np.repeat(cum[first], counts))
+    return el.reshape(n, int(n_planets), 7) if np.ndim(n_planets) == 0 else el

@@ -443,6 +443,28 @@ int bnn_first_trio_instability_ragged(const float* d_t, int64_t n_systems, const
 int bnn_decompose_uncertainty(const float* d_pred, int64_t n_rows, int64_t n_units, int64_t units_per_model,
                               float* d_out, void* stream);
 
+/* K8: the short N-body integration from initial orbits to the model's raw inputs (csrc/nbody.cu; DESIGN.md section
+ * K8).  d_elements [n_systems, n_planets, 7] holds per planet, from the inside out, (m / M_star, a, e, inc, Omega,
+ * varpi, lambda): Jacobi elements (primary = star + interior planets, mu = G (M_interior + m)), G = M_star = 1.  Each
+ * system is integrated on its own by WHFast-style Wisdom-Holman (drift-kick-drift, Jacobi interaction kick, Gauss f
+ * and g drift, no corrector) with dt = dt_frac min_i P_i (1 - e_i)^(3/2) / sqrt(1 + e_i), and sampled at the first
+ * step boundary t >= t_k = 10 k n_orbits / 999 P1, k = 0..99 (P1: the innermost initial period).  Per adjacent trio
+ * (i, i+1, i+2), rows system-major and trio-minor (the tseries / masses layout bnn_pack_inputs takes):
+ *   d_tseries [n_systems (n_planets - 2), 100, 26]: t / P1, 0 x 7, then per trio planet (a / a_{i,0}, e, inc, Omega,
+ *     varpi, theta), angles in [0, 2 pi), a_{i,0} the initial a of the trio's innermost planet;
+ *   d_masses [n_systems (n_planets - 2), 3]: (m_i, m_{i+1}, m_{i+2});
+ *   d_log10_t_unstable [n_systems]: log10(t / P1) at the first step whose kick sees two planets nearer than the sum
+ *     of their Hill radii a_{j,0} (m_j / 3)^(1/3), or after which a Jacobi orbit is unbound; NaN when the system
+ *     reaches its last output.  An unstable system's rows from that step on are NaN.
+ * Element values are not checked on the device: a system with a planet of a <= 0, e outside [0, 1), m < 0 or a
+ * non-finite value, or whose own step count exceeds 2^31, gets NaN rows and NaN log10_t_unstable (its masses are
+ * still copied).  A system's bits depend on its own elements only.  BNN_E_ARG: null pointer, n_systems outside
+ * [1, 2^31), n_planets outside [3, 8], n_orbits or dt_frac not finite and > 0, (990 / 999) n_orbits / dt_frac > 2^31
+ * (every system's step count is at least that); BNN_E_ALIGN: an array not 8-byte aligned; every check runs before the
+ * device is touched. */
+int bnn_integrate_orbits(const double* d_elements, int64_t n_systems, int32_t n_planets, double n_orbits, double dt_frac,
+                         double* d_tseries, double* d_masses, double* d_log10_t_unstable, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
